@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — throughput of the T41 receive-chain hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the fused RX chain (ProcessIQData x n_blocks) over the whole bank of
 virtual receivers of a rank.  Workload = BASELINE.json configs[1]: 1024 concurrent receivers per
@@ -53,10 +53,17 @@ UNIT = "Msamples/s"
 N_DISTINCT = 16
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % v)
+    return v
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--streams", type=int, default=1024, help="virtual receivers per GPU")
@@ -71,7 +78,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-q15", action="store_true", help="skip the device-resident q15 leg (value_q15)")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip BASELINE.json configs[2..4] (c3 / c4 / c5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (audio, spectrum and waterfall rows of "
+                         "a fixed sample of receivers) as DIR/<name>.npy in float32; with several GPUs, rank 0's "
+                         "receivers only")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 USB, LSB, AM, NFM, PSK31, SAM = 0, 1, 2, 3, 5, 8     # SDT.h:57-68 (t41rx.h T41RX_DEMOD_*)
@@ -341,6 +355,31 @@ EXTRA_CONFIGS = {
 }
 
 
+# what --dump-outputs writes stays under 64 MB in all
+DUMP_BYTES = 48 * 2 ** 20
+
+
+def dump_outputs(out_dir, audio, spec, wf):
+    """Write what one t41rx_process_device call returned to its caller - audio [S, T, 2048] float32 and, when the call
+    made rows, spectrum rows [S, R, 512] int16 and waterfall rows [S, R, 512] uint16 - as float32 DIR/<name>.npy files:
+    every receiver and block when that fits DUMP_BYTES, else a sample of receivers (and of blocks) drawn from a fixed
+    seed.  The sample depends on the shapes only, so two builds run with the same arguments write comparable files."""
+    S, T, B = audio.shape
+    R = spec.shape[1] if spec is not None else 0
+    r = np.random.Generator(np.random.PCG64(2024))
+    nb = min(T, (DUMP_BYTES // 4 - 2 * R * 512) // B)
+    nr = min(S, DUMP_BYTES // (4 * (nb * B + 2 * R * 512)))
+    recv = np.sort(r.choice(S, nr, replace=False))
+    blocks = np.sort(r.choice(T, nb, replace=False))
+    out = {"audio": audio[recv][:, blocks].cpu().numpy()}
+    if R:
+        out["spec"] = spec[recv].cpu().numpy().astype(np.float32)
+        out["wf"] = wf[recv].cpu().numpy().view(np.uint16).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_extra_config(name, world, local, dev, steps, peak):
     """One of BASELINE.json configs[2..4], device-resident, sharded over the ranks (strong scaling: the config
     fixes the receiver count).  Returns this rank's numbers; the caller reduces the time over ranks."""
@@ -465,6 +504,8 @@ def ours(args):
     total_ms = t_start.elapsed_time(t_end)
     launch_ms = [a.elapsed_time(b) for a, b in evs]
     gpu_launches = eng.kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:         # before the q15 leg below writes the same rows
+        dump_outputs(args.dump_outputs, audio, spec if row_every else None, wf if row_every else None)
 
     total_ms_max = sharding.max_over_ranks(total_ms, dev)
     samples_per_step = world * S * T * 2048
@@ -593,10 +634,10 @@ def ours(args):
         peak_gbs, _ = measured_peak()
         for name in ("c3", "c4", "c5"):
             barrier()
-            r = run_extra_config(name, world, local, dev, max(2, min(args.steps, 5)), peak_gbs)
+            r = run_extra_config(name, world, local, dev, args.steps, peak_gbs)
             ms_max = sharding.max_over_ranks(r["ms"], dev)
             extra[name] = extra_config_entry(r, ms_max, world, peak_gbs)
-            gpu_launches += r["launches"] * max(2, min(args.steps, 5))
+            gpu_launches += r["launches"] * args.steps
 
     clk = clocks.stop()
     # explanatory second roofline: share of the SMs' issue slots the stream kernel used (instruction count of the

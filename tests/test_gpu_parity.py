@@ -406,6 +406,37 @@ def test_receivers_per_cta_invariance(monkeypatch):
         assert np.array_equal(o["spec"], outs[0]["spec"])
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """`bench.py --dump-outputs` on the GPU: the files hold what the last of its calls returned - the same calls (warm-up,
+    the clock sampler's lead-in, the timed steps) replayed through the library give the same audio and rows bit for
+    bit - and `--steps` is the number of timed steps it reports."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    S, T, warmup, steps = 16, 4, 1, 2
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = {k: v for k, v in os.environ.items() if not k.startswith("T41RX_")}
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--streams", str(S), "--blocks", str(T),
+                          "--steps", str(steps), "--warmup", str(warmup), "--no-e2e", "--no-cpu-baseline", "--no-q15",
+                          "--no-extra-configs", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, env=env,
+                         timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps and line["value"] > 0
+    params, sigs = bench.workload(T)
+    iq = np.stack([sigs[s % len(sigs)] for s in range(S)])
+    with _receiver(S) as eng:
+        eng.set_params_each([params[s % len(params)] for s in range(S)])
+        for _ in range(max(3, warmup) + 3 + steps):
+            want = eng.process(iq, row_every=T)
+    got = {k: np.load(tmp_path / (k + ".npy")) for k in ("audio", "spec", "wf")}
+    assert np.array_equal(got["audio"].view(np.uint32), want["audio"].view(np.uint32))
+    assert np.array_equal(got["spec"], want["spec"].astype(np.float32))
+    assert np.array_equal(got["wf"], want["wf"].astype(np.float32))
+    assert np.abs(got["audio"]).max() > 0
+
+
 def test_c4_full_size_16384_spectrum_rows():
     S, T, D = 16384, 2, 10
     base_p = [cases.P(spectrum_zoom=k % 5, current_scale=1 + (k // 5)) for k in range(D)]

@@ -237,6 +237,39 @@ def test_bench_reference_arm_prints_one_json_line():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
 
 
+@pytest.mark.parametrize("S,T,budget,n_recv,n_blocks", [(64, 16, 2 ** 20, 7, 16), (4, 64, 2 ** 19, 1, 63)],
+                         ids=["receivers_sampled", "blocks_sampled"])
+def test_bench_dump_outputs_is_a_fixed_bounded_sample(tmp_path, monkeypatch, S, T, budget, n_recv, n_blocks):
+    """`bench.py --dump-outputs`: float32 files within the byte budget; distinct receivers and blocks in increasing order,
+    chosen by the shapes alone (the same ones for other output values); each dumped value taken unchanged from the
+    step's output (waterfall words read as unsigned)."""
+    import bench
+    torch = pytest.importorskip("torch")
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    # audio value = position in the output, so that every dumped sample names its receiver and block
+    audio = torch.arange(S * T * 2048, dtype=torch.float32).reshape(S, T, 2048)
+    spec = torch.arange(S * 512, dtype=torch.int32).reshape(S, 1, 512).to(torch.int16)
+    wf = -1 - spec
+    picked = []
+    for d, offset in (("a", 0.0), ("b", 0.5)):
+        bench.dump_outputs(str(tmp_path / d), audio + offset, spec, wf)
+        files = sorted(os.listdir(tmp_path / d))
+        assert files == ["audio.npy", "spec.npy", "wf.npy"]
+        assert sum(os.path.getsize(tmp_path / d / f) for f in files) <= budget + 3 * 128
+        out = {f[:-4]: np.load(tmp_path / d / f) for f in files}
+        assert all(a.dtype == np.float32 for a in out.values())
+        assert out["audio"].shape == (n_recv, n_blocks, 2048) and out["spec"].shape == out["wf"].shape == (n_recv, 1, 512)
+        pos = np.floor(out["audio"][:, :, 0]).astype(np.int64) // 2048
+        recv, blocks = pos[:, 0] // T, pos[0] % T
+        assert np.array_equal(pos, recv[:, None] * T + blocks[None, :])
+        assert np.all(np.diff(recv) > 0) and np.all(np.diff(blocks) > 0)
+        assert np.array_equal(out["audio"], (audio + offset).numpy()[recv][:, blocks])
+        assert np.array_equal(out["spec"], spec.numpy()[recv].astype(np.float32))
+        assert np.array_equal(out["wf"], wf.numpy()[recv].view(np.uint16).astype(np.float32))
+        picked.append((recv, blocks))
+    assert all(np.array_equal(a, b) for a, b in zip(*picked))
+
+
 def test_filter_set_slots_are_reused_in_a_tuning_sweep():
     """A long sweep of filter cut-offs on one receiver (HostModel::Apply re-uses the slot nobody references any more instead
     of growing the table, rx_host.cpp) must leave exactly the tables a fresh design of the last setting has (the AGC
