@@ -241,6 +241,44 @@ int t41rx_multi_synchronize(t41rx_multi *m);
 int t41rx_multi_gather_rows(t41rx_multi *m, const void *const *rows, size_t bytes_per_receiver, void *dst, int *used_nccl);
 const char *t41rx_multi_last_error(void);
 
+/* ---- polyphase channelizer: one wideband capture -> the receivers' iq blocks (DESIGN §3.7) ----
+ * The capture x[n] is interleaved complex float at Fs_in = M x 96 kS/s, M = n_channels in {64, 512} (6.144 or
+ * 49.152 MS/s); n counts samples since t41rx_chan_create, x[n < 0] = 0.  Prototype h[0..N), N = 10 M: Kaiser-windowed
+ * sinc (beta 8.96), cutoff 96 kHz, designed in FP64, symmetric, unit DC gain, rounded to float: flat to +-60 kHz,
+ * <= -90 dB from 132 kHz.  Decimation D = M / 2: every channel comes out at 192 kS/s, channel k centred at
+ * (k < M/2 ? k : k - M) x 96 kHz, so any frequency of the capture lies within 48 kHz of some centre.  Sample m of
+ * channel k (m counted from the call's start; a call produces n_blocks x 2048 samples per channel):
+ *     z_k[m] = conj( sum_{i<N} h[i] x[mD - i] exp(-j 2 pi k (mD - i) / M) )
+ * The conjugate mirrors the channel: the chain's front end mirrors USB / LSB / AM / SAM once more (it negates I), so a
+ * USB receiver hears the capture's upper sideband.  The channel lags the capture by (N - 1) / 2 capture samples.
+ * The zoom x1 display spectrum of a receiver fed this way (it spans +-96 kHz) shows the prototype's roll-off beyond
+ * +-60 kHz of the channel centre; a receiver placed by t41rx_chan_tune keeps its widest filter (10 kHz) inside the
+ * flat +-60 kHz.  Cutting a run into several calls, or changing the map, gives
+ * the same samples bit for bit.  Runs on the FP32 CUDA cores (sm_100a); there is no CPU path. */
+typedef struct t41rx_chan t41rx_chan;
+/* n_receivers = the n_streams of the context the iq output feeds; every receiver starts unmapped (-1).  ENODEV without
+ * a CUDA device, EINVAL for n_channels other than 64 / 512. */
+int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device);
+void t41rx_chan_destroy(t41rx_chan *c);
+/* receivers [first, first + count) take channel[i] in [0, n_channels), or -1 = not written (their iq rows keep whatever
+ * the caller put there); several receivers may share a channel.  Effective from the next call. */
+int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *channel);
+/* DEVICE pointers (8-byte aligned), asynchronous on cuda_stream (NULL = the channelizer's own stream):
+ *   capture  float [n_blocks * 2048 * n_channels / 2][2]     the next n_blocks * 2048 * D capture samples
+ *   iq       float [n_receivers][n_blocks][2048][2]          t41rx_process_device's iq: block b holds m = 2048 b ...
+ * Ordering contract of t41rx_process_device: the end of the call is recorded on the stream it was given, and
+ * t41rx_chan_set_map, t41rx_chan_synchronize and t41rx_chan_destroy wait for it.  Two calls on different streams are
+ * not ordered against each other by the library (the capture tail lives in the channelizer). */
+int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream);
+int t41rx_chan_synchronize(t41rx_chan *c);
+/* Host only, no GPU needed: the prototype (10 * n_channels floats, h[0] first), and where to put a receiver whose
+ * carrier or dial point sits offset_hz from the capture's centre: the nearest channel centre (|f_rel| <= 48 kHz) and
+ * nco_freq = 48000 + f_rel for USB / LSB / AM / SAM, 48000 - f_rel for NFM / PSK31 (rounded to integer Hz).  EINVAL
+ * outside [-Fs_in / 2, Fs_in / 2) or for a mode t41rx_set_params rejects.  Offsets within 48 kHz below +Fs_in / 2 go
+ * to channel M / 2, whose centre -Fs_in / 2 is the same frequency. */
+int t41rx_chan_taps(int n_channels, float *taps);
+int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *nco_freq);
+
 /* Audio-spectrum + S-meter by-product of the row-producing blocks (Process.cpp:550-570; NFM: 791-805):
  *   audio_ypixel      int32 [n_streams][n_rows][270]  audioYPixel[k], k < AUDIO_SPEC_BOX_W - 2 (Process.cpp:34,555)
  *   audio_max_sq_ave  float [n_streams][n_rows]       audioMaxSquaredAve after the block (Process.cpp:32,569)

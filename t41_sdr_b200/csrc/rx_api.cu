@@ -349,6 +349,11 @@ static int Fail(int code, const char *fmt, const char *detail = "") {
   return code;
 }
 
+int t41rx::SetApiError(int code, const char *text) {
+  g_last_error = text;
+  return code;
+}
+
 #define CUDA_TRY(expr)                                                              \
   do {                                                                              \
     cudaError_t e_ = (expr);                                                        \

@@ -1,0 +1,391 @@
+/*
+ * rx_chan.cu — polyphase channelizer (t41rx_chan_*, include/t41rx.h): one wideband complex capture at M x 96 kS/s
+ * (M = 64 or 512 channels) cut into M channels of 192 kS/s, delivered in t41rx_process_device's iq layout.
+ *
+ * Transform (DESIGN §3.7): prototype h[0..N), N = K M, K = 10; decimation D = M / 2; channel k centred at
+ * (k < M/2 ? k : k - M) x 96 kHz;
+ *     z_k[m] = conj( sum_{i<N} h[i] x[mD - i] exp(-j 2 pi k (mD - i) / M) ).
+ * With u_p[m] = sum_{q<K} h[p + qM] x[mD - p - qM] this is z_k[m] = (-1)^(k m) DFT_M(conj(u[m]))[k]: one M-point
+ * forward FFT per output time, shared by all channels; for odd m the (-1)^k is a circular shift of the FFT input by M/2.
+ * A call always produces a multiple of 2048 outputs (even), so m's parity is the same counted from the call or from
+ * the channelizer's creation, and the only state between calls is the capture's last N - 1 samples (the tail).
+ *
+ * Kernel: one CTA per tile of kChanTile consecutive output times.  It stages the capture span of the tile in shared
+ * memory (cp.async; samples before the call's first one come from the tail), each thread keeps the K taps of one branch
+ * p in registers and forms u_p for its output times, the conj(u) rows are transformed in place (radix-8 passes of
+ * rx_fft.h; half of the rows re-use the span's shared memory), and every mapped receiver gets its channel's kChanTile
+ * samples, a 128-byte run.  Channels no receiver takes are computed but never written.  FP32 on the CUDA cores: a DFT
+ * as a BF16 / TF32 matrix product keeps about 60 dB of dynamic range, the chain needs 90.
+ */
+#include <cuda_runtime.h>
+
+#include <algorithm>
+#include <climits>
+#include <cmath>
+#include <new>
+#include <vector>
+
+#include "../../include/t41rx.h"
+#include "rx_design.h"
+#include "rx_fft.h"
+#include "rx_host.h"
+#include "rx_launch.h"
+
+namespace t41rx {
+
+constexpr int kChanTaps = 10;             /* K: taps per branch */
+constexpr int kChanTile = 16;             /* output times per CTA: one 128-byte run per receiver */
+constexpr double kChanSpacing = 96000.0;  /* channel spacing = half the output rate (2x oversampled) */
+constexpr double kChanBeta = 8.96;        /* Kaiser beta of a 90 dB design (the firmware's n_att) */
+
+template <int M>
+struct ChanShape {
+  static constexpr int D = M / 2;
+  static constexpr int N = kChanTaps * M;
+  static constexpr int kThreads = M >= 256 ? M : 256;
+  static constexpr int kGroups = kThreads / M;                  /* threads per branch */
+  static constexpr int kTimes = kChanTile / kGroups;            /* output times per thread */
+  static constexpr int kSpan = kChanTile * D + N;               /* capture samples a tile stages (one spare at the end) */
+  static constexpr int kRow = M + 1;
+  static constexpr int kHalf = kChanTile / 2;
+  /* FFT rows: rows 0 .. kHalf - 1 after the span, rows kHalf .. in the span once it is dead.  Row r starts in bank
+     column r (8-byte columns, 16 per 128 bytes), so a half-warp reading one channel of the 16 rows is conflict-free */
+  static __device__ __forceinline__ int RowBase(int r) { return r < kHalf ? kSpan + r * kRow : (r - kHalf) * kRow + kHalf; }
+  static constexpr int kSmemBytes = (kSpan + kHalf * kRow) * (int)sizeof(float2);
+  static_assert(kChanTile % kGroups == 0 && T41RX_BLOCK_SAMPLES % kChanTile == 0, "tile shape");
+  static_assert(kSpan % 16 == 0 && (kHalf - 1) * kRow + kHalf + M <= kSpan, "row layout");
+};
+
+/* FFT row layout: element i (natural index) of a row lives at Phys(i); the DIF passes leave X[k] at OutPos(k) */
+template <int M> __device__ __forceinline__ int ChanPhys(int i) { return M == 512 ? FftPhys(i) : i; }
+template <int M> __device__ __forceinline__ int ChanOutPos(int k) {
+  return M == 512 ? FftPhys((int)OctRev3((unsigned)k)) : (((k & 7) << 3) | (k >> 3));
+}
+
+/* one radix-8 DIF butterfly of the 64-point transform (two passes), twiddles from the 512-entry table */
+__device__ __forceinline__ void Radix8Butterfly64(float2 *buf, const float2 *tw512, int pass, int b) {
+  const int n2 = pass == 0 ? 8 : 1, j = pass == 0 ? b : 0, i0 = pass == 0 ? b : b * 8;
+  float r[8], im[8];
+#pragma unroll
+  for (int m = 0; m < 8; ++m) {
+    const float2 x = buf[i0 + m * n2];
+    r[m] = x.x;
+    im[m] = x.y;
+  }
+  Dft8(r, im);
+  buf[i0] = float2{r[0], im[0]};
+#pragma unroll
+  for (int k = 1; k < 8; ++k) {
+    float re = r[k], ie = im[k];
+    if (j != 0) {
+      const float2 w = tw512[j * k * 8];
+      re = r[k] * w.x + im[k] * w.y;
+      ie = im[k] * w.x - r[k] * w.y;
+    }
+    buf[i0 + k * n2] = float2{re, ie};
+  }
+}
+
+__device__ __forceinline__ void CpAsync8(void *smem, const void *gmem) {
+  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(s), "l"(gmem) : "memory");
+}
+
+/* capture: the call's samples; tail: the N samples before them; recv / chan: the mapped receivers grouped by channel
+   (CSR order) and the channel of each; iq: [n_receivers][n_blocks][2048] */
+template <int M>
+__global__ void __launch_bounds__(ChanShape<M>::kThreads, M == 512 ? 2 : 4)
+t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__ tail, const float *__restrict__ taps,
+                  const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
+                  int n_entries, float2 *__restrict__ iq, int n_blocks) {
+  using S = ChanShape<M>;
+  extern __shared__ float2 smem[];
+  const int tid = threadIdx.x;
+  const long long m0 = (long long)blockIdx.x * kChanTile;
+  const long long n_base = m0 * S::D - S::N;    /* capture index of smem[0] */
+
+  for (int l = tid; l < S::kSpan; l += S::kThreads) {
+    const long long n = n_base + l;
+    CpAsync8(smem + l, n < 0 ? tail + (n + S::N) : capture + n);
+  }
+  asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
+
+  const int p = tid % M, g = tid / M;
+  float h[kChanTaps];
+#pragma unroll
+  for (int q = 0; q < kChanTaps; ++q) h[q] = __ldg(taps + p + q * M);
+  __syncthreads();
+
+  /* u_p[m] for this thread's output times m = g + kGroups t (smem index of x[mD - p - qM]: mD + N - p - qM), conj(u)
+     stored at index p of row m, or p + M/2 (mod M) for odd m (m0 is even: m and the tile's row have the same parity).
+     The first half of the rows lies outside the span and is written at once; the second half waits for the barrier
+     that ends the span's life.  Half the accumulators live at a time: 512 threads x 2 CTAs per SM leave 64 registers. */
+  auto branch = [&](int t) {
+    const float2 *x = smem + (g + S::kGroups * t) * S::D + S::N - p;
+    float ar = 0.f, ai = 0.f;
+#pragma unroll
+    for (int q = 0; q < kChanTaps; ++q) {
+      const float2 v = x[-q * M];
+      ar = fmaf(h[q], v.x, ar);
+      ai = fmaf(h[q], v.y, ai);
+    }
+    return float2{ar, -ai};
+  };
+  auto slot = [&](int t) {
+    const int mm = g + S::kGroups * t;
+    return S::RowBase(mm) + ChanPhys<M>((mm & 1) ? (p ^ (M / 2)) : p);
+  };
+  constexpr int kLate = S::kTimes / 2;
+#pragma unroll
+  for (int t = 0; t < kLate; ++t) smem[slot(t)] = branch(t);
+  float2 u[kLate];
+#pragma unroll
+  for (int t = 0; t < kLate; ++t) u[t] = branch(kLate + t);
+  __syncthreads();
+#pragma unroll
+  for (int t = 0; t < kLate; ++t) smem[slot(kLate + t)] = u[t];
+  __syncthreads();
+
+  constexpr int kBflyPerRow = M / 8, kBfly = kChanTile * kBflyPerRow;
+#pragma unroll
+  for (int pass = 0; pass < (M == 512 ? 3 : 2); ++pass) {
+    for (int b = tid; b < kBfly; b += S::kThreads) {
+      float2 *row = smem + S::RowBase(b / kBflyPerRow);
+      if (M == 512) Radix8Butterfly<true>(row, tw512, pass, b % kBflyPerRow);
+      else Radix8Butterfly64(row, tw512, pass, b % kBflyPerRow);
+    }
+    __syncthreads();
+  }
+
+  /* each receiver's run: kChanTile consecutive samples inside one block (the tile size divides 2048) */
+  const long long blk = m0 / T41RX_BLOCK_SAMPLES;
+  const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
+  for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+    const int e = w / kChanTile, mm = w % kChanTile;
+    const int k = __ldg(chan + e), r = __ldg(recv + e);
+    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
+  }
+}
+
+template <int M>
+static cudaError_t LaunchChan(const float2 *capture, const float2 *tail, const float *taps, const float2 *tw,
+                              const int32_t *recv, const int32_t *chan, int n_entries, float2 *iq, int n_blocks,
+                              cudaStream_t st) {
+  using S = ChanShape<M>;
+  const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
+  t41rx_chan_kernel<M><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan, n_entries, iq,
+                                                                   n_blocks);
+  return cudaGetLastError();
+}
+
+/* modified Bessel function I0 (power series; terms fall below 1e-17 of the sum well before k = 60 for beta <= 9) */
+static double BesselI0(double x) {
+  double sum = 1.0, term = 1.0;
+  const double q = 0.25 * x * x;
+  for (int k = 1; k < 60; ++k) {
+    term *= q / ((double)k * k);
+    sum += term;
+    if (term < 1e-17 * sum) break;
+  }
+  return sum;
+}
+
+/* the prototype: Kaiser-windowed sinc, cutoff 96 kHz at M x 96 kS/s (2 / M of Nyquist), designed in FP64, unit DC gain,
+   mirrored so that it is symmetric to the bit, rounded to float */
+static void DesignChanTaps(int M, float *out) {
+  const int N = kChanTaps * M;
+  const double fc = 2.0 / M, half = 0.5 * (N - 1);
+  std::vector<double> h(N);
+  double sum = 0.0;
+  for (int n = 0; n < N / 2; ++n) {
+    const double t = n - half;                       /* never 0: N is even */
+    const double sinc = sin(M_PI * fc * t) / (M_PI * fc * t);
+    const double r = (n - half) / half;
+    const double w = BesselI0(kChanBeta * sqrt(std::max(0.0, 1.0 - r * r))) / BesselI0(kChanBeta);
+    h[n] = h[N - 1 - n] = fc * sinc * w;
+    sum += 2.0 * h[n];
+  }
+  for (int n = 0; n < N; ++n) out[n] = (float)(h[n] / sum);
+}
+
+static bool ChanCountOk(int n_channels) { return n_channels == 64 || n_channels == 512; }
+
+}  // namespace t41rx
+
+using namespace t41rx;
+
+struct t41rx_chan {
+  int device = 0;
+  int n_channels = 0;
+  int n_receivers = 0;
+  cudaStream_t stream = nullptr;
+  /* t41rx_chan_process_device may enqueue on a caller-supplied stream: its end is recorded here, and set_map /
+     synchronize / destroy wait for it (the ordering contract of t41rx_process_device) */
+  cudaEvent_t ev_ext = nullptr;
+  bool ext_pending = false;
+  float *d_taps = nullptr;       /* N */
+  float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512 */
+  float2 *d_tail = nullptr;      /* the last N capture samples of the previous calls (zeros at creation) */
+  int32_t *d_recv = nullptr, *d_chan = nullptr;   /* mapped receivers grouped by channel, and their channel */
+  int n_entries = 0;
+  std::vector<int32_t> map;      /* receiver -> channel or -1 */
+};
+
+static int ChanQuiesce(t41rx_chan *c) {
+  if (c->ext_pending) {
+    if (cudaEventSynchronize(c->ev_ext) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan: synchronisation failed");
+    c->ext_pending = false;
+  }
+  if (cudaStreamSynchronize(c->stream) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan: synchronisation failed");
+  return T41RX_OK;
+}
+
+extern "C" {
+
+void t41rx_chan_destroy(t41rx_chan *c) {
+  if (!c) return;
+  cudaSetDevice(c->device);
+  if (c->ext_pending && c->ev_ext) cudaEventSynchronize(c->ev_ext);
+  if (c->stream) cudaStreamSynchronize(c->stream);
+  void *bufs[] = {c->d_taps, c->d_tw, c->d_tail, c->d_recv, c->d_chan};
+  for (void *b : bufs)
+    if (b) cudaFree(b);
+  if (c->ev_ext) cudaEventDestroy(c->ev_ext);
+  if (c->stream) cudaStreamDestroy(c->stream);
+  delete c;
+}
+
+int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device) {
+  if (!out || !ChanCountOk(n_channels) || n_receivers <= 0)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_create: bad arguments (n_channels must be 64 or 512)");
+  *out = nullptr;
+  int n_dev = 0;
+  if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev <= 0)
+    return SetApiError(T41RX_ENODEV, "t41rx_chan_create: no CUDA device (this library has no CPU path)");
+  if (device < 0 || device >= n_dev) return SetApiError(T41RX_EINVAL, "t41rx_chan_create: device index out of range");
+  if (cudaSetDevice(device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_create: cudaSetDevice failed");
+  t41rx_chan *c = new (std::nothrow) t41rx_chan();
+  if (!c) return SetApiError(T41RX_ENOMEM, "t41rx_chan_create: out of memory");
+  c->device = device;
+  c->n_channels = n_channels;
+  c->n_receivers = n_receivers;
+  c->map.assign(n_receivers, -1);
+  auto bail = [&](int code) {
+    t41rx_chan_destroy(c);
+    return code;
+  };
+  if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
+      cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
+    return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: stream/event creation failed"));
+  const cudaError_t attr = n_channels == 512
+      ? cudaFuncSetAttribute(t41rx_chan_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, ChanShape<512>::kSmemBytes)
+      : cudaFuncSetAttribute(t41rx_chan_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, ChanShape<64>::kSmemBytes);
+  if (attr != cudaSuccess)
+    return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: kernel image for this GPU missing (built for sm_100a)"));
+  const int N = kChanTaps * n_channels;
+  std::vector<float> taps(N);
+  DesignChanTaps(n_channels, taps.data());
+  std::vector<float2> tw(512);
+  for (int k = 0; k < 512; ++k) tw[k] = float2{(float)cos(2.0 * M_PI * k / 512.0), (float)sin(2.0 * M_PI * k / 512.0)};
+  if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * 512) != cudaSuccess ||
+      cudaMalloc(&c->d_tail, sizeof(float2) * N) != cudaSuccess ||
+      cudaMalloc(&c->d_recv, sizeof(int32_t) * n_receivers) != cudaSuccess ||
+      cudaMalloc(&c->d_chan, sizeof(int32_t) * n_receivers) != cudaSuccess)
+    return bail(SetApiError(T41RX_ENOMEM, "t41rx_chan_create: device allocation failed"));
+  if (cudaMemcpy(c->d_taps, taps.data(), sizeof(float) * N, cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(c->d_tw, tw.data(), sizeof(float2) * 512, cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemset(c->d_tail, 0, sizeof(float2) * N) != cudaSuccess)
+    return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: table upload failed"));
+  *out = c;
+  return T41RX_OK;
+}
+
+int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *channel) {
+  if (!c || !channel || first < 0 || count <= 0 || first + count > c->n_receivers)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_set_map: bad range");
+  for (int i = 0; i < count; ++i)
+    if (channel[i] < -1 || channel[i] >= c->n_channels)
+      return SetApiError(T41RX_EINVAL, "t41rx_chan_set_map: channel out of range");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_set_map: cudaSetDevice failed");
+  int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  std::copy(channel, channel + count, c->map.begin() + first);
+  /* CSR order: receivers grouped by channel, ascending within a channel */
+  std::vector<int32_t> start(c->n_channels + 1, 0);
+  for (int32_t k : c->map)
+    if (k >= 0) ++start[k + 1];
+  for (int k = 0; k < c->n_channels; ++k) start[k + 1] += start[k];
+  const int n = start[c->n_channels];
+  std::vector<int32_t> recv(std::max(n, 1)), chan(std::max(n, 1)), fill(start.begin(), start.end() - 1);
+  for (int r = 0; r < c->n_receivers; ++r)
+    if (c->map[r] >= 0) {
+      const int e = fill[c->map[r]]++;
+      recv[e] = r;
+      chan[e] = c->map[r];
+    }
+  if (n > 0 && (cudaMemcpy(c->d_recv, recv.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
+                cudaMemcpy(c->d_chan, chan.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess))
+    return SetApiError(T41RX_ECUDA, "t41rx_chan_set_map: upload failed");
+  c->n_entries = n;
+  return T41RX_OK;
+}
+
+int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream) {
+  if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 7) || ((uintptr_t)iq & 7))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: bad arguments (null or not 8-byte aligned pointer, n_blocks <= 0)");
+  if (n_blocks > INT_MAX / (T41RX_BLOCK_SAMPLES / kChanTile))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: n_blocks too large for one call");
+  if (cudaSetDevice(c->device) != cudaSuccess)
+    return SetApiError(T41RX_ECUDA, "t41rx_chan_process_device: cudaSetDevice failed");
+  cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
+  const float2 *cap = (const float2 *)capture;
+  cudaError_t e = cudaSuccess;
+  if (c->n_entries > 0)
+    e = c->n_channels == 512
+        ? LaunchChan<512>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->n_entries, (float2 *)iq, n_blocks, st)
+        : LaunchChan<64>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->n_entries, (float2 *)iq, n_blocks, st);
+  /* the new tail: the call's last N samples, copied after the kernel on the same stream so no tile reads it early */
+  const size_t N = (size_t)kChanTaps * c->n_channels;
+  const size_t total = (size_t)n_blocks * T41RX_BLOCK_SAMPLES * (c->n_channels / 2);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(c->d_tail, cap + (total - N), sizeof(float2) * N, cudaMemcpyDeviceToDevice, st);
+  if (st != c->stream) {
+    cudaEventRecord(c->ev_ext, st);
+    c->ext_pending = true;
+  }
+  if (e != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_process_device: launch failed");
+  return T41RX_OK;
+}
+
+int t41rx_chan_synchronize(t41rx_chan *c) {
+  if (!c) return SetApiError(T41RX_EINVAL, "t41rx_chan_synchronize: null channelizer");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_synchronize: cudaSetDevice failed");
+  return ChanQuiesce(c);
+}
+
+int t41rx_chan_taps(int n_channels, float *taps) {
+  if (!taps || !ChanCountOk(n_channels)) return SetApiError(T41RX_EINVAL, "t41rx_chan_taps: bad arguments (n_channels must be 64 or 512)");
+  DesignChanTaps(n_channels, taps);
+  return T41RX_OK;
+}
+
+int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *nco_freq) {
+  if (!channel || !nco_freq || !ChanCountOk(n_channels))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: bad arguments");
+  t41rx_params p;
+  DefaultParams(&p);
+  p.mode = mode;
+  t41rx_mode_default_cuts(mode, &p.f_lo_cut, &p.f_hi_cut);
+  if (!ValidateParams(p)) return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: invalid mode");
+  const double half = 0.5 * n_channels * kChanSpacing;
+  if (!(offset_hz >= -half && offset_hz < half))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: offset outside the capture's band [-Fs/2, Fs/2)");
+  /* nearest centre j x 96 kHz, j in [-M/2, M/2]; j = M/2 is channel M/2 (centre -Fs/2, the same frequency as +Fs/2) */
+  const int j = (int)floor(offset_hz / kChanSpacing + 0.5);
+  const double f_rel = offset_hz - j * kChanSpacing;
+  const bool mirrored = mode == T41RX_DEMOD_USB || mode == T41RX_DEMOD_LSB || mode == T41RX_DEMOD_AM || mode == T41RX_DEMOD_SAM;
+  *channel = (j + n_channels) % n_channels;
+  *nco_freq = (int32_t)llrint(mirrored ? 48000.0 + f_rel : 48000.0 - f_rel);
+  return T41RX_OK;
+}
+
+}  // extern "C"

@@ -18,5 +18,9 @@ cudaError_t LaunchRowsKernel(const LaunchArgs &a, int n_sms, cudaStream_t st);
 long long RowsDcRefilterCount();                                        /* < 0: error */
 cudaError_t RowsPhaseCycles(unsigned long long *out64, int reset);     /* developer builds (T41RX_PHASE_TIMING) */
 
+/* entry points in other units (the channelizer, rx_chan.cu) report failures through t41rx_last_error(): sets its text
+   on the calling thread and returns code */
+int SetApiError(int code, const char *text);
+
 }  // namespace t41rx
 #endif

@@ -88,7 +88,12 @@ EXPORTS = (
     "t41rx_create_multi", "t41rx_destroy_multi", "t41rx_multi_num_devices", "t41rx_multi_num_streams", "t41rx_multi_shard",
     "t41rx_multi_set_params", "t41rx_multi_set_params_each", "t41rx_multi_get_debug", "t41rx_multi_process",
     "t41rx_multi_process_q15", "t41rx_multi_process_device", "t41rx_multi_synchronize", "t41rx_multi_gather_rows",
-    "t41rx_multi_last_error", "t41rx_dc_refilter_count")
+    "t41rx_multi_last_error", "t41rx_dc_refilter_count",
+    "t41rx_chan_create", "t41rx_chan_destroy", "t41rx_chan_set_map", "t41rx_chan_process_device", "t41rx_chan_synchronize",
+    "t41rx_chan_taps", "t41rx_chan_tune")
+
+CHAN_TAPS_PER_BRANCH = 10     # prototype length = 10 * n_channels
+CHAN_SPACING = 96000.0        # channel spacing (Hz); every channel comes out at 192 kS/s
 
 
 def build_library():
@@ -156,6 +161,14 @@ def lib():
         L.t41rx_multi_gather_rows.argtypes = [vp, C.POINTER(vp), C.c_size_t, vp, C.POINTER(ip)]
         L.t41rx_multi_last_error.restype = C.c_char_p
         L.t41rx_dc_refilter_count.restype = C.c_int64
+        L.t41rx_chan_create.argtypes = [C.POINTER(vp), ip, ip, ip]
+        L.t41rx_chan_destroy.argtypes = [vp]
+        L.t41rx_chan_destroy.restype = None
+        L.t41rx_chan_set_map.argtypes = [vp, ip, ip, C.POINTER(C.c_int32)]
+        L.t41rx_chan_process_device.argtypes = [vp, vp, vp, ip, vp]
+        L.t41rx_chan_synchronize.argtypes = [vp]
+        L.t41rx_chan_taps.argtypes = [ip, C.POINTER(C.c_float)]
+        L.t41rx_chan_tune.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         _lib = L
     return _lib
 
@@ -497,3 +510,67 @@ class MultiReceiver:
         _check_multi(lib().t41rx_multi_gather_rows(self._h, (C.c_void_p * n)(*row_ptrs), bytes_per_receiver, dst_ptr,
                                                    C.byref(used)), "t41rx_multi_gather_rows")
         return bool(used.value)
+
+
+def chan_taps(n_channels):
+    """The channelizer's prototype low-pass (float32 [10 * n_channels]); host only."""
+    taps = np.empty(CHAN_TAPS_PER_BRANCH * int(n_channels), np.float32)
+    _check(lib().t41rx_chan_taps(int(n_channels), taps.ctypes.data_as(C.POINTER(C.c_float))), "t41rx_chan_taps")
+    return taps
+
+
+def chan_centre(n_channels, channel):
+    """Centre of a channel relative to the capture's centre (Hz)."""
+    return (channel if channel < n_channels // 2 else channel - n_channels) * CHAN_SPACING
+
+
+def chan_tune(n_channels, mode, offset_hz):
+    """(channel, nco_freq) that put a receiver's carrier / dial point at offset_hz from the capture's centre; host only."""
+    ch, nco = C.c_int32(), C.c_int32()
+    _check(lib().t41rx_chan_tune(int(n_channels), int(mode), float(offset_hz), C.byref(ch), C.byref(nco)),
+           "t41rx_chan_tune")
+    return ch.value, nco.value
+
+
+class Channelizer:
+    """Polyphase channelizer on one CUDA device: a wideband capture at n_channels x 96 kS/s in, the iq blocks of
+    n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr()."""
+
+    def __init__(self, n_channels, n_receivers, device=0):
+        self._h = C.c_void_p()
+        self.n_channels = int(n_channels)
+        self.n_receivers = int(n_receivers)
+        self.device = int(device)
+        _check(lib().t41rx_chan_create(C.byref(self._h), self.n_channels, self.n_receivers, self.device),
+               "t41rx_chan_create")
+
+    def close(self):
+        if getattr(self, "_h", None):
+            lib().t41rx_chan_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def set_map(self, channels, first=0):
+        """receivers first, first + 1, ... take channels[i] (-1: not written); effective from the next call"""
+        arr = np.ascontiguousarray(channels, dtype=np.int32)
+        _check(lib().t41rx_chan_set_map(self._h, int(first), int(arr.size), arr.ctypes.data_as(C.POINTER(C.c_int32))),
+               "t41rx_chan_set_map")
+
+    def process_device(self, capture_ptr, iq_ptr, n_blocks, stream=None):
+        """capture float32 [n_blocks * 2048 * n_channels / 2, 2] -> iq float32 [n_receivers, n_blocks, 2048, 2]"""
+        _check(lib().t41rx_chan_process_device(self._h, capture_ptr, iq_ptr, int(n_blocks), stream),
+               "t41rx_chan_process_device")
+
+    def synchronize(self):
+        _check(lib().t41rx_chan_synchronize(self._h), "t41rx_chan_synchronize")

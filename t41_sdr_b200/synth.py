@@ -147,29 +147,95 @@ def psk31(stream_id, text, nco_freq=0, amp=0.25, ebn0_db=20.0, symbol_offset=0):
     Returns (iq, bits)."""
     rng = rng_for(stream_id)
     bits = psk31_bits(text)
-    n_sym = bits.size
-    # differential encoding: a 0 bit flips the phase
-    level = np.empty(n_sym + 1)
-    level[0] = 1.0
-    for k in range(n_sym):
-        level[k + 1] = level[k] * (1.0 if bits[k] else -1.0)
-    sps = SYMBOL_SAMPLES_192K
-    n = (n_sym + 1) * sps
-    n_blocks = (n + symbol_offset + BLOCK - 1) // BLOCK
-    n_blocks = ((n_blocks + 2) // 3) * 3
+    n_blocks = psk31_blocks(text, symbol_offset)
     total = n_blocks * BLOCK
-    # raised-cosine transition between symbol centres
     k = np.arange(total) - symbol_offset
-    idx = np.clip(k // sps, 0, n_sym - 1)
-    frac = (k - idx * sps) / float(sps)
-    a = level[np.clip(idx, 0, n_sym)]
-    b = level[np.clip(idx + 1, 0, n_sym)]
-    shape = a + (b - a) * 0.5 * (1.0 - np.cos(np.pi * frac))
-    shape[k < 0] = level[0]
     t = np.arange(total) / FS
     f0 = rf_for_baseband(0.0, DEMOD_USB, nco_freq)
     # Eb/N0 at 31.25 Bd referenced to the 192 kS/s complex noise density
     sigma = amp / np.sqrt(2.0 * (10.0 ** (ebn0_db / 10.0)) * 31.25 / FS)
     sigma = min(sigma, 0.2)
-    z = amp * shape * np.exp(2j * np.pi * f0 * t) + _noise(rng, total, sigma)
+    z = amp * _psk31_shape(bits, k) * np.exp(2j * np.pi * f0 * t) + _noise(rng, total, sigma)
     return _pack(z), bits
+
+
+def _psk31_shape(bits, k):
+    """Amplitude of the differentially encoded BPSK31 of `bits` at (possibly fractional) sample k of 192 kS/s, k = 0
+    being the start of symbol 0: raised-cosine transitions between the symbol levels, level[0] before the start."""
+    n_sym = bits.size
+    level = np.empty(n_sym + 1)
+    level[0] = 1.0
+    for i in range(n_sym):
+        level[i + 1] = level[i] * (1.0 if bits[i] else -1.0)
+    sps = SYMBOL_SAMPLES_192K
+    idx = np.clip(np.floor(k / sps).astype(np.int64), 0, n_sym - 1)
+    frac = (k - idx * sps) / float(sps)
+    a = level[np.clip(idx, 0, n_sym)]
+    b = level[np.clip(idx + 1, 0, n_sym)]
+    shape = a + (b - a) * 0.5 * (1.0 - np.cos(np.pi * frac))
+    shape[k < 0] = level[0]
+    return shape
+
+
+# ---- wideband captures for the channelizer (t41rx_chan_*) ----
+CHAN_SPACING = 96000.0
+CHAN_TAPS_PER_BRANCH = 10
+
+
+def wideband_rate(n_channels):
+    """Sample rate of a capture for an n_channels channelizer (Hz)."""
+    return n_channels * CHAN_SPACING
+
+
+def wideband_delay(n_channels):
+    """How far (s) a channel lags the capture: the prototype's (N - 1) / 2 samples at the capture rate, that is
+    10 - 1 / n_channels output samples."""
+    return (CHAN_TAPS_PER_BRANCH * n_channels - 1) / 2.0 / wideband_rate(n_channels)
+
+
+def psk31_blocks(text, symbol_offset=0):
+    """192 kS/s blocks (a multiple of 3) that hold the PSK31 of `text` as psk31() builds it."""
+    n = (psk31_bits(text).size + 1) * SYMBOL_SAMPLES_192K
+    n_blocks = (n + symbol_offset + BLOCK - 1) // BLOCK
+    return ((n_blocks + 2) // 3) * 3
+
+
+def wideband(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
+    """A complex capture at n_channels x 96 kS/s holding n_blocks output blocks' worth of samples (n_blocks * 2048 *
+    n_channels / 2), float32 [n, 2] interleaved (I, Q), not quantised.  `signals` is a list of (kind, offset_hz, kw):
+      ("tone", f, {amp})                                   exp(2 pi j f t)
+      ("am", f, {amp, depth, f_mod})                       carrier at f
+      ("nfm", f, {amp, deviation, f_mod})                  carrier at f
+      ("psk31", f, {amp, text, symbol_offset})             BPSK31 carrier at f
+    f is relative to the capture's centre.  Envelopes are closed-form in t, evaluated at the capture rate.  PSK31 is
+    timed in the channel's clock: symbol k is centred at output sample symbol_offset + 6144 k + 3072 of the channel,
+    as psk31() centres it in its own stream, so a receiver decodes it with the same alignment.  start_block shifts t
+    (a later piece of the same capture); the noise (sigma per component) comes from seed and start_block."""
+    fs = wideband_rate(n_channels)
+    per_block = BLOCK * n_channels // 2
+    n = n_blocks * per_block
+    n0 = start_block * per_block
+    t = (n0 + np.arange(n)) / fs
+    z = np.zeros(n, np.complex128)
+    for kind, f, kw in signals:
+        carrier = np.exp(2j * np.pi * ((f * (n0 + np.arange(n))) % fs) / fs)   # phase reduced exactly for large n
+        if kind == "tone":
+            z += kw.get("amp", 0.25) * carrier
+        elif kind == "am":
+            env = 1.0 + kw.get("depth", 0.5) * np.sin(2 * np.pi * kw.get("f_mod", 400.0) * t)
+            z += kw.get("amp", 0.2) * env * carrier
+        elif kind == "nfm":
+            dev, fm = kw.get("deviation", 2500.0), kw.get("f_mod", 1000.0)
+            z += kw.get("amp", 0.25) * carrier * np.exp(1j * (dev / fm) * np.sin(2 * np.pi * fm * t))
+        elif kind == "psk31":
+            bits = psk31_bits(kw["text"])
+            k = (t + wideband_delay(n_channels)) * FS - kw.get("symbol_offset", 0)
+            z += kw.get("amp", 0.25) * _psk31_shape(bits, k) * carrier
+        else:
+            raise ValueError("unknown signal kind %r" % (kind,))
+    if sigma > 0.0:
+        z += _noise(np.random.Generator(np.random.PCG64([SEED_BASE + int(seed), int(start_block)])), n, sigma)
+    out = np.empty((n, 2), np.float32)
+    out[:, 0] = z.real
+    out[:, 1] = z.imag
+    return out

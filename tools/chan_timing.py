@@ -1,0 +1,128 @@
+"""Channelizer timing on one GPU (DESIGN §3.7): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
+
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--json OUT]
+
+Prints the card's name and power limit (a query), then CUDA-event times of
+  - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
+  - the C2 chain step alone (t41rx_process_device on the channelizer's output, USB / AM mix, one row per step),
+  - channelize + chain on one stream,
+each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
+receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+from t41_sdr_b200 import rx  # noqa: E402
+
+HBM_BYTES_PER_S = 7.7e12
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown (nvidia-smi failed)"
+
+
+def c2_params(n):
+    r = np.random.Generator(np.random.PCG64(2024))
+    out = []
+    for k in range(n):
+        nco = int(r.integers(-20000, 20001))
+        if k % 2 == 0:
+            out.append(rx.make_params(mode=rx.DEMOD_USB, f_lo_cut=300, f_hi_cut=3000, nco_freq=nco, agc_mode=1))
+        else:
+            out.append(rx.make_params(mode=rx.DEMOD_AM, nco_freq=nco, agc_mode=1))
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--channels", type=int, default=512)
+    ap.add_argument("--receivers", type=int, default=1024)
+    ap.add_argument("--blocks", type=int, default=64)
+    ap.add_argument("--calls", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--json", default=None, help="also write the result here")
+    a = ap.parse_args()
+    import torch
+    if not torch.cuda.is_available():
+        sys.exit("chan_timing: no CUDA device")
+    M, S, T = a.channels, a.receivers, a.blocks
+    per_block = rx.BLOCK * M // 2
+    n_cap = T * per_block
+    dev = torch.device("cuda:0")
+    g = torch.Generator(device=dev).manual_seed(1)
+    capture = (0.1 * torch.randn((n_cap, 2), generator=g, device=dev)).contiguous()
+    iq = torch.empty((S, T, rx.BLOCK, 2), dtype=torch.float32, device=dev)
+    audio = torch.empty((S, T, rx.BLOCK), dtype=torch.float32, device=dev)
+    spec = torch.empty((S, 1, rx.SPECTRUM_RES), dtype=torch.int16, device=dev)
+    wf = torch.empty((S, 1, rx.SPECTRUM_RES), dtype=torch.uint16, device=dev)
+    stream = torch.cuda.Stream(device=dev)
+    sp = stream.cuda_stream
+
+    chan = rx.Channelizer(M, S)
+    chan.set_map([(r // 2) % M for r in range(S)])
+    eng = rx.Receiver(S)
+    distinct = c2_params(16)
+    eng.set_params_each([distinct[s % len(distinct)] for s in range(S)])
+
+    def do_chan():
+        chan.process_device(capture.data_ptr(), iq.data_ptr(), T, stream=sp)
+
+    def do_chain():
+        eng.process_device(iq.data_ptr(), audio.data_ptr(), T, row_every=T, spec_ptr=spec.data_ptr(),
+                           wf_ptr=wf.data_ptr(), cuda_stream=sp)
+
+    def timed(fn):
+        for _ in range(a.warmup):
+            fn()
+        stream.synchronize()
+        ms = []
+        for _ in range(a.calls):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(stream)
+            fn()
+            e1.record(stream)
+            e1.synchronize()
+            ms.append(e0.elapsed_time(e1))
+        return float(np.median(ms)), float(np.min(ms)), float(np.max(ms))
+
+    t_chan = timed(do_chan)
+    t_chain = timed(do_chain)
+    t_both = timed(lambda: (do_chan(), do_chain()))
+    chan.synchronize()
+    eng.synchronize()
+    bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
+    res = {
+        "card": card(),
+        "shape": {"channels": M, "receivers": S, "receivers_per_channel": S // M, "blocks_per_call": T,
+                  "capture_msps": M * 96e3 / 1e6, "capture_bytes": n_cap * 8, "iq_bytes": S * T * rx.BLOCK * 8},
+        "calls": a.calls, "warmup": a.warmup,
+        "chan_ms": {"median": t_chan[0], "min": t_chan[1], "max": t_chan[2]},
+        "chain_c2_ms": {"median": t_chain[0], "min": t_chain[1], "max": t_chain[2]},
+        "chan_plus_chain_ms": {"median": t_both[0], "min": t_both[1], "max": t_both[2]},
+        "chan_capture_msps": n_cap / (t_chan[0] * 1e-3) / 1e6,
+        "chan_receiver_blocks_per_s": S * T / (t_chan[0] * 1e-3),
+        "chan_bytes_moved": bytes_moved,
+        "chan_hbm_share_of_7p7_tbs": bytes_moved / (t_chan[0] * 1e-3) / HBM_BYTES_PER_S,
+        "chan_over_chain": t_chan[0] / t_chain[0],
+        "goal_chan_le_25pct_of_chain": t_chan[0] <= 0.25 * t_chain[0],
+    }
+    print(json.dumps(res, indent=1))
+    if a.json:
+        with open(a.json, "w") as f:
+            json.dump(res, f, indent=1)
+    chan.close()
+    eng.close()
+
+
+if __name__ == "__main__":
+    main()
