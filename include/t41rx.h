@@ -254,7 +254,15 @@ const char *t41rx_multi_last_error(void);
  * The zoom x1 display spectrum of a receiver fed this way (it spans +-96 kHz) shows the prototype's roll-off beyond
  * +-60 kHz of the channel centre; a receiver placed by t41rx_chan_tune keeps its widest filter (10 kHz) inside the
  * flat +-60 kHz.  Cutting a run into several calls, or changing the map, gives
- * the same samples bit for bit.  Runs on the FP32 CUDA cores (sm_100a); there is no CPU path. */
+ * the same samples bit for bit.  Runs on the FP32 CUDA cores (sm_100a); there is no CPU path.
+ * Fine tuning (opt-in, t41rx_chan_set_shift): receiver r mapped to channel k gets its channel rotated,
+ *     iq_r[m] = z_k[m] exp(+j 2 pi phi_r(m) / 192000),   phi_r(m) = (P_r + shift_r m_abs) mod 192000  (integers),
+ * m_abs counting the outputs since t41rx_chan_create, so the stream is moved up by shift_r Hz.  P_r starts at 0 and
+ * t41rx_chan_set_shift sets it so that the phase is continuous at the change: the first output after it has the phase
+ * the old shift would have given it.  A receiver whose shift was never set gets z_k bit for bit; cutting a run into
+ * calls still gives the same bits, with or without shifts.  The chain's front end rejects the opposite sideband best at
+ * NCOFreq 0 (72 dB; 19 dB at 48000, DESIGN §3.7) and decodes PSK31 there: t41rx_chan_place puts a receiver on that
+ * operating point, t41rx_chan_tune (no shift) on NCOFreq 48000 +- f_rel. */
 typedef struct t41rx_chan t41rx_chan;
 /* n_receivers = the n_streams of the context the iq output feeds; every receiver starts unmapped (-1).  ENODEV without
  * a CUDA device, EINVAL for n_channels other than 64 / 512. */
@@ -263,6 +271,9 @@ void t41rx_chan_destroy(t41rx_chan *c);
 /* receivers [first, first + count) take channel[i] in [0, n_channels), or -1 = not written (their iq rows keep whatever
  * the caller put there); several receivers may share a channel.  Effective from the next call. */
 int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *channel);
+/* receivers [first, first + count) rotated by shift_hz[i], |shift_hz[i]| < 192000 (EINVAL otherwise); every receiver
+ * starts at 0.  Effective from the next call, with continuous phase; waits for the channelizer's calls like set_map. */
+int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shift_hz);
 /* DEVICE pointers (8-byte aligned), asynchronous on cuda_stream (NULL = the channelizer's own stream):
  *   capture  float [n_blocks * 2048 * n_channels / 2][2]     the next n_blocks * 2048 * D capture samples
  *   iq       float [n_receivers][n_blocks][2048][2]          t41rx_process_device's iq: block b holds m = 2048 b ...
@@ -278,6 +289,12 @@ int t41rx_chan_synchronize(t41rx_chan *c);
  * to channel M / 2, whose centre -Fs_in / 2 is the same frequency. */
 int t41rx_chan_taps(int n_channels, float *taps);
 int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *nco_freq);
+/* Host only, the placement to use with fine tuning: the channel t41rx_chan_tune picks, the shift that brings the
+ * carrier or dial point to where the chain runs at *nco_freq, and that NCOFreq (0, the chain's best operating point):
+ * shift_hz = 48000 + f_rel for USB / LSB / AM / SAM, f_rel - 48000 for NFM / PSK31 (rounded to integer Hz; the mirrored
+ * modes see the stream conjugated).  Same EINVAL rules as t41rx_chan_tune. */
+int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *shift_hz,
+                     int32_t *nco_freq);
 
 /* Audio-spectrum + S-meter by-product of the row-producing blocks (Process.cpp:550-570; NFM: 791-805):
  *   audio_ypixel      int32 [n_streams][n_rows][270]  audioYPixel[k], k < AUDIO_SPEC_BOX_W - 2 (Process.cpp:34,555)

@@ -16,6 +16,15 @@
  * rx_fft.h; half of the rows re-use the span's shared memory), and every mapped receiver gets its channel's kChanTile
  * samples, a 128-byte run.  Channels no receiver takes are computed but never written.  FP32 on the CUDA cores: a DFT
  * as a BF16 / TF32 matrix product keeps about 60 dB of dynamic range, the chain needs 90.
+ *
+ * Fine tuning (t41rx_chan_set_shift): receiver r's run is rotated on its way out,
+ *     iq_r[m] = z_k[m] exp(+j 2 pi phi_r(m) / 192000),   phi_r(m) = (P_r + shift_r m_abs) mod 192000,
+ * m_abs counting outputs since creation.  phi is exact integer arithmetic: the host keeps m_abs mod 192000 (passed per
+ * call) and P_r, so the rotation of an output depends on the output alone, not on how the run was cut into calls.  The
+ * factor comes from a two-level table, 192000 = 480 x 400: exp(j 2 pi a / 480) exp(j 2 pi b / 192000), phi = 400 a + b.
+ * A receiver whose phase is identically 0 (shift 0, P 0) is stored unmultiplied, so its bits are those of an unshifted
+ * channelizer ((x, y) (1, 0) would turn -0 into +0); a call in which no receiver is rotated runs the kernel instance
+ * without fine tuning.
  */
 #include <cuda_runtime.h>
 
@@ -23,6 +32,7 @@
 #include <climits>
 #include <cmath>
 #include <new>
+#include <string>
 #include <vector>
 
 #include "../../include/t41rx.h"
@@ -37,6 +47,9 @@ constexpr int kChanTaps = 10;             /* K: taps per branch */
 constexpr int kChanTile = 16;             /* output times per CTA: one 128-byte run per receiver */
 constexpr double kChanSpacing = 96000.0;  /* channel spacing = half the output rate (2x oversampled) */
 constexpr double kChanBeta = 8.96;        /* Kaiser beta of a 90 dB design (the firmware's n_att) */
+constexpr int kChanOutRate = 192000;      /* the phase of a fine-tuning rotation counts in 1 / 192000 of a turn */
+constexpr int kRotCoarse = 480, kRotFine = 400;   /* kChanOutRate = kRotCoarse x kRotFine */
+static_assert(kRotCoarse * kRotFine == kChanOutRate && kChanOutRate % 512 == 0, "rotation table shape");
 
 template <int M>
 struct ChanShape {
@@ -52,7 +65,10 @@ struct ChanShape {
      column r (8-byte columns, 16 per 128 bytes), so a half-warp reading one channel of the 16 rows is conflict-free */
   static __device__ __forceinline__ int RowBase(int r) { return r < kHalf ? kSpan + r * kRow : (r - kHalf) * kRow + kHalf; }
   static constexpr int kSmemBytes = (kSpan + kHalf * kRow) * (int)sizeof(float2);
-  static_assert(kChanTile % kGroups == 0 && T41RX_BLOCK_SAMPLES % kChanTile == 0, "tile shape");
+  /* with fine tuning the rotation table follows the rows (480 + 400 float2; two CTAs of 512 still fit an SM) */
+  static constexpr int kRotBase = kSpan + kHalf * kRow;
+  static constexpr int kSmemRotBytes = kSmemBytes + (kRotCoarse + kRotFine) * (int)sizeof(float2);
+  static_assert(kChanTile % kGroups == 0 && T41RX_BLOCK_SAMPLES % kChanTile == 0 && kThreads % kChanTile == 0, "tile shape");
   static_assert(kSpan % 16 == 0 && (kHalf - 1) * kRow + kHalf + M <= kSpan, "row layout");
 };
 
@@ -91,13 +107,23 @@ __device__ __forceinline__ void CpAsync8(void *smem, const void *gmem) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(s), "l"(gmem) : "memory");
 }
 
+/* phi mod 192000 of x = shift m + P < 2^36: 192000 = 512 x 375, so x mod 192000 = ((x >> 9) mod 375) 512 + (x mod 512)
+   with x >> 9 in 32 bits */
+__device__ __forceinline__ unsigned ChanPhase(unsigned shift, unsigned m, unsigned p0) {
+  const unsigned long long x = (unsigned long long)shift * m + p0;
+  return (((unsigned)(x >> 9) % 375u) << 9) | ((unsigned)x & 511u);
+}
+
 /* capture: the call's samples; tail: the N samples before them; recv / chan: the mapped receivers grouped by channel
-   (CSR order) and the channel of each; iq: [n_receivers][n_blocks][2048] */
-template <int M>
+   (CSR order) and the channel of each; phase: each entry's (shift, P) in [0, 192000), or null when no entry is
+   rotated; rot: the 480 + 400 factors of the rotation table; m_base: outputs before this call, mod 192000;
+   iq: [n_receivers][n_blocks][2048].  kRotate = false (no entry rotated) is the kernel without fine tuning. */
+template <int M, bool kRotate>
 __global__ void __launch_bounds__(ChanShape<M>::kThreads, M == 512 ? 2 : 4)
 t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__ tail, const float *__restrict__ taps,
                   const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
-                  int n_entries, float2 *__restrict__ iq, int n_blocks) {
+                  const int2 *__restrict__ phase, const float2 *__restrict__ rot, int m_base, int n_entries,
+                  float2 *__restrict__ iq, int n_blocks) {
   using S = ChanShape<M>;
   extern __shared__ float2 smem[];
   const int tid = threadIdx.x;
@@ -108,6 +134,8 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
     const long long n = n_base + l;
     CpAsync8(smem + l, n < 0 ? tail + (n + S::N) : capture + n);
   }
+  if (kRotate)
+    for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
   asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
 
   const int p = tid % M, g = tid / M;
@@ -160,21 +188,45 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
   /* each receiver's run: kChanTile consecutive samples inside one block (the tile size divides 2048) */
   const long long blk = m0 / T41RX_BLOCK_SAMPLES;
   const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
+  if (!kRotate) {
+    for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+      const int e = w / kChanTile, mm = w % kChanTile;
+      const int k = __ldg(chan + e), r = __ldg(recv + e);
+      iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
+    }
+    return;
+  }
+  /* a thread always stores the same sample mm of the tile (kThreads is a multiple of kChanTile): its m_abs mod 192000.
+     The body has no branch (an entry with phase 0 selects the sample unmultiplied), so unrolled iterations overlap. */
+  const int mm = tid % kChanTile;
+  const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
+  const float2 *tab = smem + S::kRotBase;
+#pragma unroll 4
   for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
-    const int e = w / kChanTile, mm = w % kChanTile;
+    const int e = w / kChanTile;
     const int k = __ldg(chan + e), r = __ldg(recv + e);
-    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
+    const int2 sp = __ldg(phase + e);
+    const float2 v = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
+    const unsigned phi = ChanPhase((unsigned)sp.x, m_abs, (unsigned)sp.y), a = phi / kRotFine;
+    const float2 ca = tab[a], cb = tab[kRotCoarse + (phi - a * kRotFine)];
+    const float2 f = float2{ca.x * cb.x - ca.y * cb.y, ca.x * cb.y + ca.y * cb.x};
+    const float2 vr = float2{v.x * f.x - v.y * f.y, v.x * f.y + v.y * f.x};
+    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = (sp.x | sp.y) ? vr : v;
   }
 }
 
 template <int M>
 static cudaError_t LaunchChan(const float2 *capture, const float2 *tail, const float *taps, const float2 *tw,
-                              const int32_t *recv, const int32_t *chan, int n_entries, float2 *iq, int n_blocks,
-                              cudaStream_t st) {
+                              const int32_t *recv, const int32_t *chan, const int2 *phase, const float2 *rot, int m_base,
+                              int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
   using S = ChanShape<M>;
   const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
-  t41rx_chan_kernel<M><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan, n_entries, iq,
-                                                                   n_blocks);
+  if (phase)
+    t41rx_chan_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(capture, tail, taps, tw, recv, chan, phase,
+                                                                             rot, m_base, n_entries, iq, n_blocks);
+  else
+    t41rx_chan_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan, phase,
+                                                                           rot, m_base, n_entries, iq, n_blocks);
   return cudaGetLastError();
 }
 
@@ -210,6 +262,32 @@ static void DesignChanTaps(int M, float *out) {
 
 static bool ChanCountOk(int n_channels) { return n_channels == 64 || n_channels == 512; }
 
+template <typename K>
+static cudaError_t ChanSmemAttr(K plain, int plain_bytes, K rotating, int rotating_bytes) {
+  const cudaError_t e = cudaFuncSetAttribute(plain, cudaFuncAttributeMaxDynamicSharedMemorySize, plain_bytes);
+  return e != cudaSuccess ? e : cudaFuncSetAttribute(rotating, cudaFuncAttributeMaxDynamicSharedMemorySize, rotating_bytes);
+}
+
+/* the channel centre j x 96 kHz nearest to offset_hz (j in [-M/2, M/2]; j = M/2 is channel M/2, centre -Fs/2, the same
+   frequency as +Fs/2), the offset from it, and whether the mode's front end mirrors the stream */
+static int ChanNearest(const char *fn, int n_channels, int32_t mode, double offset_hz, int32_t *channel, double *f_rel,
+                       bool *mirrored) {
+  if (!channel || !ChanCountOk(n_channels)) return SetApiError(T41RX_EINVAL, (std::string(fn) + ": bad arguments").c_str());
+  t41rx_params p;
+  DefaultParams(&p);
+  p.mode = mode;
+  t41rx_mode_default_cuts(mode, &p.f_lo_cut, &p.f_hi_cut);
+  if (!ValidateParams(p)) return SetApiError(T41RX_EINVAL, (std::string(fn) + ": invalid mode").c_str());
+  const double half = 0.5 * n_channels * kChanSpacing;
+  if (!(offset_hz >= -half && offset_hz < half))
+    return SetApiError(T41RX_EINVAL, (std::string(fn) + ": offset outside the capture's band [-Fs/2, Fs/2)").c_str());
+  const int j = (int)floor(offset_hz / kChanSpacing + 0.5);
+  *f_rel = offset_hz - j * kChanSpacing;
+  *mirrored = mode == T41RX_DEMOD_USB || mode == T41RX_DEMOD_LSB || mode == T41RX_DEMOD_AM || mode == T41RX_DEMOD_SAM;
+  *channel = (j + n_channels) % n_channels;
+  return T41RX_OK;
+}
+
 }  // namespace t41rx
 
 using namespace t41rx;
@@ -227,8 +305,13 @@ struct t41rx_chan {
   float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512 */
   float2 *d_tail = nullptr;      /* the last N capture samples of the previous calls (zeros at creation) */
   int32_t *d_recv = nullptr, *d_chan = nullptr;   /* mapped receivers grouped by channel, and their channel */
+  int2 *d_phase = nullptr;       /* each entry's (shift, P), in the order of d_recv */
+  float2 *d_rot = nullptr;       /* 480 + 400: exp(j 2 pi a / 480), exp(j 2 pi b / 192000) */
   int n_entries = 0;
+  bool any_rotated = false;      /* some entry's phase is not identically 0 */
   std::vector<int32_t> map;      /* receiver -> channel or -1 */
+  std::vector<int32_t> shift, p0;   /* receiver -> shift and phase offset P, both in [0, 192000) */
+  int m_done = 0;                /* outputs produced since creation, mod 192000 */
 };
 
 static int ChanQuiesce(t41rx_chan *c) {
@@ -247,7 +330,7 @@ void t41rx_chan_destroy(t41rx_chan *c) {
   cudaSetDevice(c->device);
   if (c->ext_pending && c->ev_ext) cudaEventSynchronize(c->ev_ext);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  void *bufs[] = {c->d_taps, c->d_tw, c->d_tail, c->d_recv, c->d_chan};
+  void *bufs[] = {c->d_taps, c->d_tw, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_rot};
   for (void *b : bufs)
     if (b) cudaFree(b);
   if (c->ev_ext) cudaEventDestroy(c->ev_ext);
@@ -270,6 +353,8 @@ int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int dev
   c->n_channels = n_channels;
   c->n_receivers = n_receivers;
   c->map.assign(n_receivers, -1);
+  c->shift.assign(n_receivers, 0);
+  c->p0.assign(n_receivers, 0);
   auto bail = [&](int code) {
     t41rx_chan_destroy(c);
     return code;
@@ -278,8 +363,10 @@ int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int dev
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: stream/event creation failed"));
   const cudaError_t attr = n_channels == 512
-      ? cudaFuncSetAttribute(t41rx_chan_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, ChanShape<512>::kSmemBytes)
-      : cudaFuncSetAttribute(t41rx_chan_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, ChanShape<64>::kSmemBytes);
+      ? ChanSmemAttr(t41rx_chan_kernel<512, false>, ChanShape<512>::kSmemBytes, t41rx_chan_kernel<512, true>,
+                     ChanShape<512>::kSmemRotBytes)
+      : ChanSmemAttr(t41rx_chan_kernel<64, false>, ChanShape<64>::kSmemBytes, t41rx_chan_kernel<64, true>,
+                     ChanShape<64>::kSmemRotBytes);
   if (attr != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: kernel image for this GPU missing (built for sm_100a)"));
   const int N = kChanTaps * n_channels;
@@ -287,18 +374,59 @@ int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int dev
   DesignChanTaps(n_channels, taps.data());
   std::vector<float2> tw(512);
   for (int k = 0; k < 512; ++k) tw[k] = float2{(float)cos(2.0 * M_PI * k / 512.0), (float)sin(2.0 * M_PI * k / 512.0)};
+  std::vector<float2> rot(kRotCoarse + kRotFine);
+  for (int a = 0; a < kRotCoarse; ++a) rot[a] = float2{(float)cos(2.0 * M_PI * a / kRotCoarse), (float)sin(2.0 * M_PI * a / kRotCoarse)};
+  for (int b = 0; b < kRotFine; ++b)
+    rot[kRotCoarse + b] = float2{(float)cos(2.0 * M_PI * b / kChanOutRate), (float)sin(2.0 * M_PI * b / kChanOutRate)};
   if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * 512) != cudaSuccess ||
       cudaMalloc(&c->d_tail, sizeof(float2) * N) != cudaSuccess ||
       cudaMalloc(&c->d_recv, sizeof(int32_t) * n_receivers) != cudaSuccess ||
-      cudaMalloc(&c->d_chan, sizeof(int32_t) * n_receivers) != cudaSuccess)
+      cudaMalloc(&c->d_chan, sizeof(int32_t) * n_receivers) != cudaSuccess ||
+      cudaMalloc(&c->d_phase, sizeof(int2) * n_receivers) != cudaSuccess ||
+      cudaMalloc(&c->d_rot, sizeof(float2) * rot.size()) != cudaSuccess)
     return bail(SetApiError(T41RX_ENOMEM, "t41rx_chan_create: device allocation failed"));
   if (cudaMemcpy(c->d_taps, taps.data(), sizeof(float) * N, cudaMemcpyHostToDevice) != cudaSuccess ||
       cudaMemcpy(c->d_tw, tw.data(), sizeof(float2) * 512, cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(c->d_rot, rot.data(), sizeof(float2) * rot.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
       cudaMemset(c->d_tail, 0, sizeof(float2) * N) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: table upload failed"));
   *out = c;
   return T41RX_OK;
 }
+
+}  // extern "C"
+
+/* the map, shifts and phase offsets as the kernel reads them (after ChanQuiesce): CSR order, receivers grouped by
+   channel, ascending within a channel, each entry with its channel and (shift, P) */
+static int ChanUpload(t41rx_chan *c, const char *what) {
+  std::vector<int32_t> start(c->n_channels + 1, 0);
+  for (int32_t k : c->map)
+    if (k >= 0) ++start[k + 1];
+  for (int k = 0; k < c->n_channels; ++k) start[k + 1] += start[k];
+  const int n = start[c->n_channels];
+  std::vector<int32_t> recv(std::max(n, 1)), chan(std::max(n, 1)), fill(start.begin(), start.end() - 1);
+  std::vector<int2> phase(std::max(n, 1));
+  bool any = false;
+  for (int r = 0; r < c->n_receivers; ++r)
+    if (c->map[r] >= 0) {
+      const int e = fill[c->map[r]]++;
+      recv[e] = r;
+      chan[e] = c->map[r];
+      phase[e] = int2{c->shift[r], c->p0[r]};
+      any = any || c->shift[r] != 0 || c->p0[r] != 0;
+    }
+  if (n > 0 && (cudaMemcpy(c->d_recv, recv.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
+                cudaMemcpy(c->d_chan, chan.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
+                cudaMemcpy(c->d_phase, phase.data(), sizeof(int2) * n, cudaMemcpyHostToDevice) != cudaSuccess)) {
+    c->n_entries = 0;    /* a partial upload must not be used */
+    return SetApiError(T41RX_ECUDA, what);
+  }
+  c->n_entries = n;
+  c->any_rotated = any;
+  return T41RX_OK;
+}
+
+extern "C" {
 
 int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *channel) {
   if (!c || !channel || first < 0 || count <= 0 || first + count > c->n_receivers)
@@ -310,24 +438,27 @@ int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *chann
   int rc = ChanQuiesce(c);
   if (rc) return rc;
   std::copy(channel, channel + count, c->map.begin() + first);
-  /* CSR order: receivers grouped by channel, ascending within a channel */
-  std::vector<int32_t> start(c->n_channels + 1, 0);
-  for (int32_t k : c->map)
-    if (k >= 0) ++start[k + 1];
-  for (int k = 0; k < c->n_channels; ++k) start[k + 1] += start[k];
-  const int n = start[c->n_channels];
-  std::vector<int32_t> recv(std::max(n, 1)), chan(std::max(n, 1)), fill(start.begin(), start.end() - 1);
-  for (int r = 0; r < c->n_receivers; ++r)
-    if (c->map[r] >= 0) {
-      const int e = fill[c->map[r]]++;
-      recv[e] = r;
-      chan[e] = c->map[r];
-    }
-  if (n > 0 && (cudaMemcpy(c->d_recv, recv.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
-                cudaMemcpy(c->d_chan, chan.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess))
-    return SetApiError(T41RX_ECUDA, "t41rx_chan_set_map: upload failed");
-  c->n_entries = n;
-  return T41RX_OK;
+  return ChanUpload(c, "t41rx_chan_set_map: upload failed");
+}
+
+int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shift_hz) {
+  if (!c || !shift_hz || first < 0 || count <= 0 || first + count > c->n_receivers)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_set_shift: bad range");
+  for (int i = 0; i < count; ++i)
+    if (shift_hz[i] <= -kChanOutRate || shift_hz[i] >= kChanOutRate)
+      return SetApiError(T41RX_EINVAL, "t41rx_chan_set_shift: |shift| must be below 192000 Hz");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_set_shift: cudaSetDevice failed");
+  int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  /* continuous phase: the next output, m_abs = m_done, keeps the phase the old shift gives it */
+  for (int i = 0; i < count; ++i) {
+    const int r = first + i;
+    const int32_t s_new = (shift_hz[i] + kChanOutRate) % kChanOutRate;
+    const long long p = c->p0[r] + (long long)(c->shift[r] - s_new) * c->m_done;
+    c->p0[r] = (int32_t)(((p % kChanOutRate) + kChanOutRate) % kChanOutRate);
+    c->shift[r] = s_new;
+  }
+  return ChanUpload(c, "t41rx_chan_set_shift: upload failed");
 }
 
 int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream) {
@@ -340,14 +471,19 @@ int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, in
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
   const float2 *cap = (const float2 *)capture;
   cudaError_t e = cudaSuccess;
+  const int2 *phase = c->any_rotated ? c->d_phase : nullptr;
   if (c->n_entries > 0)
     e = c->n_channels == 512
-        ? LaunchChan<512>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->n_entries, (float2 *)iq, n_blocks, st)
-        : LaunchChan<64>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->n_entries, (float2 *)iq, n_blocks, st);
+        ? LaunchChan<512>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
+                          c->n_entries, (float2 *)iq, n_blocks, st)
+        : LaunchChan<64>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
+                         c->n_entries, (float2 *)iq, n_blocks, st);
   /* the new tail: the call's last N samples, copied after the kernel on the same stream so no tile reads it early */
   const size_t N = (size_t)kChanTaps * c->n_channels;
   const size_t total = (size_t)n_blocks * T41RX_BLOCK_SAMPLES * (c->n_channels / 2);
   if (e == cudaSuccess) e = cudaMemcpyAsync(c->d_tail, cap + (total - N), sizeof(float2) * N, cudaMemcpyDeviceToDevice, st);
+  if (e == cudaSuccess)
+    c->m_done = (int)((c->m_done + (long long)n_blocks * T41RX_BLOCK_SAMPLES) % kChanOutRate);
   if (st != c->stream) {
     cudaEventRecord(c->ev_ext, st);
     c->ext_pending = true;
@@ -369,22 +505,26 @@ int t41rx_chan_taps(int n_channels, float *taps) {
 }
 
 int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *nco_freq) {
-  if (!channel || !nco_freq || !ChanCountOk(n_channels))
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: bad arguments");
-  t41rx_params p;
-  DefaultParams(&p);
-  p.mode = mode;
-  t41rx_mode_default_cuts(mode, &p.f_lo_cut, &p.f_hi_cut);
-  if (!ValidateParams(p)) return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: invalid mode");
-  const double half = 0.5 * n_channels * kChanSpacing;
-  if (!(offset_hz >= -half && offset_hz < half))
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: offset outside the capture's band [-Fs/2, Fs/2)");
-  /* nearest centre j x 96 kHz, j in [-M/2, M/2]; j = M/2 is channel M/2 (centre -Fs/2, the same frequency as +Fs/2) */
-  const int j = (int)floor(offset_hz / kChanSpacing + 0.5);
-  const double f_rel = offset_hz - j * kChanSpacing;
-  const bool mirrored = mode == T41RX_DEMOD_USB || mode == T41RX_DEMOD_LSB || mode == T41RX_DEMOD_AM || mode == T41RX_DEMOD_SAM;
-  *channel = (j + n_channels) % n_channels;
+  if (!nco_freq) return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: bad arguments");
+  double f_rel = 0.0;
+  bool mirrored = false;
+  const int rc = ChanNearest("t41rx_chan_tune", n_channels, mode, offset_hz, channel, &f_rel, &mirrored);
+  if (rc) return rc;
   *nco_freq = (int32_t)llrint(mirrored ? 48000.0 + f_rel : 48000.0 - f_rel);
+  return T41RX_OK;
+}
+
+int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *shift_hz,
+                     int32_t *nco_freq) {
+  if (!shift_hz || !nco_freq) return SetApiError(T41RX_EINVAL, "t41rx_chan_place: bad arguments");
+  double f_rel = 0.0;
+  bool mirrored = false;
+  const int rc = ChanNearest("t41rx_chan_place", n_channels, mode, offset_hz, channel, &f_rel, &mirrored);
+  if (rc) return rc;
+  /* the signal moved from where t41rx_chan_tune's NCOFreq picks it up to NCOFreq 0: the mirrored modes see the stream
+     conjugated, so their shift has the opposite sign */
+  *shift_hz = (int32_t)llrint(mirrored ? 48000.0 + f_rel : f_rel - 48000.0);
+  *nco_freq = 0;
   return T41RX_OK;
 }
 

@@ -90,7 +90,7 @@ EXPORTS = (
     "t41rx_multi_process_q15", "t41rx_multi_process_device", "t41rx_multi_synchronize", "t41rx_multi_gather_rows",
     "t41rx_multi_last_error", "t41rx_dc_refilter_count",
     "t41rx_chan_create", "t41rx_chan_destroy", "t41rx_chan_set_map", "t41rx_chan_process_device", "t41rx_chan_synchronize",
-    "t41rx_chan_taps", "t41rx_chan_tune")
+    "t41rx_chan_taps", "t41rx_chan_tune", "t41rx_chan_set_shift", "t41rx_chan_place")
 
 CHAN_TAPS_PER_BRANCH = 10     # prototype length = 10 * n_channels
 CHAN_SPACING = 96000.0        # channel spacing (Hz); every channel comes out at 192 kS/s
@@ -169,6 +169,9 @@ def lib():
         L.t41rx_chan_synchronize.argtypes = [vp]
         L.t41rx_chan_taps.argtypes = [ip, C.POINTER(C.c_float)]
         L.t41rx_chan_tune.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.t41rx_chan_set_shift.argtypes = [vp, ip, ip, C.POINTER(C.c_int32)]
+        L.t41rx_chan_place.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                       C.POINTER(C.c_int32)]
         _lib = L
     return _lib
 
@@ -532,6 +535,16 @@ def chan_tune(n_channels, mode, offset_hz):
     return ch.value, nco.value
 
 
+def chan_place(n_channels, mode, offset_hz):
+    """(channel, shift, nco_freq) that put a receiver's carrier / dial point at offset_hz from the capture's centre with
+    fine tuning: the receiver is mapped to channel, rotated by shift (Channelizer.set_shift) and runs at nco_freq, the
+    chain's best operating point (0); host only."""
+    ch, shift, nco = C.c_int32(), C.c_int32(), C.c_int32()
+    _check(lib().t41rx_chan_place(int(n_channels), int(mode), float(offset_hz), C.byref(ch), C.byref(shift),
+                                  C.byref(nco)), "t41rx_chan_place")
+    return ch.value, shift.value, nco.value
+
+
 class Channelizer:
     """Polyphase channelizer on one CUDA device: a wideband capture at n_channels x 96 kS/s in, the iq blocks of
     n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr()."""
@@ -566,6 +579,13 @@ class Channelizer:
         arr = np.ascontiguousarray(channels, dtype=np.int32)
         _check(lib().t41rx_chan_set_map(self._h, int(first), int(arr.size), arr.ctypes.data_as(C.POINTER(C.c_int32))),
                "t41rx_chan_set_map")
+
+    def set_shift(self, shifts, first=0):
+        """receivers first, first + 1, ... rotated up by shifts[i] Hz (|shift| < 192000; 0 at creation); effective from
+        the next call, with continuous phase"""
+        arr = np.ascontiguousarray(shifts, dtype=np.int32)
+        _check(lib().t41rx_chan_set_shift(self._h, int(first), int(arr.size), arr.ctypes.data_as(C.POINTER(C.c_int32))),
+               "t41rx_chan_set_shift")
 
     def process_device(self, capture_ptr, iq_ptr, n_blocks, stream=None):
         """capture float32 [n_blocks * 2048 * n_channels / 2, 2] -> iq float32 [n_receivers, n_blocks, 2048, 2]"""

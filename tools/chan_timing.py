@@ -1,11 +1,13 @@
 """Channelizer timing on one GPU (DESIGN §3.7): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
 
-    python tools/chan_timing.py [--calls 20] [--warmup 3] [--json OUT]
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--json OUT]
 
 Prints the card's name and power limit (a query), then CUDA-event times of
   - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
   - the C2 chain step alone (t41rx_process_device on the channelizer's output, USB / AM mix, one row per step),
   - channelize + chain on one stream,
+  - with --shift, t41rx_chan_process_device again after every receiver has been given its own fine-tuning shift
+    (t41rx_chan_set_shift, seeded, 0 < |shift| <= 96 kHz as t41rx_chan_place gives them), in the same run,
 each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
 receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
 """
@@ -50,6 +52,7 @@ def main():
     ap.add_argument("--blocks", type=int, default=64)
     ap.add_argument("--calls", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--shift", action="store_true", help="also time the channelizer with every receiver shifted")
     ap.add_argument("--json", default=None, help="also write the result here")
     a = ap.parse_args()
     import torch
@@ -98,6 +101,12 @@ def main():
     t_chan = timed(do_chan)
     t_chain = timed(do_chain)
     t_both = timed(lambda: (do_chan(), do_chain()))
+    t_shift = None
+    if a.shift:
+        r = np.random.Generator(np.random.PCG64(2025))
+        shifts = r.integers(1, 96001, S) * r.choice([-1, 1], S)
+        chan.set_shift(shifts)
+        t_shift = timed(do_chan)
     chan.synchronize()
     eng.synchronize()
     bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
@@ -116,6 +125,10 @@ def main():
         "chan_over_chain": t_chan[0] / t_chain[0],
         "goal_chan_le_25pct_of_chain": t_chan[0] <= 0.25 * t_chain[0],
     }
+    if t_shift:
+        res["chan_all_shifted_ms"] = {"median": t_shift[0], "min": t_shift[1], "max": t_shift[2]}
+        res["shift_overhead"] = t_shift[0] / t_chan[0] - 1.0
+        res["goal_shift_overhead_le_10pct"] = t_shift[0] <= 1.10 * t_chan[0]
     print(json.dumps(res, indent=1))
     if a.json:
         with open(a.json, "w") as f:
