@@ -345,6 +345,8 @@ int ValidateParams(const t41rx_params &p) {
   if (p.current_scale < 0 || p.current_scale > 4) return 0;
   if (p.f_hi_cut <= p.f_lo_cut) return 0;
   if (p.audio_volume < 0 || p.audio_volume > 100) return 0;
+  /* the range over which the throughput kernel holds its tolerance (t41rx.h) */
+  if (p.rf_gain_all_bands < -T41RX_RF_GAIN_ALL_BANDS_MAX || p.rf_gain_all_bands > T41RX_RF_GAIN_ALL_BANDS_MAX) return 0;
   if (p.nr_option < 0 || p.nr_option > 3) return 0;
   if (p.cw_filter_index < 0 || p.cw_filter_index > 5) return 0;
   return 1;

@@ -1778,8 +1778,8 @@ struct AgcLane {
  *
  * Almost every sample CONTINUES the state the envelope detector is in (attack, fast decay, hang, slow decay, hang
  * decay), where the update is v <- max(v + (r - v) c, min_volts) with a per-state constant and no branch.  The
- * warp runs 8 samples at a time speculatively on that form (all lanes), votes once, and only re-runs the chunk
- * through the exact per-sample state machine (Step) when some lane saw a transition between states. */
+ * warp runs 8 samples at a time speculatively on that form (all lanes), and a lane re-runs the chunk through the
+ * exact per-sample state machine (Step) only when it saw a transition between states. */
 __device__ __forceinline__ void AgcBlock(AgcLane &g, float *sta, bool active) {
   constexpr int kC = 8;
   /* window maxima and back-average advances of the chunk being processed; the next chunk's are fetched
@@ -1820,7 +1820,9 @@ __device__ __forceinline__ void AgcBlock(AgcLane &g, float *sta, bool active) {
       v = fmaxf(last, g.minv);
       vo[k] = v;
     }
-    if (__all_sync(kFull, ok || !active)) {
+    /* per lane, not per warp: a receiver's result must not depend on whether a neighbour in its CTA took a
+       transition in this chunk (the quiet form and Step round differently) */
+    if (ok || !active) {
       g.v = v;
       g.fast = fmaf(g.om8f, g.fast, pf.x);
       g.hang = fmaf(g.om8h, g.hang, pf.y);

@@ -91,6 +91,14 @@ def test_invalid_parameters_are_rejected():
             rx.design_tables([rx_driver.to_rx_params(p)])
         with pytest.raises(ValueError):
             O.OracleStream().set_params(p)
+    # rfGainAllBands: the product accepts +-40 dB (t41rx.h T41RX_RF_GAIN_ALL_BANDS_MAX; the reference has no bound, but
+    # larger steps between calls take the throughput kernel below its tolerance, and from about -760 dB the FP32 gain
+    # rounds to 0 and the kernel's DC-block state became 0 / 0)
+    for g in (-41, 41, -200, 200, -1000, -2 ** 31, 2 ** 31 - 1):
+        with pytest.raises(rx.T41RxError):
+            rx.design_tables([rx_driver.to_rx_params(cases.P(rf_gain_all_bands=g))])
+    for g in (-40, 40):
+        rx.design_tables([rx_driver.to_rx_params(cases.P(rf_gain_all_bands=g))])
 
 
 @pytest.mark.skipif(_have_gpu(), reason="checks the no-GPU behaviour")
