@@ -289,7 +289,7 @@ int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shi
  * not ordered against each other by the library (the capture tail lives in the channelizer). */
 int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream);
 int t41rx_chan_synchronize(t41rx_chan *c);
-/* Host only, no GPU needed: the prototype (10 * n_channels floats, h[0] first), and where to put a receiver whose
+/* Host only, no GPU needed: the prototype (10 * n_channels floats, h[0] first; n_channels 64, 128, 512 or 1024), and where to put a receiver whose
  * carrier or dial point sits offset_hz from the capture's centre: the nearest channel centre (|f_rel| <= 48 kHz) and
  * nco_freq = 48000 + f_rel for USB / LSB / AM / SAM, 48000 - f_rel for NFM / PSK31 (rounded to integer Hz).  EINVAL
  * outside [-Fs_in / 2, Fs_in / 2) or for a mode t41rx_set_params rejects.  Offsets within 48 kHz below +Fs_in / 2 go
@@ -302,6 +302,27 @@ int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *cha
  * modes see the stream conjugated).  Same EINVAL rules as t41rx_chan_tune. */
 int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *shift_hz,
                      int32_t *nco_freq);
+/* Real captures (DESIGN §3.8), as a direct-sampling ADC delivers them: s[n] int16 at Fs_in = M x 96 kS/s, M =
+ * n_channels in {128, 1024} (12.288 MS/s: 0 - 6.144 MHz; 98.304 MS/s: 0 - 49.152 MHz, all of HF).  x[n] = s[n] / 32768
+ * (as arm_q15_to_float), then the formula above unchanged (prototype N = 10 M, D = M / 2, the conjugate).  Only
+ * channels k = 0 ... M / 2 are distinct, channel k centred at +k x 96 kHz; a real tone A cos(2 pi f t) appears in its
+ * channel with amplitude A / 2.  Mirror caveat: channel 0 holds its band together with its mirror image about 0 Hz,
+ * channel M / 2 the same about Fs_in / 2, so a receiver placed below 48 kHz or above Fs_in / 2 - 48 kHz (channel 0 or
+ * M / 2) hears the band and its mirror image at once.
+ * t41rx_chan_set_map takes channels in [0, M / 2] on a real channelizer; set_map, set_shift, synchronize, destroy, the
+ * iq layout, the phase rule and the ordering contract are those of the complex channelizer.
+ * t41rx_chan_create_real: ENODEV without a CUDA device, EINVAL for n_channels other than 128 / 1024.
+ * t41rx_chan_process_device_real: capture int16 [n_blocks * 2048 * n_channels / 2], a DEVICE pointer, 16-byte aligned;
+ * iq and cuda_stream as t41rx_chan_process_device.  Each kind of channelizer rejects the other's process call (EINVAL).
+ * t41rx_chan_tune_real / t41rx_chan_place_real: host only, freq_hz the absolute frequency in [0, Fs_in / 2] (EINVAL
+ * outside it, for NaN, for a mode t41rx_set_params rejects, for n_channels other than 128 / 1024): channel =
+ * round(freq_hz / 96000), f_rel = freq_hz - channel x 96000, nco_freq and shift_hz by the rules of t41rx_chan_tune /
+ * t41rx_chan_place. */
+int t41rx_chan_create_real(t41rx_chan **out, int n_channels, int n_receivers, int device);
+int t41rx_chan_process_device_real(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream);
+int t41rx_chan_tune_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *nco_freq);
+int t41rx_chan_place_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *shift_hz,
+                          int32_t *nco_freq);
 
 /* Audio-spectrum + S-meter by-product of the row-producing blocks (Process.cpp:550-570; NFM: 791-805):
  *   audio_ypixel      int32 [n_streams][n_rows][270]  audioYPixel[k], k < AUDIO_SPEC_BOX_W - 2 (Process.cpp:34,555)

@@ -25,6 +25,13 @@
  * A receiver whose phase is identically 0 (shift 0, P 0) is stored unmultiplied, so its bits are those of an unshifted
  * channelizer ((x, y) (1, 0) would turn -0 into +0); a call in which no receiver is rotated runs the kernel instance
  * without fine tuning.
+ *
+ * Real captures (t41rx_chan_create_real, DESIGN §3.8): int16 s[n] at M x 96 kS/s, M = 128 or 1024, x = s / 32768, the
+ * same formula; channels k = 0 .. M/2 are distinct, channel k centred at +k x 96 kHz.  u_p[m] is real, so the M-point DFT
+ * of a row is one M/2-point complex FFT of y[n] = u[2n] + j u[2n + 1] and a split,
+ *     X[k] = (Y[k] + conj Y[-k]) / 2 - j e^(-j 2 pi k / M) (Y[k] - conj Y[-k]) / 2,   k = 0 .. M/2, indices mod M/2;
+ * the odd-m shift of u by M/2 is a shift of y by M/4.  t41rx_chan_real_kernel is the complex kernel at M/2: thread n owns
+ * branches 2n and 2n + 1 (20 taps), the span is staged as int16, the split runs in the store loop.
  */
 #include <cuda_runtime.h>
 
@@ -107,11 +114,38 @@ __device__ __forceinline__ void CpAsync8(void *smem, const void *gmem) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(s), "l"(gmem) : "memory");
 }
 
+__device__ __forceinline__ void CpAsync16(void *smem, const void *gmem) {
+  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem) : "memory");
+}
+
 /* phi mod 192000 of x = shift m + P < 2^36: 192000 = 512 x 375, so x mod 192000 = ((x >> 9) mod 375) 512 + (x mod 512)
    with x >> 9 in 32 bits */
 __device__ __forceinline__ unsigned ChanPhase(unsigned shift, unsigned m, unsigned p0) {
   const unsigned long long x = (unsigned long long)shift * m + p0;
   return (((unsigned)(x >> 9) % 375u) << 9) | ((unsigned)x & 511u);
+}
+
+/* exp(j 2 pi phi / 192000) for the entry (shift, P) = sp at output m_abs, from the staged two-level table */
+__device__ __forceinline__ float2 ChanRotor(const float2 *tab, int2 sp, unsigned m_abs) {
+  const unsigned phi = ChanPhase((unsigned)sp.x, m_abs, (unsigned)sp.y), a = phi / kRotFine;
+  const float2 ca = tab[a], cb = tab[kRotCoarse + (phi - a * kRotFine)];
+  return float2{ca.x * cb.x - ca.y * cb.y, ca.x * cb.y + ca.y * cb.x};
+}
+
+/* the in-place FFTs of the kChanTile rows of a tile (M-point; S::RowBase places the rows) */
+template <int M, typename S>
+__device__ __forceinline__ void ChanRowsFft(float2 *smem, const float2 *tw512, int tid) {
+  constexpr int kBflyPerRow = M / 8, kBfly = kChanTile * kBflyPerRow;
+#pragma unroll
+  for (int pass = 0; pass < (M == 512 ? 3 : 2); ++pass) {
+    for (int b = tid; b < kBfly; b += S::kThreads) {
+      float2 *row = smem + S::RowBase(b / kBflyPerRow);
+      if (M == 512) Radix8Butterfly<true>(row, tw512, pass, b % kBflyPerRow);
+      else Radix8Butterfly64(row, tw512, pass, b % kBflyPerRow);
+    }
+    __syncthreads();
+  }
 }
 
 /* capture: the call's samples; tail: the N samples before them; recv / chan: the mapped receivers grouped by channel
@@ -174,16 +208,7 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
   for (int t = 0; t < kLate; ++t) smem[slot(kLate + t)] = u[t];
   __syncthreads();
 
-  constexpr int kBflyPerRow = M / 8, kBfly = kChanTile * kBflyPerRow;
-#pragma unroll
-  for (int pass = 0; pass < (M == 512 ? 3 : 2); ++pass) {
-    for (int b = tid; b < kBfly; b += S::kThreads) {
-      float2 *row = smem + S::RowBase(b / kBflyPerRow);
-      if (M == 512) Radix8Butterfly<true>(row, tw512, pass, b % kBflyPerRow);
-      else Radix8Butterfly64(row, tw512, pass, b % kBflyPerRow);
-    }
-    __syncthreads();
-  }
+  ChanRowsFft<M, S>(smem, tw512, tid);
 
   /* each receiver's run: kChanTile consecutive samples inside one block (the tile size divides 2048) */
   const long long blk = m0 / T41RX_BLOCK_SAMPLES;
@@ -207,9 +232,135 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
     const int k = __ldg(chan + e), r = __ldg(recv + e);
     const int2 sp = __ldg(phase + e);
     const float2 v = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
-    const unsigned phi = ChanPhase((unsigned)sp.x, m_abs, (unsigned)sp.y), a = phi / kRotFine;
-    const float2 ca = tab[a], cb = tab[kRotCoarse + (phi - a * kRotFine)];
-    const float2 f = float2{ca.x * cb.x - ca.y * cb.y, ca.x * cb.y + ca.y * cb.x};
+    const float2 f = ChanRotor(tab, sp, m_abs);
+    const float2 vr = float2{v.x * f.x - v.y * f.y, v.x * f.y + v.y * f.x};
+    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = (sp.x | sp.y) ? vr : v;
+  }
+}
+
+template <int M>
+struct ChanRealShape {
+  static constexpr int Mc = M / 2;                              /* length of the complex FFT */
+  static constexpr int D = M / 2;
+  static constexpr int N = kChanTaps * M;
+  static constexpr int kThreads = Mc >= 256 ? Mc : 256;
+  static constexpr int kGroups = kThreads / Mc;                 /* threads per branch pair */
+  static constexpr int kTimes = kChanTile / kGroups;
+  static constexpr int kSpan = kChanTile * D + N;               /* int16 capture samples a tile stages */
+  static constexpr int kSpanF2 = kSpan * 2 / (int)sizeof(float2);
+  static constexpr int kRow = Mc + 1;
+  /* the int16 span is half the size of the complex kernel's, so only a quarter of the rows wait for it to die: the
+     thread holds 4 accumulators beside its 20 taps (8 spill at the 64 registers two CTAs of 512 allow) */
+  static constexpr int kLateTimes = kTimes / 4;
+  static constexpr int kEarly = kChanTile - kGroups * kLateTimes;   /* rows outside the span */
+  /* row r starts in bank column r, as in t41rx_chan_kernel */
+  static __device__ __forceinline__ int RowBase(int r) { return r < kEarly ? kSpanF2 + r * kRow : (r - kEarly) * kRow + kEarly; }
+  static constexpr int kSplitBase = kSpanF2 + kEarly * kRow;    /* Mc + 1 (cos, sin) of 2 pi k / M */
+  static constexpr int kRotBase = kSplitBase + Mc + 1;
+  static constexpr int kSmemBytes = kRotBase * (int)sizeof(float2);
+  static constexpr int kSmemRotBytes = kSmemBytes + (kRotCoarse + kRotFine) * (int)sizeof(float2);
+  static_assert(kChanTile % kGroups == 0 && kThreads % kChanTile == 0, "tile shape");
+  static_assert(kSpan % 8 == 0 && N % 8 == 0 && kSpanF2 % 16 == 0 && kTimes % 4 == 0, "span shape");
+  static_assert((kChanTile - 1 - kEarly) * kRow + kEarly + Mc <= kSpanF2, "late rows inside the span");
+};
+
+/* int16 -> float, exactly: 0x4B400000 + v are the bits of 1.5 x 2^23 + v (|v| < 2^22 keeps the exponent), one integer
+   add and one float subtract where a conversion instruction issues at an eighth of the FMA rate */
+__device__ __forceinline__ float ChanS16(short v) { return __int_as_float(0x4B400000 + (int)v) - 12582912.0f; }
+
+/* capture / tail: int16, 16-byte aligned; taps: h / 65536 (the 1 / 32768 of the input scale and the split's 1 / 2,
+   both exact); split: (cos, sin) of 2 pi k / M, k <= M / 2; the rest as t41rx_chan_kernel.  Channel k in [0, M/2]. */
+template <int M, bool kRotate>
+__global__ void __launch_bounds__(ChanRealShape<M>::kThreads, M == 1024 ? 2 : 4)
+t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restrict__ tail, const float *__restrict__ taps,
+                       const float2 *__restrict__ tw512, const float2 *__restrict__ split, const int32_t *__restrict__ recv,
+                       const int32_t *__restrict__ chan, const int2 *__restrict__ phase, const float2 *__restrict__ rot,
+                       int m_base, int n_entries, float2 *__restrict__ iq, int n_blocks) {
+  using S = ChanRealShape<M>;
+  constexpr int Mc = S::Mc;
+  extern __shared__ float2 smem[];
+  const short *span = reinterpret_cast<const short *>(smem);
+  const int tid = threadIdx.x;
+  const long long m0 = (long long)blockIdx.x * kChanTile;
+  const long long n_base = m0 * S::D - S::N;    /* capture index of span[0]; a multiple of 8, as N is */
+
+  for (int l = tid; l < S::kSpan / 8; l += S::kThreads) {
+    const long long n = n_base + 8 * l;
+    CpAsync16(smem + 2 * l, n < 0 ? tail + (n + S::N) : capture + n);
+  }
+  for (int l = tid; l <= Mc; l += S::kThreads) CpAsync8(smem + S::kSplitBase + l, split + l);
+  if (kRotate)
+    for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
+  asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
+
+  const int p = tid % Mc, g = tid / Mc;
+  float he[kChanTaps], ho[kChanTaps];
+#pragma unroll
+  for (int q = 0; q < kChanTaps; ++q) {
+    he[q] = __ldg(taps + 2 * p + q * M);
+    ho[q] = __ldg(taps + 2 * p + 1 + q * M);
+  }
+  __syncthreads();
+
+  /* y_p[m] = u_2p[m] + j u_2p+1[m] (span index of x[mD - 2p - qM]: mD + N - 2p - qM), stored at index p of row m, or
+     p + Mc/2 (mod Mc) for odd m; the late rows wait for the barrier that ends the span's life, as in t41rx_chan_kernel */
+  auto branch = [&](int t) {
+    const short *x = span + (g + S::kGroups * t) * S::D + S::N - 2 * p;
+    float ar = 0.f, ai = 0.f;
+#pragma unroll
+    for (int q = 0; q < kChanTaps; ++q) {
+      ar = fmaf(he[q], ChanS16(x[-q * M]), ar);
+      ai = fmaf(ho[q], ChanS16(x[-q * M - 1]), ai);
+    }
+    return float2{ar, ai};
+  };
+  auto slot = [&](int t) {
+    const int mm = g + S::kGroups * t;
+    return S::RowBase(mm) + ChanPhys<Mc>((mm & 1) ? (p ^ (Mc / 2)) : p);
+  };
+  constexpr int kEarlyTimes = S::kTimes - S::kLateTimes;
+  /* not unrolled: interleaving the output times' loads pushes two taps out of the 64 registers at M = 1024 */
+#pragma unroll 1
+  for (int t = 0; t < kEarlyTimes; ++t) smem[slot(t)] = branch(t);
+  float2 u[S::kLateTimes];
+#pragma unroll
+  for (int t = 0; t < S::kLateTimes; ++t) u[t] = branch(kEarlyTimes + t);
+  __syncthreads();
+#pragma unroll
+  for (int t = 0; t < S::kLateTimes; ++t) smem[slot(kEarlyTimes + t)] = u[t];
+  __syncthreads();
+
+  ChanRowsFft<Mc, S>(smem, tw512, tid);
+
+  /* X[k] of row mm from Y[k] and Y[Mc - k] (the 1 / 2 is in the taps) */
+  const float2 *w_tab = smem + S::kSplitBase;
+  auto sample = [&](int mm, int k) {
+    const float2 a = smem[S::RowBase(mm) + ChanOutPos<Mc>(k & (Mc - 1))];
+    const float2 b = smem[S::RowBase(mm) + ChanOutPos<Mc>((Mc - k) & (Mc - 1))];
+    const float2 w = w_tab[k];
+    const float sr = a.x + b.x, si = a.y - b.y, dr = a.x - b.x, di = a.y + b.y;
+    return float2{sr + w.x * di - w.y * dr, si - w.y * di - w.x * dr};
+  };
+  const long long blk = m0 / T41RX_BLOCK_SAMPLES;
+  const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
+  const int mm = tid % kChanTile;    /* w % kChanTile below: kThreads is a multiple of kChanTile */
+  if (!kRotate) {
+    for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+      const int e = w / kChanTile;
+      const int k = __ldg(chan + e), r = __ldg(recv + e);
+      iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = sample(mm, k);
+    }
+    return;
+  }
+  const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
+  const float2 *tab = smem + S::kRotBase;
+#pragma unroll 4
+  for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+    const int e = w / kChanTile;
+    const int k = __ldg(chan + e), r = __ldg(recv + e);
+    const int2 sp = __ldg(phase + e);
+    const float2 v = sample(mm, k);
+    const float2 f = ChanRotor(tab, sp, m_abs);
     const float2 vr = float2{v.x * f.x - v.y * f.y, v.x * f.y + v.y * f.x};
     iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = (sp.x | sp.y) ? vr : v;
   }
@@ -227,6 +378,21 @@ static cudaError_t LaunchChan(const float2 *capture, const float2 *tail, const f
   else
     t41rx_chan_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan, phase,
                                                                            rot, m_base, n_entries, iq, n_blocks);
+  return cudaGetLastError();
+}
+
+template <int M>
+static cudaError_t LaunchChanReal(const short *capture, const short *tail, const float *taps, const float2 *tw,
+                                  const float2 *split, const int32_t *recv, const int32_t *chan, const int2 *phase,
+                                  const float2 *rot, int m_base, int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
+  using S = ChanRealShape<M>;
+  const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
+  if (phase)
+    t41rx_chan_real_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
+        capture, tail, taps, tw, split, recv, chan, phase, rot, m_base, n_entries, iq, n_blocks);
+  else
+    t41rx_chan_real_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
+        capture, tail, taps, tw, split, recv, chan, phase, rot, m_base, n_entries, iq, n_blocks);
   return cudaGetLastError();
 }
 
@@ -261,6 +427,7 @@ static void DesignChanTaps(int M, float *out) {
 }
 
 static bool ChanCountOk(int n_channels) { return n_channels == 64 || n_channels == 512; }
+static bool ChanRealCountOk(int n_channels) { return n_channels == 128 || n_channels == 1024; }
 
 template <typename K>
 static cudaError_t ChanSmemAttr(K plain, int plain_bytes, K rotating, int rotating_bytes) {
@@ -269,22 +436,52 @@ static cudaError_t ChanSmemAttr(K plain, int plain_bytes, K rotating, int rotati
 }
 
 /* the channel centre j x 96 kHz nearest to offset_hz (j in [-M/2, M/2]; j = M/2 is channel M/2, centre -Fs/2, the same
-   frequency as +Fs/2), the offset from it, and whether the mode's front end mirrors the stream */
-static int ChanNearest(const char *fn, int n_channels, int32_t mode, double offset_hz, int32_t *channel, double *f_rel,
-                       bool *mirrored) {
-  if (!channel || !ChanCountOk(n_channels)) return SetApiError(T41RX_EINVAL, (std::string(fn) + ": bad arguments").c_str());
+   frequency as +Fs/2), the offset from it, and whether the mode's front end mirrors the stream.  real: a real
+   channelizer's M, offset_hz is the absolute frequency in [0, Fs/2] and the channel is j itself, in [0, M/2]. */
+static int ChanNearest(const char *fn, bool real, int n_channels, int32_t mode, double offset_hz, int32_t *channel,
+                       double *f_rel, bool *mirrored) {
+  if (!channel || !(real ? ChanRealCountOk(n_channels) : ChanCountOk(n_channels)))
+    return SetApiError(T41RX_EINVAL, (std::string(fn) + ": bad arguments").c_str());
   t41rx_params p;
   DefaultParams(&p);
   p.mode = mode;
   t41rx_mode_default_cuts(mode, &p.f_lo_cut, &p.f_hi_cut);
   if (!ValidateParams(p)) return SetApiError(T41RX_EINVAL, (std::string(fn) + ": invalid mode").c_str());
   const double half = 0.5 * n_channels * kChanSpacing;
-  if (!(offset_hz >= -half && offset_hz < half))
-    return SetApiError(T41RX_EINVAL, (std::string(fn) + ": offset outside the capture's band [-Fs/2, Fs/2)").c_str());
+  if (real ? !(offset_hz >= 0.0 && offset_hz <= half) : !(offset_hz >= -half && offset_hz < half))
+    return SetApiError(T41RX_EINVAL, (std::string(fn) + (real ? ": frequency outside the capture's band [0, Fs/2]"
+                                                               : ": offset outside the capture's band [-Fs/2, Fs/2)")).c_str());
   const int j = (int)floor(offset_hz / kChanSpacing + 0.5);
   *f_rel = offset_hz - j * kChanSpacing;
   *mirrored = mode == T41RX_DEMOD_USB || mode == T41RX_DEMOD_LSB || mode == T41RX_DEMOD_AM || mode == T41RX_DEMOD_SAM;
-  *channel = (j + n_channels) % n_channels;
+  *channel = real ? j : (j + n_channels) % n_channels;
+  return T41RX_OK;
+}
+
+/* t41rx_chan_tune / _tune_real */
+static int ChanTune(const char *fn, bool real, int n_channels, int32_t mode, double offset_hz, int32_t *channel,
+                    int32_t *nco_freq) {
+  if (!nco_freq) return SetApiError(T41RX_EINVAL, (std::string(fn) + ": bad arguments").c_str());
+  double f_rel = 0.0;
+  bool mirrored = false;
+  const int rc = ChanNearest(fn, real, n_channels, mode, offset_hz, channel, &f_rel, &mirrored);
+  if (rc) return rc;
+  *nco_freq = (int32_t)llrint(mirrored ? 48000.0 + f_rel : 48000.0 - f_rel);
+  return T41RX_OK;
+}
+
+/* t41rx_chan_place / _place_real */
+static int ChanPlace(const char *fn, bool real, int n_channels, int32_t mode, double offset_hz, int32_t *channel,
+                     int32_t *shift_hz, int32_t *nco_freq) {
+  if (!shift_hz || !nco_freq) return SetApiError(T41RX_EINVAL, (std::string(fn) + ": bad arguments").c_str());
+  double f_rel = 0.0;
+  bool mirrored = false;
+  const int rc = ChanNearest(fn, real, n_channels, mode, offset_hz, channel, &f_rel, &mirrored);
+  if (rc) return rc;
+  /* the signal moved from where t41rx_chan_tune's NCOFreq picks it up to NCOFreq 0: the mirrored modes see the stream
+     conjugated, so their shift has the opposite sign */
+  *shift_hz = (int32_t)llrint(mirrored ? 48000.0 + f_rel : f_rel - 48000.0);
+  *nco_freq = 0;
   return T41RX_OK;
 }
 
@@ -296,14 +493,16 @@ struct t41rx_chan {
   int device = 0;
   int n_channels = 0;
   int n_receivers = 0;
+  bool real = false;             /* int16 real capture (t41rx_chan_create_real): channels 0 .. n_channels / 2 */
   cudaStream_t stream = nullptr;
   /* t41rx_chan_process_device may enqueue on a caller-supplied stream: its end is recorded here, and set_map /
      synchronize / destroy wait for it (the ordering contract of t41rx_process_device) */
   cudaEvent_t ev_ext = nullptr;
   bool ext_pending = false;
-  float *d_taps = nullptr;       /* N */
+  float *d_taps = nullptr;       /* N (real: h / 65536) */
   float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512 */
-  float2 *d_tail = nullptr;      /* the last N capture samples of the previous calls (zeros at creation) */
+  float2 *d_split = nullptr;     /* real: n_channels / 2 + 1 (cos, sin) of 2 pi k / n_channels */
+  void *d_tail = nullptr;        /* the last N capture samples of the previous calls (zeros at creation) */
   int32_t *d_recv = nullptr, *d_chan = nullptr;   /* mapped receivers grouped by channel, and their channel */
   int2 *d_phase = nullptr;       /* each entry's (shift, P), in the order of d_recv */
   float2 *d_rot = nullptr;       /* 480 + 400: exp(j 2 pi a / 480), exp(j 2 pi b / 192000) */
@@ -330,7 +529,7 @@ void t41rx_chan_destroy(t41rx_chan *c) {
   cudaSetDevice(c->device);
   if (c->ext_pending && c->ev_ext) cudaEventSynchronize(c->ev_ext);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  void *bufs[] = {c->d_taps, c->d_tw, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_rot};
+  void *bufs[] = {c->d_taps, c->d_tw, c->d_split, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_rot};
   for (void *b : bufs)
     if (b) cudaFree(b);
   if (c->ev_ext) cudaEventDestroy(c->ev_ext);
@@ -338,20 +537,26 @@ void t41rx_chan_destroy(t41rx_chan *c) {
   delete c;
 }
 
-int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device) {
-  if (!out || !ChanCountOk(n_channels) || n_receivers <= 0)
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_create: bad arguments (n_channels must be 64 or 512)");
+}  // extern "C"
+
+/* t41rx_chan_create / _create_real; fn names the entry point in error messages */
+static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channels, int n_receivers, int device) {
+  const std::string f(fn);
+  if (!out || !(real ? ChanRealCountOk(n_channels) : ChanCountOk(n_channels)) || n_receivers <= 0)
+    return SetApiError(T41RX_EINVAL, (f + (real ? ": bad arguments (n_channels must be 128 or 1024)"
+                                               : ": bad arguments (n_channels must be 64 or 512)")).c_str());
   *out = nullptr;
   int n_dev = 0;
   if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev <= 0)
-    return SetApiError(T41RX_ENODEV, "t41rx_chan_create: no CUDA device (this library has no CPU path)");
-  if (device < 0 || device >= n_dev) return SetApiError(T41RX_EINVAL, "t41rx_chan_create: device index out of range");
-  if (cudaSetDevice(device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_create: cudaSetDevice failed");
+    return SetApiError(T41RX_ENODEV, (f + ": no CUDA device (this library has no CPU path)").c_str());
+  if (device < 0 || device >= n_dev) return SetApiError(T41RX_EINVAL, (f + ": device index out of range").c_str());
+  if (cudaSetDevice(device) != cudaSuccess) return SetApiError(T41RX_ECUDA, (f + ": cudaSetDevice failed").c_str());
   t41rx_chan *c = new (std::nothrow) t41rx_chan();
-  if (!c) return SetApiError(T41RX_ENOMEM, "t41rx_chan_create: out of memory");
+  if (!c) return SetApiError(T41RX_ENOMEM, (f + ": out of memory").c_str());
   c->device = device;
   c->n_channels = n_channels;
   c->n_receivers = n_receivers;
+  c->real = real;
   c->map.assign(n_receivers, -1);
   c->shift.assign(n_receivers, 0);
   c->p0.assign(n_receivers, 0);
@@ -361,37 +566,68 @@ int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int dev
   };
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
-    return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: stream/event creation failed"));
-  const cudaError_t attr = n_channels == 512
-      ? ChanSmemAttr(t41rx_chan_kernel<512, false>, ChanShape<512>::kSmemBytes, t41rx_chan_kernel<512, true>,
-                     ChanShape<512>::kSmemRotBytes)
-      : ChanSmemAttr(t41rx_chan_kernel<64, false>, ChanShape<64>::kSmemBytes, t41rx_chan_kernel<64, true>,
-                     ChanShape<64>::kSmemRotBytes);
+    return bail(SetApiError(T41RX_ECUDA, (f + ": stream/event creation failed").c_str()));
+  cudaError_t attr;
+  switch (n_channels) {
+    case 512:
+      attr = ChanSmemAttr(t41rx_chan_kernel<512, false>, ChanShape<512>::kSmemBytes, t41rx_chan_kernel<512, true>,
+                          ChanShape<512>::kSmemRotBytes);
+      break;
+    case 64:
+      attr = ChanSmemAttr(t41rx_chan_kernel<64, false>, ChanShape<64>::kSmemBytes, t41rx_chan_kernel<64, true>,
+                          ChanShape<64>::kSmemRotBytes);
+      break;
+    case 1024:
+      attr = ChanSmemAttr(t41rx_chan_real_kernel<1024, false>, ChanRealShape<1024>::kSmemBytes,
+                          t41rx_chan_real_kernel<1024, true>, ChanRealShape<1024>::kSmemRotBytes);
+      break;
+    default:
+      attr = ChanSmemAttr(t41rx_chan_real_kernel<128, false>, ChanRealShape<128>::kSmemBytes,
+                          t41rx_chan_real_kernel<128, true>, ChanRealShape<128>::kSmemRotBytes);
+  }
   if (attr != cudaSuccess)
-    return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: kernel image for this GPU missing (built for sm_100a)"));
+    return bail(SetApiError(T41RX_ECUDA, (f + ": kernel image for this GPU missing (built for sm_100a)").c_str()));
   const int N = kChanTaps * n_channels;
   std::vector<float> taps(N);
   DesignChanTaps(n_channels, taps.data());
+  if (real)
+    for (float &h : taps) h = ldexpf(h, -16);   /* x = s / 32768 and the split's 1 / 2, exact */
   std::vector<float2> tw(512);
   for (int k = 0; k < 512; ++k) tw[k] = float2{(float)cos(2.0 * M_PI * k / 512.0), (float)sin(2.0 * M_PI * k / 512.0)};
+  std::vector<float2> split(real ? n_channels / 2 + 1 : 0);
+  for (size_t k = 0; k < split.size(); ++k)
+    split[k] = float2{(float)cos(2.0 * M_PI * k / n_channels), (float)sin(2.0 * M_PI * k / n_channels)};
   std::vector<float2> rot(kRotCoarse + kRotFine);
   for (int a = 0; a < kRotCoarse; ++a) rot[a] = float2{(float)cos(2.0 * M_PI * a / kRotCoarse), (float)sin(2.0 * M_PI * a / kRotCoarse)};
   for (int b = 0; b < kRotFine; ++b)
     rot[kRotCoarse + b] = float2{(float)cos(2.0 * M_PI * b / kChanOutRate), (float)sin(2.0 * M_PI * b / kChanOutRate)};
+  const size_t tail_bytes = (real ? sizeof(int16_t) : sizeof(float2)) * N;
   if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * 512) != cudaSuccess ||
-      cudaMalloc(&c->d_tail, sizeof(float2) * N) != cudaSuccess ||
+      (real && cudaMalloc(&c->d_split, sizeof(float2) * split.size()) != cudaSuccess) ||
+      cudaMalloc(&c->d_tail, tail_bytes) != cudaSuccess ||
       cudaMalloc(&c->d_recv, sizeof(int32_t) * n_receivers) != cudaSuccess ||
       cudaMalloc(&c->d_chan, sizeof(int32_t) * n_receivers) != cudaSuccess ||
       cudaMalloc(&c->d_phase, sizeof(int2) * n_receivers) != cudaSuccess ||
       cudaMalloc(&c->d_rot, sizeof(float2) * rot.size()) != cudaSuccess)
-    return bail(SetApiError(T41RX_ENOMEM, "t41rx_chan_create: device allocation failed"));
+    return bail(SetApiError(T41RX_ENOMEM, (f + ": device allocation failed").c_str()));
   if (cudaMemcpy(c->d_taps, taps.data(), sizeof(float) * N, cudaMemcpyHostToDevice) != cudaSuccess ||
       cudaMemcpy(c->d_tw, tw.data(), sizeof(float2) * 512, cudaMemcpyHostToDevice) != cudaSuccess ||
+      (real && cudaMemcpy(c->d_split, split.data(), sizeof(float2) * split.size(), cudaMemcpyHostToDevice) != cudaSuccess) ||
       cudaMemcpy(c->d_rot, rot.data(), sizeof(float2) * rot.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
-      cudaMemset(c->d_tail, 0, sizeof(float2) * N) != cudaSuccess)
-    return bail(SetApiError(T41RX_ECUDA, "t41rx_chan_create: table upload failed"));
+      cudaMemset(c->d_tail, 0, tail_bytes) != cudaSuccess)
+    return bail(SetApiError(T41RX_ECUDA, (f + ": table upload failed").c_str()));
   *out = c;
   return T41RX_OK;
+}
+
+extern "C" {
+
+int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device) {
+  return ChanCreate("t41rx_chan_create", false, out, n_channels, n_receivers, device);
+}
+
+int t41rx_chan_create_real(t41rx_chan **out, int n_channels, int n_receivers, int device) {
+  return ChanCreate("t41rx_chan_create_real", true, out, n_channels, n_receivers, device);
 }
 
 }  // extern "C"
@@ -431,8 +667,9 @@ extern "C" {
 int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *channel) {
   if (!c || !channel || first < 0 || count <= 0 || first + count > c->n_receivers)
     return SetApiError(T41RX_EINVAL, "t41rx_chan_set_map: bad range");
+  const int last = c->real ? c->n_channels / 2 : c->n_channels - 1;
   for (int i = 0; i < count; ++i)
-    if (channel[i] < -1 || channel[i] >= c->n_channels)
+    if (channel[i] < -1 || channel[i] > last)
       return SetApiError(T41RX_EINVAL, "t41rx_chan_set_map: channel out of range");
   if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_set_map: cudaSetDevice failed");
   int rc = ChanQuiesce(c);
@@ -461,35 +698,71 @@ int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shi
   return ChanUpload(c, "t41rx_chan_set_shift: upload failed");
 }
 
-int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream) {
-  if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 7) || ((uintptr_t)iq & 7))
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: bad arguments (null or not 8-byte aligned pointer, n_blocks <= 0)");
+}  // extern "C"
+
+/* one call of either kind (the caller has checked the pointers): capture holds n_blocks x 2048 x D samples of
+   sample_bytes each */
+static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, size_t sample_bytes, float *iq, int n_blocks,
+                       void *cuda_stream) {
+  const std::string f(fn);
   if (n_blocks > INT_MAX / (T41RX_BLOCK_SAMPLES / kChanTile))
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: n_blocks too large for one call");
-  if (cudaSetDevice(c->device) != cudaSuccess)
-    return SetApiError(T41RX_ECUDA, "t41rx_chan_process_device: cudaSetDevice failed");
+    return SetApiError(T41RX_EINVAL, (f + ": n_blocks too large for one call").c_str());
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, (f + ": cudaSetDevice failed").c_str());
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
-  const float2 *cap = (const float2 *)capture;
   cudaError_t e = cudaSuccess;
   const int2 *phase = c->any_rotated ? c->d_phase : nullptr;
-  if (c->n_entries > 0)
-    e = c->n_channels == 512
-        ? LaunchChan<512>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
-                          c->n_entries, (float2 *)iq, n_blocks, st)
-        : LaunchChan<64>(cap, c->d_tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
-                         c->n_entries, (float2 *)iq, n_blocks, st);
+  const float2 *cap = (const float2 *)capture, *tail = (const float2 *)c->d_tail;
+  const short *cap16 = (const short *)capture, *tail16 = (const short *)c->d_tail;
+  if (c->n_entries > 0) switch (c->n_channels) {
+      case 512:
+        e = LaunchChan<512>(cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
+                            c->n_entries, (float2 *)iq, n_blocks, st);
+        break;
+      case 64:
+        e = LaunchChan<64>(cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
+                           c->n_entries, (float2 *)iq, n_blocks, st);
+        break;
+      case 1024:
+        e = LaunchChanReal<1024>(cap16, tail16, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, phase, c->d_rot,
+                                 c->m_done, c->n_entries, (float2 *)iq, n_blocks, st);
+        break;
+      default:
+        e = LaunchChanReal<128>(cap16, tail16, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, phase, c->d_rot,
+                                c->m_done, c->n_entries, (float2 *)iq, n_blocks, st);
+    }
   /* the new tail: the call's last N samples, copied after the kernel on the same stream so no tile reads it early */
   const size_t N = (size_t)kChanTaps * c->n_channels;
   const size_t total = (size_t)n_blocks * T41RX_BLOCK_SAMPLES * (c->n_channels / 2);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(c->d_tail, cap + (total - N), sizeof(float2) * N, cudaMemcpyDeviceToDevice, st);
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(c->d_tail, (const char *)capture + (total - N) * sample_bytes, sample_bytes * N,
+                        cudaMemcpyDeviceToDevice, st);
   if (e == cudaSuccess)
     c->m_done = (int)((c->m_done + (long long)n_blocks * T41RX_BLOCK_SAMPLES) % kChanOutRate);
   if (st != c->stream) {
     cudaEventRecord(c->ev_ext, st);
     c->ext_pending = true;
   }
-  if (e != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_process_device: launch failed");
+  if (e != cudaSuccess) return SetApiError(T41RX_ECUDA, (f + ": launch failed").c_str());
   return T41RX_OK;
+}
+
+extern "C" {
+
+int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream) {
+  if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 7) || ((uintptr_t)iq & 7))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: bad arguments (null or not 8-byte aligned pointer, n_blocks <= 0)");
+  if (c->real)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: a real channelizer takes t41rx_chan_process_device_real");
+  return ChanProcess("t41rx_chan_process_device", c, capture, sizeof(float2), iq, n_blocks, cuda_stream);
+}
+
+int t41rx_chan_process_device_real(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream) {
+  if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 15) || ((uintptr_t)iq & 7))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_real: bad arguments (null pointer, capture not 16-byte or "
+                                     "iq not 8-byte aligned, n_blocks <= 0)");
+  if (!c->real)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_real: a complex channelizer takes t41rx_chan_process_device");
+  return ChanProcess("t41rx_chan_process_device_real", c, capture, sizeof(int16_t), iq, n_blocks, cuda_stream);
 }
 
 int t41rx_chan_synchronize(t41rx_chan *c) {
@@ -499,33 +772,28 @@ int t41rx_chan_synchronize(t41rx_chan *c) {
 }
 
 int t41rx_chan_taps(int n_channels, float *taps) {
-  if (!taps || !ChanCountOk(n_channels)) return SetApiError(T41RX_EINVAL, "t41rx_chan_taps: bad arguments (n_channels must be 64 or 512)");
+  if (!taps || !(ChanCountOk(n_channels) || ChanRealCountOk(n_channels)))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_taps: bad arguments (n_channels must be 64, 128, 512 or 1024)");
   DesignChanTaps(n_channels, taps);
   return T41RX_OK;
 }
 
 int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *nco_freq) {
-  if (!nco_freq) return SetApiError(T41RX_EINVAL, "t41rx_chan_tune: bad arguments");
-  double f_rel = 0.0;
-  bool mirrored = false;
-  const int rc = ChanNearest("t41rx_chan_tune", n_channels, mode, offset_hz, channel, &f_rel, &mirrored);
-  if (rc) return rc;
-  *nco_freq = (int32_t)llrint(mirrored ? 48000.0 + f_rel : 48000.0 - f_rel);
-  return T41RX_OK;
+  return ChanTune("t41rx_chan_tune", false, n_channels, mode, offset_hz, channel, nco_freq);
 }
 
 int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *shift_hz,
                      int32_t *nco_freq) {
-  if (!shift_hz || !nco_freq) return SetApiError(T41RX_EINVAL, "t41rx_chan_place: bad arguments");
-  double f_rel = 0.0;
-  bool mirrored = false;
-  const int rc = ChanNearest("t41rx_chan_place", n_channels, mode, offset_hz, channel, &f_rel, &mirrored);
-  if (rc) return rc;
-  /* the signal moved from where t41rx_chan_tune's NCOFreq picks it up to NCOFreq 0: the mirrored modes see the stream
-     conjugated, so their shift has the opposite sign */
-  *shift_hz = (int32_t)llrint(mirrored ? 48000.0 + f_rel : f_rel - 48000.0);
-  *nco_freq = 0;
-  return T41RX_OK;
+  return ChanPlace("t41rx_chan_place", false, n_channels, mode, offset_hz, channel, shift_hz, nco_freq);
+}
+
+int t41rx_chan_tune_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *nco_freq) {
+  return ChanTune("t41rx_chan_tune_real", true, n_channels, mode, freq_hz, channel, nco_freq);
+}
+
+int t41rx_chan_place_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *shift_hz,
+                          int32_t *nco_freq) {
+  return ChanPlace("t41rx_chan_place_real", true, n_channels, mode, freq_hz, channel, shift_hz, nco_freq);
 }
 
 }  // extern "C"

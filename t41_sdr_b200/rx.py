@@ -90,7 +90,8 @@ EXPORTS = (
     "t41rx_multi_process_q15", "t41rx_multi_process_device", "t41rx_multi_synchronize", "t41rx_multi_gather_rows",
     "t41rx_multi_last_error", "t41rx_dc_refilter_count",
     "t41rx_chan_create", "t41rx_chan_destroy", "t41rx_chan_set_map", "t41rx_chan_process_device", "t41rx_chan_synchronize",
-    "t41rx_chan_taps", "t41rx_chan_tune", "t41rx_chan_set_shift", "t41rx_chan_place")
+    "t41rx_chan_taps", "t41rx_chan_tune", "t41rx_chan_set_shift", "t41rx_chan_place",
+    "t41rx_chan_create_real", "t41rx_chan_process_device_real", "t41rx_chan_tune_real", "t41rx_chan_place_real")
 
 CHAN_TAPS_PER_BRANCH = 10     # prototype length = 10 * n_channels
 CHAN_SPACING = 96000.0        # channel spacing (Hz); every channel comes out at 192 kS/s
@@ -170,6 +171,11 @@ def lib():
         L.t41rx_chan_taps.argtypes = [ip, C.POINTER(C.c_float)]
         L.t41rx_chan_tune.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.t41rx_chan_set_shift.argtypes = [vp, ip, ip, C.POINTER(C.c_int32)]
+        L.t41rx_chan_create_real.argtypes = [C.POINTER(vp), ip, ip, ip]
+        L.t41rx_chan_process_device_real.argtypes = [vp, vp, vp, ip, vp]
+        L.t41rx_chan_tune_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.t41rx_chan_place_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                            C.POINTER(C.c_int32)]
         L.t41rx_chan_place.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                        C.POINTER(C.c_int32)]
         _lib = L
@@ -545,17 +551,42 @@ def chan_place(n_channels, mode, offset_hz):
     return ch.value, shift.value, nco.value
 
 
+def chan_centre_real(channel):
+    """Centre of a real channelizer's channel (Hz from 0)."""
+    return channel * CHAN_SPACING
+
+
+def chan_tune_real(n_channels, mode, freq_hz):
+    """chan_tune for a real capture (n_channels 128 or 1024): freq_hz absolute, in [0, Fs/2]; host only."""
+    ch, nco = C.c_int32(), C.c_int32()
+    _check(lib().t41rx_chan_tune_real(int(n_channels), int(mode), float(freq_hz), C.byref(ch), C.byref(nco)),
+           "t41rx_chan_tune_real")
+    return ch.value, nco.value
+
+
+def chan_place_real(n_channels, mode, freq_hz):
+    """chan_place for a real capture (n_channels 128 or 1024): freq_hz absolute, in [0, Fs/2]; host only."""
+    ch, shift, nco = C.c_int32(), C.c_int32(), C.c_int32()
+    _check(lib().t41rx_chan_place_real(int(n_channels), int(mode), float(freq_hz), C.byref(ch), C.byref(shift),
+                                       C.byref(nco)), "t41rx_chan_place_real")
+    return ch.value, shift.value, nco.value
+
+
 class Channelizer:
     """Polyphase channelizer on one CUDA device: a wideband capture at n_channels x 96 kS/s in, the iq blocks of
-    n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr()."""
+    n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr().
+    real=True: an int16 real capture (n_channels 128 or 1024, channels 0 ... n_channels / 2); else complex float
+    (n_channels 64 or 512)."""
 
-    def __init__(self, n_channels, n_receivers, device=0):
+    def __init__(self, n_channels, n_receivers, device=0, real=False):
         self._h = C.c_void_p()
         self.n_channels = int(n_channels)
         self.n_receivers = int(n_receivers)
         self.device = int(device)
-        _check(lib().t41rx_chan_create(C.byref(self._h), self.n_channels, self.n_receivers, self.device),
-               "t41rx_chan_create")
+        self.real = bool(real)
+        create = lib().t41rx_chan_create_real if self.real else lib().t41rx_chan_create
+        _check(create(C.byref(self._h), self.n_channels, self.n_receivers, self.device),
+               "t41rx_chan_create_real" if self.real else "t41rx_chan_create")
 
     def close(self):
         if getattr(self, "_h", None):
@@ -588,9 +619,14 @@ class Channelizer:
                "t41rx_chan_set_shift")
 
     def process_device(self, capture_ptr, iq_ptr, n_blocks, stream=None):
-        """capture float32 [n_blocks * 2048 * n_channels / 2, 2] -> iq float32 [n_receivers, n_blocks, 2048, 2]"""
-        _check(lib().t41rx_chan_process_device(self._h, capture_ptr, iq_ptr, int(n_blocks), stream),
-               "t41rx_chan_process_device")
+        """capture float32 [n_blocks * 2048 * n_channels / 2, 2] (real: int16 [n_blocks * 2048 * n_channels / 2],
+        16-byte aligned) -> iq float32 [n_receivers, n_blocks, 2048, 2]"""
+        if self.real:
+            _check(lib().t41rx_chan_process_device_real(self._h, capture_ptr, iq_ptr, int(n_blocks), stream),
+                   "t41rx_chan_process_device_real")
+        else:
+            _check(lib().t41rx_chan_process_device(self._h, capture_ptr, iq_ptr, int(n_blocks), stream),
+                   "t41rx_chan_process_device")
 
     def synchronize(self):
         _check(lib().t41rx_chan_synchronize(self._h), "t41rx_chan_synchronize")

@@ -211,6 +211,23 @@ def wideband(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
     timed in the channel's clock: symbol k is centred at output sample symbol_offset + 6144 k + 3072 of the channel,
     as psk31() centres it in its own stream, so a receiver decodes it with the same alignment.  start_block shifts t
     (a later piece of the same capture); the noise (sigma per component) comes from seed and start_block."""
+    z = _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block)
+    out = np.empty((z.size, 2), np.float32)
+    out[:, 0] = z.real
+    out[:, 1] = z.imag
+    return out
+
+
+def wideband_real(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
+    """A real capture at n_channels x 96 kS/s (n_channels 128 or 1024) as a direct-sampling ADC delivers it: int16
+    round(32768 Re z), saturated, n_blocks * 2048 * n_channels / 2 samples.  z is the sum wideband() forms with the
+    same arguments, f measured from 0 Hz, so a ("tone", f, {amp}) is amp cos(2 pi f t)."""
+    z = _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block)
+    return np.clip(np.round(32768.0 * z.real), -32768, 32767).astype(np.int16)
+
+
+def _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block):
+    """complex128 signal sum and noise of wideband() / wideband_real()"""
     fs = wideband_rate(n_channels)
     per_block = BLOCK * n_channels // 2
     n = n_blocks * per_block
@@ -235,7 +252,4 @@ def wideband(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
             raise ValueError("unknown signal kind %r" % (kind,))
     if sigma > 0.0:
         z += _noise(np.random.Generator(np.random.PCG64([SEED_BASE + int(seed), int(start_block)])), n, sigma)
-    out = np.empty((n, 2), np.float32)
-    out[:, 0] = z.real
-    out[:, 1] = z.imag
-    return out
+    return z

@@ -1,6 +1,6 @@
 """Channelizer timing on one GPU (DESIGN §3.7): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
 
-    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--json OUT]
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--json OUT]
 
 Prints the card's name and power limit (a query), then CUDA-event times of
   - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
@@ -8,6 +8,9 @@ Prints the card's name and power limit (a query), then CUDA-event times of
   - channelize + chain on one stream,
   - with --shift, t41rx_chan_process_device again after every receiver has been given its own fine-tuning shift
     (t41rx_chan_set_shift, seeded, 0 < |shift| <= 96 kHz as t41rx_chan_place gives them), in the same run,
+  - with --real, t41rx_chan_process_device_real on a real int16 capture at M = 1024 (98.304 MS/s, the same 1024
+    receivers on channels 0 ... 511, 64 blocks: 134 MB of capture, also larger than the L2), and with --shift also
+    with every receiver shifted,
 each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
 receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
 """
@@ -53,6 +56,7 @@ def main():
     ap.add_argument("--calls", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--shift", action="store_true", help="also time the channelizer with every receiver shifted")
+    ap.add_argument("--real", action="store_true", help="also time the real M = 1024 channelizer")
     ap.add_argument("--json", default=None, help="also write the result here")
     a = ap.parse_args()
     import torch
@@ -102,12 +106,29 @@ def main():
     t_chain = timed(do_chain)
     t_both = timed(lambda: (do_chan(), do_chain()))
     t_shift = None
+    r = np.random.Generator(np.random.PCG64(2025))
+    shifts = r.integers(1, 96001, S) * r.choice([-1, 1], S)
     if a.shift:
-        r = np.random.Generator(np.random.PCG64(2025))
-        shifts = r.integers(1, 96001, S) * r.choice([-1, 1], S)
         chan.set_shift(shifts)
         t_shift = timed(do_chan)
     chan.synchronize()
+    t_real = t_real_shift = None
+    if a.real:
+        M_real = 2 * M
+        n_cap_real = T * rx.BLOCK * M_real // 2
+        capture_real = torch.randint(-3277, 3278, (n_cap_real,), generator=g, device=dev, dtype=torch.int16)
+        chan_real = rx.Channelizer(M_real, S, real=True)
+        chan_real.set_map([(r // 2) % M for r in range(S)])
+
+        def do_real():
+            chan_real.process_device(capture_real.data_ptr(), iq.data_ptr(), T, stream=sp)
+
+        t_real = timed(do_real)
+        if a.shift:
+            chan_real.set_shift(shifts)
+            t_real_shift = timed(do_real)
+        chan_real.synchronize()
+        chan_real.close()
     eng.synchronize()
     bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
     res = {
@@ -129,6 +150,17 @@ def main():
         res["chan_all_shifted_ms"] = {"median": t_shift[0], "min": t_shift[1], "max": t_shift[2]}
         res["shift_overhead"] = t_shift[0] / t_chan[0] - 1.0
         res["goal_shift_overhead_le_10pct"] = t_shift[0] <= 1.10 * t_chan[0]
+    if t_real:
+        real_bytes = n_cap_real * 2 + S * T * rx.BLOCK * 8
+        res["real"] = {"channels": M_real, "capture_msps": M_real * 96e3 / 1e6, "capture_bytes": n_cap_real * 2,
+                       "chan_ms": {"median": t_real[0], "min": t_real[1], "max": t_real[2]},
+                       "bytes_moved": real_bytes,
+                       "hbm_share_of_7p7_tbs": real_bytes / (t_real[0] * 1e-3) / HBM_BYTES_PER_S,
+                       "over_complex": t_real[0] / t_chan[0],
+                       "goal_le_1p1_of_complex": t_real[0] <= 1.10 * t_chan[0]}
+        if t_real_shift:
+            res["real"]["all_shifted_ms"] = {"median": t_real_shift[0], "min": t_real_shift[1], "max": t_real_shift[2]}
+            res["real"]["shift_overhead"] = t_real_shift[0] / t_real[0] - 1.0
     print(json.dumps(res, indent=1))
     if a.json:
         with open(a.json, "w") as f:
