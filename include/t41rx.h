@@ -313,7 +313,8 @@ int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *ch
  * iq layout, the phase rule and the ordering contract are those of the complex channelizer.
  * t41rx_chan_create_real: ENODEV without a CUDA device, EINVAL for n_channels other than 128 / 1024.
  * t41rx_chan_process_device_real: capture int16 [n_blocks * 2048 * n_channels / 2], a DEVICE pointer, 16-byte aligned;
- * iq and cuda_stream as t41rx_chan_process_device.  Each kind of channelizer rejects the other's process call (EINVAL).
+ * iq and cuda_stream as t41rx_chan_process_device.  Each kind of channelizer rejects the other kinds' process calls
+ * (EINVAL).
  * t41rx_chan_tune_real / t41rx_chan_place_real: host only, freq_hz the absolute frequency in [0, Fs_in / 2] (EINVAL
  * outside it, for NaN, for a mode t41rx_set_params rejects, for n_channels other than 128 / 1024): channel =
  * round(freq_hz / 96000), f_rel = freq_hz - channel x 96000, nco_freq and shift_hz by the rules of t41rx_chan_tune /
@@ -323,6 +324,17 @@ int t41rx_chan_process_device_real(t41rx_chan *c, const int16_t *capture, float 
 int t41rx_chan_tune_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *nco_freq);
 int t41rx_chan_place_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *shift_hz,
                           int32_t *nco_freq);
+/* Complex int16 captures (DESIGN §3.9), as wideband I/Q digitizers stream them (sc16: USRP-class, AD936x / LMS7002,
+ * SDRplay): interleaved (I, Q) int16 pairs at Fs_in = M x 96 kS/s, M = n_channels in {64, 512}.  x[n] = (I[n] + j Q[n])
+ * / 32768 (as arm_q15_to_float), then the complex channelizer unchanged: channels, fine tuning, t41rx_chan_tune /
+ * t41rx_chan_place, set_map (channels [0, M)), set_shift, synchronize, destroy, the iq layout, the n_blocks limit and
+ * the ordering contract.  The output is bit for bit that of t41rx_chan_create's channelizer fed with s / 32768 as
+ * float (exact), while the capture takes half the bytes and needs no conversion pass.
+ * t41rx_chan_create_q15: ENODEV without a CUDA device, EINVAL for n_channels other than 64 / 512.
+ * t41rx_chan_process_device_q15: capture int16 [n_blocks * 2048 * n_channels / 2][2], a DEVICE pointer, 16-byte
+ * aligned; iq and cuda_stream as t41rx_chan_process_device. */
+int t41rx_chan_create_q15(t41rx_chan **out, int n_channels, int n_receivers, int device);
+int t41rx_chan_process_device_q15(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream);
 
 /* Audio-spectrum + S-meter by-product of the row-producing blocks (Process.cpp:550-570; NFM: 791-805):
  *   audio_ypixel      int32 [n_streams][n_rows][270]  audioYPixel[k], k < AUDIO_SPEC_BOX_W - 2 (Process.cpp:34,555)

@@ -32,6 +32,10 @@
  *     X[k] = (Y[k] + conj Y[-k]) / 2 - j e^(-j 2 pi k / M) (Y[k] - conj Y[-k]) / 2,   k = 0 .. M/2, indices mod M/2;
  * the odd-m shift of u by M/2 is a shift of y by M/4.  t41rx_chan_real_kernel is the complex kernel at M/2: thread n owns
  * branches 2n and 2n + 1 (20 taps), the span is staged as int16, the split runs in the store loop.
+ *
+ * Complex int16 captures (t41rx_chan_create_q15, DESIGN §3.9): (I, Q) int16 pairs, x = (I + jQ) / 32768, M = 64 or 512.
+ * t41rx_chan_q15_kernel converts the span once as it stages it and is t41rx_chan_kernel from there on, with the 1 / 32768
+ * in the taps: the same FMAs on the same values, so the same bits as the float channelizer on s / 32768.
  */
 #include <cuda_runtime.h>
 
@@ -238,6 +242,116 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
   }
 }
 
+/* int16 -> float, exactly: 0x4B400000 + v are the bits of 1.5 x 2^23 + v (|v| < 2^22 keeps the exponent), one integer
+   add and one float subtract where a conversion instruction issues at an eighth of the FMA rate */
+__device__ __forceinline__ float ChanS16(short v) { return __int_as_float(0x4B400000 + (int)v) - 12582912.0f; }
+
+/* capture / tail: int16 (I, Q) pairs, 16-byte aligned; taps: h / 32768 (the input scale, exact); the rest as
+   t41rx_chan_kernel.  The span goes through registers (16-byte loads of four pairs) and lands converted, (I, Q) as
+   integer-valued floats, where t41rx_chan_kernel stages its float2 span: each sample is converted once, not at each of
+   the ~9 branch loads that read it, and the tile is t41rx_chan_kernel's from there on.  h / 32768 times I is h times
+   I / 32768 exactly, so every FMA, and every output bit, is that of t41rx_chan_kernel on x = s / 32768. */
+template <int M, bool kRotate>
+__global__ void __launch_bounds__(ChanShape<M>::kThreads, M == 512 ? 2 : 4)
+t41rx_chan_q15_kernel(const short *__restrict__ capture, const short *__restrict__ tail, const float *__restrict__ taps,
+                      const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
+                      const int2 *__restrict__ phase, const float2 *__restrict__ rot, int m_base, int n_entries,
+                      float2 *__restrict__ iq, int n_blocks) {
+  using S = ChanShape<M>;
+  constexpr int kQuads = S::kSpan / 4;                                  /* 16 bytes of int16 pairs each */
+  constexpr int kPerThread = (kQuads + S::kThreads - 1) / S::kThreads;
+  /* its own name for the dynamic shared memory: the float4 stores below would otherwise change what the compiler infers
+     about t41rx_chan_kernel's smem, and with it that kernel's code; 16-byte aligned for those stores */
+  extern __shared__ __align__(16) float2 smem_q15[];
+  float2 *smem = smem_q15;
+  const int tid = threadIdx.x;
+  const long long m0 = (long long)blockIdx.x * kChanTile;
+  const long long n_base = m0 * S::D - S::N;    /* capture index of smem[0]; a multiple of 4, as N is */
+
+  if (kRotate)
+    for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
+  asm volatile("cp.async.commit_group;\n" ::: "memory");
+  uint4 quad[kPerThread];
+#pragma unroll
+  for (int i = 0; i < kPerThread; ++i) {
+    const int l = tid + i * S::kThreads;
+    const long long n = n_base + 4 * l;
+    if (l < kQuads) quad[i] = __ldg(reinterpret_cast<const uint4 *>(n < 0 ? tail + 2 * (n + S::N) : capture + 2 * n));
+  }
+  auto pair = [](unsigned v) { return float2{ChanS16((short)(v & 0xFFFFu)), ChanS16((short)(v >> 16))}; };
+#pragma unroll
+  for (int i = 0; i < kPerThread; ++i) {
+    const int l = tid + i * S::kThreads;
+    if (l < kQuads) {
+      float4 *dst = reinterpret_cast<float4 *>(smem + 4 * l);
+      const float2 a = pair(quad[i].x), b = pair(quad[i].y), c = pair(quad[i].z), d = pair(quad[i].w);
+      dst[0] = float4{a.x, a.y, b.x, b.y};
+      dst[1] = float4{c.x, c.y, d.x, d.y};
+    }
+  }
+  asm volatile("cp.async.wait_group 0;\n" ::: "memory");
+
+  const int p = tid % M, g = tid / M;
+  float h[kChanTaps];
+#pragma unroll
+  for (int q = 0; q < kChanTaps; ++q) h[q] = __ldg(taps + p + q * M);
+  __syncthreads();
+
+  /* from here on t41rx_chan_kernel, statement for statement: branches (the same FMAs in the same order), rows, FFTs,
+     stores */
+  auto branch = [&](int t) {
+    const float2 *x = smem + (g + S::kGroups * t) * S::D + S::N - p;
+    float ar = 0.f, ai = 0.f;
+#pragma unroll
+    for (int q = 0; q < kChanTaps; ++q) {
+      const float2 v = x[-q * M];
+      ar = fmaf(h[q], v.x, ar);
+      ai = fmaf(h[q], v.y, ai);
+    }
+    return float2{ar, -ai};
+  };
+  auto slot = [&](int t) {
+    const int mm = g + S::kGroups * t;
+    return S::RowBase(mm) + ChanPhys<M>((mm & 1) ? (p ^ (M / 2)) : p);
+  };
+  constexpr int kLate = S::kTimes / 2;
+#pragma unroll
+  for (int t = 0; t < kLate; ++t) smem[slot(t)] = branch(t);
+  float2 u[kLate];
+#pragma unroll
+  for (int t = 0; t < kLate; ++t) u[t] = branch(kLate + t);
+  __syncthreads();
+#pragma unroll
+  for (int t = 0; t < kLate; ++t) smem[slot(kLate + t)] = u[t];
+  __syncthreads();
+
+  ChanRowsFft<M, S>(smem, tw512, tid);
+
+  const long long blk = m0 / T41RX_BLOCK_SAMPLES;
+  const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
+  if (!kRotate) {
+    for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+      const int e = w / kChanTile, mm = w % kChanTile;
+      const int k = __ldg(chan + e), r = __ldg(recv + e);
+      iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
+    }
+    return;
+  }
+  const int mm = tid % kChanTile;
+  const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
+  const float2 *tab = smem + S::kRotBase;
+#pragma unroll 4
+  for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+    const int e = w / kChanTile;
+    const int k = __ldg(chan + e), r = __ldg(recv + e);
+    const int2 sp = __ldg(phase + e);
+    const float2 v = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
+    const float2 f = ChanRotor(tab, sp, m_abs);
+    const float2 vr = float2{v.x * f.x - v.y * f.y, v.x * f.y + v.y * f.x};
+    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = (sp.x | sp.y) ? vr : v;
+  }
+}
+
 template <int M>
 struct ChanRealShape {
   static constexpr int Mc = M / 2;                              /* length of the complex FFT */
@@ -263,10 +377,6 @@ struct ChanRealShape {
   static_assert(kSpan % 8 == 0 && N % 8 == 0 && kSpanF2 % 16 == 0 && kTimes % 4 == 0, "span shape");
   static_assert((kChanTile - 1 - kEarly) * kRow + kEarly + Mc <= kSpanF2, "late rows inside the span");
 };
-
-/* int16 -> float, exactly: 0x4B400000 + v are the bits of 1.5 x 2^23 + v (|v| < 2^22 keeps the exponent), one integer
-   add and one float subtract where a conversion instruction issues at an eighth of the FMA rate */
-__device__ __forceinline__ float ChanS16(short v) { return __int_as_float(0x4B400000 + (int)v) - 12582912.0f; }
 
 /* capture / tail: int16, 16-byte aligned; taps: h / 65536 (the 1 / 32768 of the input scale and the split's 1 / 2,
    both exact); split: (cos, sin) of 2 pi k / M, k <= M / 2; the rest as t41rx_chan_kernel.  Channel k in [0, M/2]. */
@@ -382,6 +492,21 @@ static cudaError_t LaunchChan(const float2 *capture, const float2 *tail, const f
 }
 
 template <int M>
+static cudaError_t LaunchChanQ15(const short *capture, const short *tail, const float *taps, const float2 *tw,
+                                 const int32_t *recv, const int32_t *chan, const int2 *phase, const float2 *rot, int m_base,
+                                 int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
+  using S = ChanShape<M>;
+  const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
+  if (phase)
+    t41rx_chan_q15_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(capture, tail, taps, tw, recv, chan,
+                                                                                 phase, rot, m_base, n_entries, iq, n_blocks);
+  else
+    t41rx_chan_q15_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan,
+                                                                               phase, rot, m_base, n_entries, iq, n_blocks);
+  return cudaGetLastError();
+}
+
+template <int M>
 static cudaError_t LaunchChanReal(const short *capture, const short *tail, const float *taps, const float2 *tw,
                                   const float2 *split, const int32_t *recv, const int32_t *chan, const int2 *phase,
                                   const float2 *rot, int m_base, int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
@@ -485,6 +610,23 @@ static int ChanPlace(const char *fn, bool real, int n_channels, int32_t mode, do
   return T41RX_OK;
 }
 
+/* what a channelizer takes: complex float (t41rx_chan_create), real int16 (t41rx_chan_create_real, channels
+   0 .. n_channels / 2), complex int16 pairs (t41rx_chan_create_q15) */
+enum class ChanKind { kFloat, kReal, kQ15 };
+
+/* bytes of one capture sample of a kind (the tail keeps N of them) */
+static size_t ChanSampleBytes(ChanKind kind) {
+  return kind == ChanKind::kFloat ? sizeof(float2) : kind == ChanKind::kReal ? sizeof(int16_t) : 2 * sizeof(int16_t);
+}
+
+/* fn was called on a channelizer of another kind: EINVAL, naming the entry point this one takes */
+static int ChanWrongKind(const char *fn, ChanKind kind) {
+  const char *takes = kind == ChanKind::kFloat ? ": a complex float channelizer takes t41rx_chan_process_device"
+                      : kind == ChanKind::kReal ? ": a real channelizer takes t41rx_chan_process_device_real"
+                                                : ": a q15 channelizer takes t41rx_chan_process_device_q15";
+  return SetApiError(T41RX_EINVAL, (std::string(fn) + takes).c_str());
+}
+
 }  // namespace t41rx
 
 using namespace t41rx;
@@ -493,13 +635,13 @@ struct t41rx_chan {
   int device = 0;
   int n_channels = 0;
   int n_receivers = 0;
-  bool real = false;             /* int16 real capture (t41rx_chan_create_real): channels 0 .. n_channels / 2 */
+  ChanKind kind = ChanKind::kFloat;
   cudaStream_t stream = nullptr;
   /* t41rx_chan_process_device may enqueue on a caller-supplied stream: its end is recorded here, and set_map /
      synchronize / destroy wait for it (the ordering contract of t41rx_process_device) */
   cudaEvent_t ev_ext = nullptr;
   bool ext_pending = false;
-  float *d_taps = nullptr;       /* N (real: h / 65536) */
+  float *d_taps = nullptr;       /* N (real: h / 65536, q15: h / 32768) */
   float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512 */
   float2 *d_split = nullptr;     /* real: n_channels / 2 + 1 (cos, sin) of 2 pi k / n_channels */
   void *d_tail = nullptr;        /* the last N capture samples of the previous calls (zeros at creation) */
@@ -539,9 +681,10 @@ void t41rx_chan_destroy(t41rx_chan *c) {
 
 }  // extern "C"
 
-/* t41rx_chan_create / _create_real; fn names the entry point in error messages */
-static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channels, int n_receivers, int device) {
+/* t41rx_chan_create / _create_real / _create_q15; fn names the entry point in error messages */
+static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_channels, int n_receivers, int device) {
   const std::string f(fn);
+  const bool real = kind == ChanKind::kReal;
   if (!out || !(real ? ChanRealCountOk(n_channels) : ChanCountOk(n_channels)) || n_receivers <= 0)
     return SetApiError(T41RX_EINVAL, (f + (real ? ": bad arguments (n_channels must be 128 or 1024)"
                                                : ": bad arguments (n_channels must be 64 or 512)")).c_str());
@@ -556,7 +699,7 @@ static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channel
   c->device = device;
   c->n_channels = n_channels;
   c->n_receivers = n_receivers;
-  c->real = real;
+  c->kind = kind;
   c->map.assign(n_receivers, -1);
   c->shift.assign(n_receivers, 0);
   c->p0.assign(n_receivers, 0);
@@ -568,7 +711,12 @@ static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channel
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": stream/event creation failed").c_str()));
   cudaError_t attr;
-  switch (n_channels) {
+  if (kind == ChanKind::kQ15)
+    attr = n_channels == 512 ? ChanSmemAttr(t41rx_chan_q15_kernel<512, false>, ChanShape<512>::kSmemBytes,
+                                            t41rx_chan_q15_kernel<512, true>, ChanShape<512>::kSmemRotBytes)
+                             : ChanSmemAttr(t41rx_chan_q15_kernel<64, false>, ChanShape<64>::kSmemBytes,
+                                            t41rx_chan_q15_kernel<64, true>, ChanShape<64>::kSmemRotBytes);
+  else switch (n_channels) {
     case 512:
       attr = ChanSmemAttr(t41rx_chan_kernel<512, false>, ChanShape<512>::kSmemBytes, t41rx_chan_kernel<512, true>,
                           ChanShape<512>::kSmemRotBytes);
@@ -592,6 +740,8 @@ static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channel
   DesignChanTaps(n_channels, taps.data());
   if (real)
     for (float &h : taps) h = ldexpf(h, -16);   /* x = s / 32768 and the split's 1 / 2, exact */
+  if (kind == ChanKind::kQ15)
+    for (float &h : taps) h = ldexpf(h, -15);   /* x = s / 32768, exact */
   std::vector<float2> tw(512);
   for (int k = 0; k < 512; ++k) tw[k] = float2{(float)cos(2.0 * M_PI * k / 512.0), (float)sin(2.0 * M_PI * k / 512.0)};
   std::vector<float2> split(real ? n_channels / 2 + 1 : 0);
@@ -601,7 +751,7 @@ static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channel
   for (int a = 0; a < kRotCoarse; ++a) rot[a] = float2{(float)cos(2.0 * M_PI * a / kRotCoarse), (float)sin(2.0 * M_PI * a / kRotCoarse)};
   for (int b = 0; b < kRotFine; ++b)
     rot[kRotCoarse + b] = float2{(float)cos(2.0 * M_PI * b / kChanOutRate), (float)sin(2.0 * M_PI * b / kChanOutRate)};
-  const size_t tail_bytes = (real ? sizeof(int16_t) : sizeof(float2)) * N;
+  const size_t tail_bytes = ChanSampleBytes(kind) * N;
   if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * 512) != cudaSuccess ||
       (real && cudaMalloc(&c->d_split, sizeof(float2) * split.size()) != cudaSuccess) ||
       cudaMalloc(&c->d_tail, tail_bytes) != cudaSuccess ||
@@ -623,11 +773,15 @@ static int ChanCreate(const char *fn, bool real, t41rx_chan **out, int n_channel
 extern "C" {
 
 int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device) {
-  return ChanCreate("t41rx_chan_create", false, out, n_channels, n_receivers, device);
+  return ChanCreate("t41rx_chan_create", ChanKind::kFloat, out, n_channels, n_receivers, device);
 }
 
 int t41rx_chan_create_real(t41rx_chan **out, int n_channels, int n_receivers, int device) {
-  return ChanCreate("t41rx_chan_create_real", true, out, n_channels, n_receivers, device);
+  return ChanCreate("t41rx_chan_create_real", ChanKind::kReal, out, n_channels, n_receivers, device);
+}
+
+int t41rx_chan_create_q15(t41rx_chan **out, int n_channels, int n_receivers, int device) {
+  return ChanCreate("t41rx_chan_create_q15", ChanKind::kQ15, out, n_channels, n_receivers, device);
 }
 
 }  // extern "C"
@@ -667,7 +821,7 @@ extern "C" {
 int t41rx_chan_set_map(t41rx_chan *c, int first, int count, const int32_t *channel) {
   if (!c || !channel || first < 0 || count <= 0 || first + count > c->n_receivers)
     return SetApiError(T41RX_EINVAL, "t41rx_chan_set_map: bad range");
-  const int last = c->real ? c->n_channels / 2 : c->n_channels - 1;
+  const int last = c->kind == ChanKind::kReal ? c->n_channels / 2 : c->n_channels - 1;
   for (int i = 0; i < count; ++i)
     if (channel[i] < -1 || channel[i] > last)
       return SetApiError(T41RX_EINVAL, "t41rx_chan_set_map: channel out of range");
@@ -700,10 +854,9 @@ int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shi
 
 }  // extern "C"
 
-/* one call of either kind (the caller has checked the pointers): capture holds n_blocks x 2048 x D samples of
-   sample_bytes each */
-static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, size_t sample_bytes, float *iq, int n_blocks,
-                       void *cuda_stream) {
+/* one call of any kind (the caller has checked the pointers and the kind): capture holds n_blocks x 2048 x D samples
+   of ChanSampleBytes(c->kind) each */
+static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, float *iq, int n_blocks, void *cuda_stream) {
   const std::string f(fn);
   if (n_blocks > INT_MAX / (T41RX_BLOCK_SAMPLES / kChanTile))
     return SetApiError(T41RX_EINVAL, (f + ": n_blocks too large for one call").c_str());
@@ -713,7 +866,13 @@ static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, size_
   const int2 *phase = c->any_rotated ? c->d_phase : nullptr;
   const float2 *cap = (const float2 *)capture, *tail = (const float2 *)c->d_tail;
   const short *cap16 = (const short *)capture, *tail16 = (const short *)c->d_tail;
-  if (c->n_entries > 0) switch (c->n_channels) {
+  if (c->n_entries > 0 && c->kind == ChanKind::kQ15)
+    e = c->n_channels == 512
+            ? LaunchChanQ15<512>(cap16, tail16, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
+                                 c->n_entries, (float2 *)iq, n_blocks, st)
+            : LaunchChanQ15<64>(cap16, tail16, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
+                                c->n_entries, (float2 *)iq, n_blocks, st);
+  else if (c->n_entries > 0) switch (c->n_channels) {
       case 512:
         e = LaunchChan<512>(cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
                             c->n_entries, (float2 *)iq, n_blocks, st);
@@ -733,6 +892,7 @@ static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, size_
   /* the new tail: the call's last N samples, copied after the kernel on the same stream so no tile reads it early */
   const size_t N = (size_t)kChanTaps * c->n_channels;
   const size_t total = (size_t)n_blocks * T41RX_BLOCK_SAMPLES * (c->n_channels / 2);
+  const size_t sample_bytes = ChanSampleBytes(c->kind);
   if (e == cudaSuccess)
     e = cudaMemcpyAsync(c->d_tail, (const char *)capture + (total - N) * sample_bytes, sample_bytes * N,
                         cudaMemcpyDeviceToDevice, st);
@@ -751,18 +911,24 @@ extern "C" {
 int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream) {
   if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 7) || ((uintptr_t)iq & 7))
     return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: bad arguments (null or not 8-byte aligned pointer, n_blocks <= 0)");
-  if (c->real)
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: a real channelizer takes t41rx_chan_process_device_real");
-  return ChanProcess("t41rx_chan_process_device", c, capture, sizeof(float2), iq, n_blocks, cuda_stream);
+  if (c->kind != ChanKind::kFloat) return ChanWrongKind("t41rx_chan_process_device", c->kind);
+  return ChanProcess("t41rx_chan_process_device", c, capture, iq, n_blocks, cuda_stream);
 }
 
 int t41rx_chan_process_device_real(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream) {
   if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 15) || ((uintptr_t)iq & 7))
     return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_real: bad arguments (null pointer, capture not 16-byte or "
                                      "iq not 8-byte aligned, n_blocks <= 0)");
-  if (!c->real)
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_real: a complex channelizer takes t41rx_chan_process_device");
-  return ChanProcess("t41rx_chan_process_device_real", c, capture, sizeof(int16_t), iq, n_blocks, cuda_stream);
+  if (c->kind != ChanKind::kReal) return ChanWrongKind("t41rx_chan_process_device_real", c->kind);
+  return ChanProcess("t41rx_chan_process_device_real", c, capture, iq, n_blocks, cuda_stream);
+}
+
+int t41rx_chan_process_device_q15(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream) {
+  if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 15) || ((uintptr_t)iq & 7))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_q15: bad arguments (null pointer, capture not 16-byte or "
+                                     "iq not 8-byte aligned, n_blocks <= 0)");
+  if (c->kind != ChanKind::kQ15) return ChanWrongKind("t41rx_chan_process_device_q15", c->kind);
+  return ChanProcess("t41rx_chan_process_device_q15", c, capture, iq, n_blocks, cuda_stream);
 }
 
 int t41rx_chan_synchronize(t41rx_chan *c) {

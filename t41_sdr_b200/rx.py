@@ -91,7 +91,8 @@ EXPORTS = (
     "t41rx_multi_last_error", "t41rx_dc_refilter_count",
     "t41rx_chan_create", "t41rx_chan_destroy", "t41rx_chan_set_map", "t41rx_chan_process_device", "t41rx_chan_synchronize",
     "t41rx_chan_taps", "t41rx_chan_tune", "t41rx_chan_set_shift", "t41rx_chan_place",
-    "t41rx_chan_create_real", "t41rx_chan_process_device_real", "t41rx_chan_tune_real", "t41rx_chan_place_real")
+    "t41rx_chan_create_real", "t41rx_chan_process_device_real", "t41rx_chan_tune_real", "t41rx_chan_place_real",
+    "t41rx_chan_create_q15", "t41rx_chan_process_device_q15")
 
 CHAN_TAPS_PER_BRANCH = 10     # prototype length = 10 * n_channels
 CHAN_SPACING = 96000.0        # channel spacing (Hz); every channel comes out at 192 kS/s
@@ -173,6 +174,8 @@ def lib():
         L.t41rx_chan_set_shift.argtypes = [vp, ip, ip, C.POINTER(C.c_int32)]
         L.t41rx_chan_create_real.argtypes = [C.POINTER(vp), ip, ip, ip]
         L.t41rx_chan_process_device_real.argtypes = [vp, vp, vp, ip, vp]
+        L.t41rx_chan_create_q15.argtypes = [C.POINTER(vp), ip, ip, ip]
+        L.t41rx_chan_process_device_q15.argtypes = [vp, vp, vp, ip, vp]
         L.t41rx_chan_tune_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.t41rx_chan_place_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                             C.POINTER(C.c_int32)]
@@ -575,18 +578,24 @@ def chan_place_real(n_channels, mode, freq_hz):
 class Channelizer:
     """Polyphase channelizer on one CUDA device: a wideband capture at n_channels x 96 kS/s in, the iq blocks of
     n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr().
-    real=True: an int16 real capture (n_channels 128 or 1024, channels 0 ... n_channels / 2); else complex float
+    real=True: an int16 real capture (n_channels 128 or 1024, channels 0 ... n_channels / 2); q15=True: a complex
+    capture of interleaved int16 (I, Q) pairs, x = (I + jQ) / 32768 (n_channels 64 or 512); else complex float
     (n_channels 64 or 512)."""
 
-    def __init__(self, n_channels, n_receivers, device=0, real=False):
+    def __init__(self, n_channels, n_receivers, device=0, real=False, q15=False):
+        if real and q15:
+            raise ValueError("Channelizer: real and q15 are different capture kinds; pass at most one")
         self._h = C.c_void_p()
         self.n_channels = int(n_channels)
         self.n_receivers = int(n_receivers)
         self.device = int(device)
         self.real = bool(real)
-        create = lib().t41rx_chan_create_real if self.real else lib().t41rx_chan_create
-        _check(create(C.byref(self._h), self.n_channels, self.n_receivers, self.device),
-               "t41rx_chan_create_real" if self.real else "t41rx_chan_create")
+        self.q15 = bool(q15)
+        self._create, self._process = (("t41rx_chan_create_real", "t41rx_chan_process_device_real") if self.real else
+                                       ("t41rx_chan_create_q15", "t41rx_chan_process_device_q15") if self.q15 else
+                                       ("t41rx_chan_create", "t41rx_chan_process_device"))
+        _check(getattr(lib(), self._create)(C.byref(self._h), self.n_channels, self.n_receivers, self.device),
+               self._create)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -619,14 +628,10 @@ class Channelizer:
                "t41rx_chan_set_shift")
 
     def process_device(self, capture_ptr, iq_ptr, n_blocks, stream=None):
-        """capture float32 [n_blocks * 2048 * n_channels / 2, 2] (real: int16 [n_blocks * 2048 * n_channels / 2],
-        16-byte aligned) -> iq float32 [n_receivers, n_blocks, 2048, 2]"""
-        if self.real:
-            _check(lib().t41rx_chan_process_device_real(self._h, capture_ptr, iq_ptr, int(n_blocks), stream),
-                   "t41rx_chan_process_device_real")
-        else:
-            _check(lib().t41rx_chan_process_device(self._h, capture_ptr, iq_ptr, int(n_blocks), stream),
-                   "t41rx_chan_process_device")
+        """capture float32 [n_blocks * 2048 * n_channels / 2, 2] (real: int16 [n_blocks * 2048 * n_channels / 2];
+        q15: int16 [n_blocks * 2048 * n_channels / 2, 2]; both 16-byte aligned) -> iq float32 [n_receivers, n_blocks,
+        2048, 2]"""
+        _check(getattr(lib(), self._process)(self._h, capture_ptr, iq_ptr, int(n_blocks), stream), self._process)
 
     def synchronize(self):
         _check(lib().t41rx_chan_synchronize(self._h), "t41rx_chan_synchronize")

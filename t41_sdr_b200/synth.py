@@ -226,8 +226,19 @@ def wideband_real(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0)
     return np.clip(np.round(32768.0 * z.real), -32768, 32767).astype(np.int16)
 
 
+def wideband_q15(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
+    """A complex capture at n_channels x 96 kS/s (n_channels 64 or 512) as a wideband I/Q digitizer streams it (sc16):
+    int16 [n, 2] interleaved (I, Q), round(32768 z) saturated to [-32768, 32767] per component.  z is the sum
+    wideband() forms with the same arguments, so wideband_q15 / 32768 is wideband() quantised."""
+    z = _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block)
+    out = np.empty((z.size, 2), np.int16)
+    out[:, 0] = np.clip(np.round(32768.0 * z.real), -32768, 32767)
+    out[:, 1] = np.clip(np.round(32768.0 * z.imag), -32768, 32767)
+    return out
+
+
 def _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block):
-    """complex128 signal sum and noise of wideband() / wideband_real()"""
+    """complex128 signal sum and noise of wideband() / wideband_real() / wideband_q15()"""
     fs = wideband_rate(n_channels)
     per_block = BLOCK * n_channels // 2
     n = n_blocks * per_block

@@ -1,6 +1,6 @@
-"""Channelizer timing on one GPU (DESIGN §3.7): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
+"""Channelizer timing on one GPU (DESIGN §3.7 - 3.9): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
 
-    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--json OUT]
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--json OUT]
 
 Prints the card's name and power limit (a query), then CUDA-event times of
   - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
@@ -11,6 +11,9 @@ Prints the card's name and power limit (a query), then CUDA-event times of
   - with --real, t41rx_chan_process_device_real on a real int16 capture at M = 1024 (98.304 MS/s, the same 1024
     receivers on channels 0 ... 511, 64 blocks: 134 MB of capture, also larger than the L2), and with --shift also
     with every receiver shifted,
+  - with --q15, at the same M and 1024 receivers: t41rx_chan_process_device_q15 on an interleaved int16 capture (134 MB
+    at M = 512), and what a user of the float call does with such a capture: int16 -> float32 / 32768 with torch into
+    a float capture, then t41rx_chan_process_device (with --shift also the q15 call with every receiver shifted),
 each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
 receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
 """
@@ -57,6 +60,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--shift", action="store_true", help="also time the channelizer with every receiver shifted")
     ap.add_argument("--real", action="store_true", help="also time the real M = 1024 channelizer")
+    ap.add_argument("--q15", action="store_true", help="also time the q15 channelizer and torch conversion + float")
     ap.add_argument("--json", default=None, help="also write the result here")
     a = ap.parse_args()
     import torch
@@ -129,6 +133,31 @@ def main():
             t_real_shift = timed(do_real)
         chan_real.synchronize()
         chan_real.close()
+    t_q15 = t_q15_shift = t_conv = None
+    if a.q15:
+        capture_q15 = torch.randint(-3277, 3278, (n_cap, 2), generator=g, device=dev, dtype=torch.int16)
+        capture_conv = torch.empty((n_cap, 2), dtype=torch.float32, device=dev)
+        chan_q15 = rx.Channelizer(M, S, q15=True)
+        chan_q15.set_map([(r // 2) % M for r in range(S)])
+        chan_conv = rx.Channelizer(M, S)
+        chan_conv.set_map([(r // 2) % M for r in range(S)])
+
+        def do_q15():
+            chan_q15.process_device(capture_q15.data_ptr(), iq.data_ptr(), T, stream=sp)
+
+        def do_conv():
+            with torch.cuda.stream(stream):
+                torch.mul(capture_q15, 1.0 / 32768.0, out=capture_conv)
+            chan_conv.process_device(capture_conv.data_ptr(), iq.data_ptr(), T, stream=sp)
+
+        t_q15 = timed(do_q15)
+        t_conv = timed(do_conv)
+        if a.shift:
+            chan_q15.set_shift(shifts)
+            t_q15_shift = timed(do_q15)
+        for c in (chan_q15, chan_conv):
+            c.synchronize()
+            c.close()
     eng.synchronize()
     bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
     res = {
@@ -161,6 +190,22 @@ def main():
         if t_real_shift:
             res["real"]["all_shifted_ms"] = {"median": t_real_shift[0], "min": t_real_shift[1], "max": t_real_shift[2]}
             res["real"]["shift_overhead"] = t_real_shift[0] / t_real[0] - 1.0
+    if t_q15:
+        iq_bytes = S * T * rx.BLOCK * 8
+        q15_bytes = n_cap * 4 + iq_bytes
+        conv_bytes = n_cap * 4 + n_cap * 8 + bytes_moved     # int16 read, float written, then the float call
+        res["q15"] = {"capture_bytes": n_cap * 4,
+                      "chan_ms": {"median": t_q15[0], "min": t_q15[1], "max": t_q15[2]},
+                      "bytes_moved": q15_bytes,
+                      "hbm_share_of_7p7_tbs": q15_bytes / (t_q15[0] * 1e-3) / HBM_BYTES_PER_S,
+                      "over_float": t_q15[0] / t_chan[0],
+                      "goal_le_float": t_q15[0] <= t_chan[0],
+                      "convert_plus_float_ms": {"median": t_conv[0], "min": t_conv[1], "max": t_conv[2]},
+                      "convert_plus_float_bytes_moved": conv_bytes,
+                      "convert_plus_float_hbm_share_of_7p7_tbs": conv_bytes / (t_conv[0] * 1e-3) / HBM_BYTES_PER_S}
+        if t_q15_shift:
+            res["q15"]["all_shifted_ms"] = {"median": t_q15_shift[0], "min": t_q15_shift[1], "max": t_q15_shift[2]}
+            res["q15"]["shift_overhead"] = t_q15_shift[0] / t_q15[0] - 1.0
     print(json.dumps(res, indent=1))
     if a.json:
         with open(a.json, "w") as f:
