@@ -34,8 +34,9 @@
  * branches 2n and 2n + 1 (20 taps), the span is staged as int16, the split runs in the store loop.
  *
  * Complex int16 captures (t41rx_chan_create_q15, DESIGN §3.9): (I, Q) int16 pairs, x = (I + jQ) / 32768, M = 64 or 512.
- * t41rx_chan_q15_kernel converts the span once as it stages it and is t41rx_chan_kernel from there on, with the 1 / 32768
- * in the taps: the same FMAs on the same values, so the same bits as the float channelizer on s / 32768.
+ * t41rx_chan_kernel<M, kRotate, short> converts the span once as it stages it; the rest of the kernel is the float
+ * instance's, with the 1 / 32768 in the taps: the same FMAs on the same values, so the same bits as the float
+ * channelizer on s / 32768.
  */
 #include <cuda_runtime.h>
 
@@ -44,6 +45,7 @@
 #include <cmath>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/t41rx.h"
@@ -152,29 +154,78 @@ __device__ __forceinline__ void ChanRowsFft(float2 *smem, const float2 *tw512, i
   }
 }
 
-/* capture: the call's samples; tail: the N samples before them; recv / chan: the mapped receivers grouped by channel
-   (CSR order) and the channel of each; phase: each entry's (shift, P) in [0, 192000), or null when no entry is
+/* int16 -> float, exactly: 0x4B400000 + v are the bits of 1.5 x 2^23 + v (|v| < 2^22 keeps the exponent), one integer
+   add and one float subtract where a conversion instruction issues at an eighth of the FMA rate */
+__device__ __forceinline__ float ChanS16(short v) { return __int_as_float(0x4B400000 + (int)v) - 12582912.0f; }
+
+/* t41rx_chan_kernel's dynamic shared memory.  The q15 instances have their own name for it: their float4 stores would
+   otherwise change what the compiler infers about the float instances' smem, and with it their code; 16-byte aligned
+   for those stores */
+template <typename T> __device__ __forceinline__ float2 *ChanSmem();
+template <> __device__ __forceinline__ float2 *ChanSmem<float2>() {
+  extern __shared__ float2 smem[];
+  return smem;
+}
+template <> __device__ __forceinline__ float2 *ChanSmem<short>() {
+  extern __shared__ __align__(16) float2 smem_q15[];
+  return smem_q15;
+}
+
+/* capture: the call's samples; tail: the N samples before them; T = float2 (complex float) or short (int16 (I, Q)
+   pairs, 16-byte aligned, with h / 32768 in taps: the input scale, exact); recv / chan: the mapped receivers grouped by
+   channel (CSR order) and the channel of each; phase: each entry's (shift, P) in [0, 192000), or null when no entry is
    rotated; rot: the 480 + 400 factors of the rotation table; m_base: outputs before this call, mod 192000;
-   iq: [n_receivers][n_blocks][2048].  kRotate = false (no entry rotated) is the kernel without fine tuning. */
-template <int M, bool kRotate>
+   iq: [n_receivers][n_blocks][2048].  kRotate = false (no entry rotated) is the kernel without fine tuning.
+   The int16 span goes through registers (16-byte loads of four pairs) and lands converted, (I, Q) as integer-valued
+   floats, where the float span is staged: each sample is converted once, not at each of the ~9 branch loads that read
+   it, and the rest of the kernel is the same for both.  h / 32768 times I is h times I / 32768 exactly, so every FMA,
+   and every output bit, is that of the float instance on x = s / 32768. */
+template <int M, bool kRotate, typename T>
 __global__ void __launch_bounds__(ChanShape<M>::kThreads, M == 512 ? 2 : 4)
-t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__ tail, const float *__restrict__ taps,
+t41rx_chan_kernel(const T *__restrict__ capture, const T *__restrict__ tail, const float *__restrict__ taps,
                   const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
                   const int2 *__restrict__ phase, const float2 *__restrict__ rot, int m_base, int n_entries,
                   float2 *__restrict__ iq, int n_blocks) {
   using S = ChanShape<M>;
-  extern __shared__ float2 smem[];
+  float2 *smem = ChanSmem<T>();
   const int tid = threadIdx.x;
   const long long m0 = (long long)blockIdx.x * kChanTile;
-  const long long n_base = m0 * S::D - S::N;    /* capture index of smem[0] */
+  const long long n_base = m0 * S::D - S::N;    /* capture index of smem[0]; a multiple of 4, as N is */
 
-  for (int l = tid; l < S::kSpan; l += S::kThreads) {
-    const long long n = n_base + l;
-    CpAsync8(smem + l, n < 0 ? tail + (n + S::N) : capture + n);
+  if constexpr (std::is_same_v<T, float2>) {
+    for (int l = tid; l < S::kSpan; l += S::kThreads) {
+      const long long n = n_base + l;
+      CpAsync8(smem + l, n < 0 ? tail + (n + S::N) : capture + n);
+    }
+    if (kRotate)
+      for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
+    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
+  } else {
+    constexpr int kQuads = S::kSpan / 4;                                  /* 16 bytes of int16 pairs each */
+    constexpr int kPerThread = (kQuads + S::kThreads - 1) / S::kThreads;
+    if (kRotate)
+      for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
+    asm volatile("cp.async.commit_group;\n" ::: "memory");
+    uint4 quad[kPerThread];
+#pragma unroll
+    for (int i = 0; i < kPerThread; ++i) {
+      const int l = tid + i * S::kThreads;
+      const long long n = n_base + 4 * l;
+      if (l < kQuads) quad[i] = __ldg(reinterpret_cast<const uint4 *>(n < 0 ? tail + 2 * (n + S::N) : capture + 2 * n));
+    }
+    auto pair = [](unsigned v) { return float2{ChanS16((short)(v & 0xFFFFu)), ChanS16((short)(v >> 16))}; };
+#pragma unroll
+    for (int i = 0; i < kPerThread; ++i) {
+      const int l = tid + i * S::kThreads;
+      if (l < kQuads) {
+        float4 *dst = reinterpret_cast<float4 *>(smem + 4 * l);
+        const float2 a = pair(quad[i].x), b = pair(quad[i].y), c = pair(quad[i].z), d = pair(quad[i].w);
+        dst[0] = float4{a.x, a.y, b.x, b.y};
+        dst[1] = float4{c.x, c.y, d.x, d.y};
+      }
+    }
+    asm volatile("cp.async.wait_group 0;\n" ::: "memory");
   }
-  if (kRotate)
-    for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
-  asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
 
   const int p = tid % M, g = tid / M;
   float h[kChanTaps];
@@ -214,7 +265,9 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
 
   ChanRowsFft<M, S>(smem, tw512, tid);
 
-  /* each receiver's run: kChanTile consecutive samples inside one block (the tile size divides 2048) */
+  /* each receiver's run: kChanTile consecutive samples inside one block (the tile size divides 2048).  The store loops
+     are written out here and again in t41rx_chan_real_kernel: as one __device__ function taking the sample as a lambda
+     they compile to different (longer) code in every instance of this kernel. */
   const long long blk = m0 / T41RX_BLOCK_SAMPLES;
   const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
   if (!kRotate) {
@@ -227,116 +280,6 @@ t41rx_chan_kernel(const float2 *__restrict__ capture, const float2 *__restrict__
   }
   /* a thread always stores the same sample mm of the tile (kThreads is a multiple of kChanTile): its m_abs mod 192000.
      The body has no branch (an entry with phase 0 selects the sample unmultiplied), so unrolled iterations overlap. */
-  const int mm = tid % kChanTile;
-  const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
-  const float2 *tab = smem + S::kRotBase;
-#pragma unroll 4
-  for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
-    const int e = w / kChanTile;
-    const int k = __ldg(chan + e), r = __ldg(recv + e);
-    const int2 sp = __ldg(phase + e);
-    const float2 v = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
-    const float2 f = ChanRotor(tab, sp, m_abs);
-    const float2 vr = float2{v.x * f.x - v.y * f.y, v.x * f.y + v.y * f.x};
-    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = (sp.x | sp.y) ? vr : v;
-  }
-}
-
-/* int16 -> float, exactly: 0x4B400000 + v are the bits of 1.5 x 2^23 + v (|v| < 2^22 keeps the exponent), one integer
-   add and one float subtract where a conversion instruction issues at an eighth of the FMA rate */
-__device__ __forceinline__ float ChanS16(short v) { return __int_as_float(0x4B400000 + (int)v) - 12582912.0f; }
-
-/* capture / tail: int16 (I, Q) pairs, 16-byte aligned; taps: h / 32768 (the input scale, exact); the rest as
-   t41rx_chan_kernel.  The span goes through registers (16-byte loads of four pairs) and lands converted, (I, Q) as
-   integer-valued floats, where t41rx_chan_kernel stages its float2 span: each sample is converted once, not at each of
-   the ~9 branch loads that read it, and the tile is t41rx_chan_kernel's from there on.  h / 32768 times I is h times
-   I / 32768 exactly, so every FMA, and every output bit, is that of t41rx_chan_kernel on x = s / 32768. */
-template <int M, bool kRotate>
-__global__ void __launch_bounds__(ChanShape<M>::kThreads, M == 512 ? 2 : 4)
-t41rx_chan_q15_kernel(const short *__restrict__ capture, const short *__restrict__ tail, const float *__restrict__ taps,
-                      const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
-                      const int2 *__restrict__ phase, const float2 *__restrict__ rot, int m_base, int n_entries,
-                      float2 *__restrict__ iq, int n_blocks) {
-  using S = ChanShape<M>;
-  constexpr int kQuads = S::kSpan / 4;                                  /* 16 bytes of int16 pairs each */
-  constexpr int kPerThread = (kQuads + S::kThreads - 1) / S::kThreads;
-  /* its own name for the dynamic shared memory: the float4 stores below would otherwise change what the compiler infers
-     about t41rx_chan_kernel's smem, and with it that kernel's code; 16-byte aligned for those stores */
-  extern __shared__ __align__(16) float2 smem_q15[];
-  float2 *smem = smem_q15;
-  const int tid = threadIdx.x;
-  const long long m0 = (long long)blockIdx.x * kChanTile;
-  const long long n_base = m0 * S::D - S::N;    /* capture index of smem[0]; a multiple of 4, as N is */
-
-  if (kRotate)
-    for (int l = tid; l < kRotCoarse + kRotFine; l += S::kThreads) CpAsync8(smem + S::kRotBase + l, rot + l);
-  asm volatile("cp.async.commit_group;\n" ::: "memory");
-  uint4 quad[kPerThread];
-#pragma unroll
-  for (int i = 0; i < kPerThread; ++i) {
-    const int l = tid + i * S::kThreads;
-    const long long n = n_base + 4 * l;
-    if (l < kQuads) quad[i] = __ldg(reinterpret_cast<const uint4 *>(n < 0 ? tail + 2 * (n + S::N) : capture + 2 * n));
-  }
-  auto pair = [](unsigned v) { return float2{ChanS16((short)(v & 0xFFFFu)), ChanS16((short)(v >> 16))}; };
-#pragma unroll
-  for (int i = 0; i < kPerThread; ++i) {
-    const int l = tid + i * S::kThreads;
-    if (l < kQuads) {
-      float4 *dst = reinterpret_cast<float4 *>(smem + 4 * l);
-      const float2 a = pair(quad[i].x), b = pair(quad[i].y), c = pair(quad[i].z), d = pair(quad[i].w);
-      dst[0] = float4{a.x, a.y, b.x, b.y};
-      dst[1] = float4{c.x, c.y, d.x, d.y};
-    }
-  }
-  asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-
-  const int p = tid % M, g = tid / M;
-  float h[kChanTaps];
-#pragma unroll
-  for (int q = 0; q < kChanTaps; ++q) h[q] = __ldg(taps + p + q * M);
-  __syncthreads();
-
-  /* from here on t41rx_chan_kernel, statement for statement: branches (the same FMAs in the same order), rows, FFTs,
-     stores */
-  auto branch = [&](int t) {
-    const float2 *x = smem + (g + S::kGroups * t) * S::D + S::N - p;
-    float ar = 0.f, ai = 0.f;
-#pragma unroll
-    for (int q = 0; q < kChanTaps; ++q) {
-      const float2 v = x[-q * M];
-      ar = fmaf(h[q], v.x, ar);
-      ai = fmaf(h[q], v.y, ai);
-    }
-    return float2{ar, -ai};
-  };
-  auto slot = [&](int t) {
-    const int mm = g + S::kGroups * t;
-    return S::RowBase(mm) + ChanPhys<M>((mm & 1) ? (p ^ (M / 2)) : p);
-  };
-  constexpr int kLate = S::kTimes / 2;
-#pragma unroll
-  for (int t = 0; t < kLate; ++t) smem[slot(t)] = branch(t);
-  float2 u[kLate];
-#pragma unroll
-  for (int t = 0; t < kLate; ++t) u[t] = branch(kLate + t);
-  __syncthreads();
-#pragma unroll
-  for (int t = 0; t < kLate; ++t) smem[slot(kLate + t)] = u[t];
-  __syncthreads();
-
-  ChanRowsFft<M, S>(smem, tw512, tid);
-
-  const long long blk = m0 / T41RX_BLOCK_SAMPLES;
-  const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
-  if (!kRotate) {
-    for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
-      const int e = w / kChanTile, mm = w % kChanTile;
-      const int k = __ldg(chan + e), r = __ldg(recv + e);
-      iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = smem[S::RowBase(mm) + ChanOutPos<M>(k)];
-    }
-    return;
-  }
   const int mm = tid % kChanTile;
   const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
   const float2 *tab = smem + S::kRotBase;
@@ -476,51 +419,6 @@ t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restric
   }
 }
 
-template <int M>
-static cudaError_t LaunchChan(const float2 *capture, const float2 *tail, const float *taps, const float2 *tw,
-                              const int32_t *recv, const int32_t *chan, const int2 *phase, const float2 *rot, int m_base,
-                              int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
-  using S = ChanShape<M>;
-  const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
-  if (phase)
-    t41rx_chan_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(capture, tail, taps, tw, recv, chan, phase,
-                                                                             rot, m_base, n_entries, iq, n_blocks);
-  else
-    t41rx_chan_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan, phase,
-                                                                           rot, m_base, n_entries, iq, n_blocks);
-  return cudaGetLastError();
-}
-
-template <int M>
-static cudaError_t LaunchChanQ15(const short *capture, const short *tail, const float *taps, const float2 *tw,
-                                 const int32_t *recv, const int32_t *chan, const int2 *phase, const float2 *rot, int m_base,
-                                 int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
-  using S = ChanShape<M>;
-  const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
-  if (phase)
-    t41rx_chan_q15_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(capture, tail, taps, tw, recv, chan,
-                                                                                 phase, rot, m_base, n_entries, iq, n_blocks);
-  else
-    t41rx_chan_q15_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(capture, tail, taps, tw, recv, chan,
-                                                                               phase, rot, m_base, n_entries, iq, n_blocks);
-  return cudaGetLastError();
-}
-
-template <int M>
-static cudaError_t LaunchChanReal(const short *capture, const short *tail, const float *taps, const float2 *tw,
-                                  const float2 *split, const int32_t *recv, const int32_t *chan, const int2 *phase,
-                                  const float2 *rot, int m_base, int n_entries, float2 *iq, int n_blocks, cudaStream_t st) {
-  using S = ChanRealShape<M>;
-  const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
-  if (phase)
-    t41rx_chan_real_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
-        capture, tail, taps, tw, split, recv, chan, phase, rot, m_base, n_entries, iq, n_blocks);
-  else
-    t41rx_chan_real_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
-        capture, tail, taps, tw, split, recv, chan, phase, rot, m_base, n_entries, iq, n_blocks);
-  return cudaGetLastError();
-}
-
 /* modified Bessel function I0 (power series; terms fall below 1e-17 of the sum well before k = 60 for beta <= 9) */
 static double BesselI0(double x) {
   double sum = 1.0, term = 1.0;
@@ -627,6 +525,13 @@ static int ChanWrongKind(const char *fn, ChanKind kind) {
   return SetApiError(T41RX_EINVAL, (std::string(fn) + takes).c_str());
 }
 
+/* a channelizer's kernel pair (without and with fine tuning), chosen by kind and M at creation: prepare raises the
+   pair's dynamic shared memory limits, launch enqueues one call */
+struct ChanKernels {
+  cudaError_t (*prepare)();
+  cudaError_t (*launch)(const t41rx_chan *c, const void *capture, float2 *iq, int n_blocks, cudaStream_t st);
+};
+
 }  // namespace t41rx
 
 using namespace t41rx;
@@ -653,7 +558,52 @@ struct t41rx_chan {
   std::vector<int32_t> map;      /* receiver -> channel or -1 */
   std::vector<int32_t> shift, p0;   /* receiver -> shift and phase offset P, both in [0, 192000) */
   int m_done = 0;                /* outputs produced since creation, mod 192000 */
+  ChanKernels kernels{};
 };
+
+/* T = float2 (t41rx_chan_create) or short (t41rx_chan_create_q15) */
+template <int M, typename T>
+struct ChanComplex {
+  using S = ChanShape<M>;
+  static cudaError_t Prepare() {
+    return ChanSmemAttr(t41rx_chan_kernel<M, false, T>, S::kSmemBytes, t41rx_chan_kernel<M, true, T>, S::kSmemRotBytes);
+  }
+  static cudaError_t Launch(const t41rx_chan *c, const void *capture, float2 *iq, int n_blocks, cudaStream_t st) {
+    const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
+    const T *cap = (const T *)capture, *tail = (const T *)c->d_tail;
+    if (c->any_rotated)
+      t41rx_chan_kernel<M, true, T><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
+          cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->d_phase, c->d_rot, c->m_done, c->n_entries, iq, n_blocks);
+    else
+      t41rx_chan_kernel<M, false, T><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
+          cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, nullptr, c->d_rot, c->m_done, c->n_entries, iq, n_blocks);
+    return cudaGetLastError();
+  }
+};
+
+template <int M>
+struct ChanReal {
+  using S = ChanRealShape<M>;
+  static cudaError_t Prepare() {
+    return ChanSmemAttr(t41rx_chan_real_kernel<M, false>, S::kSmemBytes, t41rx_chan_real_kernel<M, true>, S::kSmemRotBytes);
+  }
+  static cudaError_t Launch(const t41rx_chan *c, const void *capture, float2 *iq, int n_blocks, cudaStream_t st) {
+    const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
+    const short *cap = (const short *)capture, *tail = (const short *)c->d_tail;
+    if (c->any_rotated)
+      t41rx_chan_real_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
+          cap, tail, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, c->d_phase, c->d_rot, c->m_done, c->n_entries,
+          iq, n_blocks);
+    else
+      t41rx_chan_real_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
+          cap, tail, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, nullptr, c->d_rot, c->m_done, c->n_entries, iq,
+          n_blocks);
+    return cudaGetLastError();
+  }
+};
+
+template <typename K>
+constexpr ChanKernels kChanKernels{K::Prepare, K::Launch};
 
 static int ChanQuiesce(t41rx_chan *c) {
   if (c->ext_pending) {
@@ -710,30 +660,11 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": stream/event creation failed").c_str()));
-  cudaError_t attr;
-  if (kind == ChanKind::kQ15)
-    attr = n_channels == 512 ? ChanSmemAttr(t41rx_chan_q15_kernel<512, false>, ChanShape<512>::kSmemBytes,
-                                            t41rx_chan_q15_kernel<512, true>, ChanShape<512>::kSmemRotBytes)
-                             : ChanSmemAttr(t41rx_chan_q15_kernel<64, false>, ChanShape<64>::kSmemBytes,
-                                            t41rx_chan_q15_kernel<64, true>, ChanShape<64>::kSmemRotBytes);
-  else switch (n_channels) {
-    case 512:
-      attr = ChanSmemAttr(t41rx_chan_kernel<512, false>, ChanShape<512>::kSmemBytes, t41rx_chan_kernel<512, true>,
-                          ChanShape<512>::kSmemRotBytes);
-      break;
-    case 64:
-      attr = ChanSmemAttr(t41rx_chan_kernel<64, false>, ChanShape<64>::kSmemBytes, t41rx_chan_kernel<64, true>,
-                          ChanShape<64>::kSmemRotBytes);
-      break;
-    case 1024:
-      attr = ChanSmemAttr(t41rx_chan_real_kernel<1024, false>, ChanRealShape<1024>::kSmemBytes,
-                          t41rx_chan_real_kernel<1024, true>, ChanRealShape<1024>::kSmemRotBytes);
-      break;
-    default:
-      attr = ChanSmemAttr(t41rx_chan_real_kernel<128, false>, ChanRealShape<128>::kSmemBytes,
-                          t41rx_chan_real_kernel<128, true>, ChanRealShape<128>::kSmemRotBytes);
-  }
-  if (attr != cudaSuccess)
+  const bool large = n_channels == 512 || n_channels == 1024;
+  c->kernels = real ? (large ? kChanKernels<ChanReal<1024>> : kChanKernels<ChanReal<128>>)
+               : kind == ChanKind::kQ15 ? (large ? kChanKernels<ChanComplex<512, short>> : kChanKernels<ChanComplex<64, short>>)
+               : large ? kChanKernels<ChanComplex<512, float2>> : kChanKernels<ChanComplex<64, float2>>;
+  if (c->kernels.prepare() != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": kernel image for this GPU missing (built for sm_100a)").c_str()));
   const int N = kChanTaps * n_channels;
   std::vector<float> taps(N);
@@ -862,33 +793,7 @@ static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, float
     return SetApiError(T41RX_EINVAL, (f + ": n_blocks too large for one call").c_str());
   if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, (f + ": cudaSetDevice failed").c_str());
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
-  cudaError_t e = cudaSuccess;
-  const int2 *phase = c->any_rotated ? c->d_phase : nullptr;
-  const float2 *cap = (const float2 *)capture, *tail = (const float2 *)c->d_tail;
-  const short *cap16 = (const short *)capture, *tail16 = (const short *)c->d_tail;
-  if (c->n_entries > 0 && c->kind == ChanKind::kQ15)
-    e = c->n_channels == 512
-            ? LaunchChanQ15<512>(cap16, tail16, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
-                                 c->n_entries, (float2 *)iq, n_blocks, st)
-            : LaunchChanQ15<64>(cap16, tail16, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
-                                c->n_entries, (float2 *)iq, n_blocks, st);
-  else if (c->n_entries > 0) switch (c->n_channels) {
-      case 512:
-        e = LaunchChan<512>(cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
-                            c->n_entries, (float2 *)iq, n_blocks, st);
-        break;
-      case 64:
-        e = LaunchChan<64>(cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, phase, c->d_rot, c->m_done,
-                           c->n_entries, (float2 *)iq, n_blocks, st);
-        break;
-      case 1024:
-        e = LaunchChanReal<1024>(cap16, tail16, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, phase, c->d_rot,
-                                 c->m_done, c->n_entries, (float2 *)iq, n_blocks, st);
-        break;
-      default:
-        e = LaunchChanReal<128>(cap16, tail16, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, phase, c->d_rot,
-                                c->m_done, c->n_entries, (float2 *)iq, n_blocks, st);
-    }
+  cudaError_t e = c->n_entries > 0 ? c->kernels.launch(c, capture, (float2 *)iq, n_blocks, st) : cudaSuccess;
   /* the new tail: the call's last N samples, copied after the kernel on the same stream so no tile reads it early */
   const size_t N = (size_t)kChanTaps * c->n_channels;
   const size_t total = (size_t)n_blocks * T41RX_BLOCK_SAMPLES * (c->n_channels / 2);

@@ -14,6 +14,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+from chan_driver import channelize
 from t41_sdr_b200 import rx, synth
 
 CHANNELS = (64, 512)
@@ -71,29 +72,6 @@ def test_wideband_q15_is_the_quantised_wideband_sum():
 
 # ---------------------------------------------------------------- GPU tier
 
-def _channelize(M, n_recv, capture, calls, maps, shifts, q15):
-    """One channelizer over `capture` (q15: int16 [n, 2]; else float32 [n, 2]) in calls of calls[i] blocks; maps[i]
-    and shifts[i] (each None or a list for receivers 0 ...) are set before call i.  Returns host iq
-    [n_recv, sum(calls), 2048, 2] (rows not written keep FILL)."""
-    import torch
-    per_block = BLOCK * M // 2
-    d_cap = torch.from_numpy(np.ascontiguousarray(capture)).cuda()
-    outs = []
-    with rx.Channelizer(M, n_recv, q15=q15) as ch:
-        b0 = 0
-        for nb, chmap, sh in zip(calls, maps, shifts):
-            if chmap is not None:
-                ch.set_map(chmap)
-            if sh is not None:
-                ch.set_shift(sh)
-            d_iq = torch.full((n_recv, nb, BLOCK, 2), FILL, dtype=torch.float32, device="cuda")
-            ch.process_device(d_cap[b0 * per_block:(b0 + nb) * per_block].data_ptr(), d_iq.data_ptr(), nb)
-            ch.synchronize()
-            outs.append(d_iq.cpu().numpy())
-            b0 += nb
-    return np.concatenate(outs, axis=1)
-
-
 def _test_capture(M, n_blocks, seed):
     """a seeded wideband_q15 capture with full-scale samples (-32768 and 32767, in I and in Q) scattered through it"""
     r = np.random.default_rng(seed)
@@ -122,8 +100,8 @@ def test_q15_is_bit_identical_to_float_on_s_over_32768(M):
     shifts1 = [12345, -54321, 96000, -96000, 0, 777, -191999]
     shifts2 = [191999, -191999, 4000, 0]
     calls, maps, shifts = [1, 2, 5], [map1, None, map2], [shifts1, shifts2, None]
-    got = _channelize(M, len(map1), capture, calls, maps, shifts, q15=True)
-    want = _channelize(M, len(map1), capture.astype(np.float32) / 32768.0, calls, maps, shifts, q15=False)
+    got = channelize(M, len(map1), capture, calls, maps, shifts, q15=True)
+    want = channelize(M, len(map1), capture.astype(np.float32) / 32768.0, calls, maps, shifts, q15=False)
     assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
     assert np.all(got[7, :3] == FILL)
     assert np.all(got[1, 3:] == FILL) and np.all(got[8, 3:] == FILL)
@@ -138,8 +116,8 @@ def test_split_calls_are_bit_identical_q15(M):
     capture = _test_capture(M, 8, 7)
     chmap = [3, 40 % M, -1, 3, M // 2, 0]
     for sh in (None, [48000, -20000, 0, 0, 95999, -191999]):
-        one = _channelize(M, 6, capture, [8], [chmap], [sh], q15=True)
-        split = _channelize(M, 6, capture, [1, 2, 5], [chmap, None, None], [sh, None, None], q15=True)
+        one = channelize(M, 6, capture, [8], [chmap], [sh], q15=True)
+        split = channelize(M, 6, capture, [1, 2, 5], [chmap, None, None], [sh, None, None], q15=True)
         assert np.array_equal(one.view(np.uint32), split.view(np.uint32))
         assert np.all(one[2] == FILL)
 

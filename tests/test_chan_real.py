@@ -13,9 +13,8 @@ import pytest
 
 import cases
 import oracle_py as O
+from chan_driver import chain, channelize, error_ratio, reference_channel, response_db, rotate
 from t41_sdr_b200 import rx, synth
-from test_chan_tuning import rotate
-from test_channelizer import _response_db, reference_channel
 
 CHANNELS = (128, 1024)
 MIRRORED = (rx.DEMOD_USB, rx.DEMOD_LSB, rx.DEMOD_AM, rx.DEMOD_SAM)
@@ -32,7 +31,7 @@ def test_prototype_design_real(M):
     assert taps.dtype == np.float32 and taps.size == 10 * M
     assert np.array_equal(taps, taps[::-1])
     assert abs(float(np.sum(taps, dtype=np.float64)) - 1.0) <= 1e-6
-    f, db = _response_db(taps, M, n_fft=1 << 21)
+    f, db = response_db(taps, M, n_fft=1 << 21)
     passband = db[np.abs(f) <= 60e3]
     assert passband.min() >= -0.01 and passband.max() <= 0.01
     assert db[np.abs(f) >= 132e3].max() <= -90.0
@@ -92,29 +91,6 @@ def test_create_real_without_device_is_enodev():
 
 # ---------------------------------------------------------------- GPU tier
 
-def _channelize(M, n_recv, capture, calls, maps, shifts=None, fill=12345.0):
-    """One real channelizer over the int16 `capture` in calls of calls[i] blocks; maps[i] and shifts[i] (each None or a
-    list for receivers 0 ...) are set before call i.  Returns host iq [n_recv, sum(calls), 2048, 2]."""
-    import torch
-    shifts = shifts or [None] * len(calls)
-    per_block = BLOCK * M // 2
-    d_cap = torch.from_numpy(np.ascontiguousarray(capture)).cuda()
-    outs = []
-    with rx.Channelizer(M, n_recv, real=True) as ch:
-        b0 = 0
-        for nb, chmap, sh in zip(calls, maps, shifts):
-            if chmap is not None:
-                ch.set_map(chmap)
-            if sh is not None:
-                ch.set_shift(sh)
-            d_iq = torch.full((n_recv, nb, BLOCK, 2), fill, dtype=torch.float32, device="cuda")
-            ch.process_device(d_cap[b0 * per_block:(b0 + nb) * per_block].data_ptr(), d_iq.data_ptr(), nb)
-            ch.synchronize()
-            outs.append(d_iq.cpu().numpy())
-            b0 += nb
-    return np.concatenate(outs, axis=1)
-
-
 def _x(capture):
     return capture.astype(np.float64) / 32768.0
 
@@ -128,15 +104,6 @@ def _test_capture(M, n_blocks, seed):
     return synth.wideband_real(seed, M, n_blocks, sig, sigma=0.05)
 
 
-def _error_ratio(got, want_by_receiver, x):
-    err2, n_vals = 0.0, 0
-    for r, want in want_by_receiver.items():
-        g = got[r].reshape(-1, 2)
-        err2 += np.sum((g[:, 0] - want.real) ** 2 + (g[:, 1] - want.imag) ** 2)
-        n_vals += want.size
-    return np.sqrt(err2 / n_vals) / np.sqrt(np.mean(x ** 2))
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("M", CHANNELS)
 def test_formula_parity_real(M):
@@ -147,12 +114,12 @@ def test_formula_parity_real(M):
     capture = _test_capture(M, n_blocks, 300 + M)
     chmap = [0, 1, M // 4, M // 2 - 1, M // 2, 7, 7, 1, M // 2, 0, -1]
     shifts = [0, 0, 0, 0, 0, 0, 12345, -54321, 96000, -96000, 777]
-    got = _channelize(M, len(chmap), capture, [1, n_blocks - 1], [chmap, None], [shifts, None])
+    got = channelize(M, len(chmap), capture, [1, n_blocks - 1], [chmap, None], [shifts, None], real=True)
     x, taps = _x(capture), rx.chan_taps(M)
     ref = {k: reference_channel(x, taps, M, k, n_blocks * BLOCK) for k in set(chmap) if k >= 0}
     want = {r: rotate(ref[k], 0, s) for r, (k, s) in enumerate(zip(chmap, shifts)) if k >= 0}
     assert np.all(got[chmap.index(-1)] == 12345.0)
-    ratio = _error_ratio(got, want, x)
+    ratio = error_ratio(got, want, x)
     print("M=%d: error RMS / capture RMS = %.3g" % (M, ratio))
     assert ratio <= 1e-6
 
@@ -167,12 +134,12 @@ def test_split_calls_and_map_changes_are_bit_identical_real():
     map2 = [40, 3, 64, -1, 0, 3]
     shifts = [48000, -20000, 0, 0, 95999, 777]
     for sh in (None, shifts):
-        one = _channelize(M, 6, capture, [T], [map1], [sh])
-        split = _channelize(M, 6, capture, [1, 2, 5], [map1, None, None], [sh, None, None])
+        one = channelize(M, 6, capture, [T], [map1], [sh], real=True)
+        split = channelize(M, 6, capture, [1, 2, 5], [map1, None, None], [sh, None, None], real=True)
         assert np.array_equal(one.view(np.uint32), split.view(np.uint32))
         assert np.all(one[2] == 12345.0)
-    one = _channelize(M, 6, capture, [T], [map1])
-    changed = _channelize(M, 6, capture, [1, 2, 5], [map1, None, map2])
+    one = channelize(M, 6, capture, [T], [map1], real=True)
+    changed = channelize(M, 6, capture, [1, 2, 5], [map1, None, map2], real=True)
     assert np.array_equal(changed[:, :3].view(np.uint32), one[:, :3].view(np.uint32))
     by_channel = {k: one[r] for r, k in enumerate(map1) if k >= 0}
     for r, k in enumerate(map2):
@@ -189,7 +156,7 @@ def test_real_tone_gain_and_rejection(M, k):
     further (after the first block, the filter's start-up)."""
     T, amp = 3, 0.5
     capture = synth.wideband_real(0, M, T, [("tone", rx.chan_centre_real(k), {"amp": amp})])
-    got = _channelize(M, M // 2 + 1, capture, [T], [list(range(M // 2 + 1))])[:, 1:]
+    got = channelize(M, M // 2 + 1, capture, [T], [list(range(M // 2 + 1))], real=True)[:, 1:]
     level = 20.0 * np.log10(np.sqrt(np.mean(got.astype(np.float64) ** 2 * 2, axis=(1, 2, 3))) / (amp / 2))
     print("M=%d k=%d: %.4f dB at the channel, worst %.1f dB two or more away" %
           (M, k, level[k], max(level[j] for j in range(M // 2 + 1) if abs(j - k) >= 2)))
@@ -222,14 +189,6 @@ def test_argument_checks_real():
     assert rx.lib().t41rx_chan_create(C.byref(h), 128, 4, 0) == EINVAL
 
 
-def _chain(params, iq, want_psk=False):
-    with rx.Receiver(len(params)) as eng:
-        eng.set_params_each(params)
-        out = eng.process(iq, want_psk=want_psk, flags=0)
-        out["debug"] = [eng.debug(s) for s in range(len(params))]
-    return out
-
-
 @pytest.mark.gpu
 def test_sideband_at_a_channel_centre_real():
     """A tone 1 kHz above a USB dial at the centre of channel 147 (14.112 MHz) of M = 1024, placed by
@@ -240,10 +199,10 @@ def test_sideband_at_a_channel_centre_real():
     assert placed == rx.chan_place_real(M, rx.DEMOD_LSB, dial) == (147, 48000, 0)
     ch, shift, nco = placed
     capture = synth.wideband_real(1, M, T, [("tone", dial + 1000.0, {"amp": 0.2})])
-    iq = _channelize(M, 2, capture, [T], [[ch, ch]], [[shift, shift]])
+    iq = channelize(M, 2, capture, [T], [[ch, ch]], [[shift, shift]], real=True)
     ps = [rx.make_params(mode=rx.DEMOD_USB, nco_freq=nco, agc_mode=0),
           rx.make_params(mode=rx.DEMOD_LSB, nco_freq=nco, agc_mode=0)]
-    audio = _chain(ps, iq)["audio"][:, 4:].reshape(2, -1).astype(np.float64)
+    audio = chain(ps, iq)["audio"][:, 4:].reshape(2, -1).astype(np.float64)
     spec = np.abs(np.fft.rfft(audio[0] * np.hanning(audio.shape[1])))
     f_peak = np.argmax(spec) * 192000.0 / audio.shape[1]
     assert abs(f_peak - 1000.0) <= 2 * 192000.0 / audio.shape[1], f_peak
@@ -270,7 +229,7 @@ def _psk_through_the_channelizer(M, freq, step):
             chan.process_device(cap.data_ptr(), iq[0, b0].data_ptr(), nb)
             chan.synchronize()
     ps =[rx.make_params(mode=rx.DEMOD_USB, f_lo_cut=-100, f_hi_cut=100, agc_mode=0, psk31_enable=1, nco_freq=nco)]
-    out = _chain(ps, iq.cpu().numpy(), want_psk=True)
+    out = chain(ps, iq.cpu().numpy(), want_psk=True)
     return bytes(out["psk_chars"][0][out["psk_chars"][0] > 0])
 
 
@@ -319,14 +278,14 @@ def test_bank_placed_by_chan_place_real_matches_rotated_reference_feed():
             params.append(rx.make_params(mode=mode, nco_freq=nco))
     capture = synth.wideband_real(9, M, T, signals, sigma=0.002)
     assert np.abs(capture).max() < 32767
-    got_iq = _channelize(M, n, capture, [T], [chmap], [shifts])
+    got_iq = channelize(M, n, capture, [T], [chmap], [shifts], real=True)
     x, taps = _x(capture), rx.chan_taps(M)
     ref_iq = np.empty_like(got_iq)
     for s, (k, sh) in enumerate(zip(chmap, shifts)):
         z = rotate(reference_channel(x, taps, M, k, T * BLOCK), 0, sh)
         ref_iq[s, ..., 0] = z.real.reshape(T, BLOCK)
         ref_iq[s, ..., 1] = z.imag.reshape(T, BLOCK)
-    got, want = _chain(params, got_iq), _chain(params, ref_iq)
+    got, want = chain(params, got_iq), chain(params, ref_iq)
     worst = np.inf
     for s in range(n):
         snr = O.snr_db(want["audio"][s, 2:], got["audio"][s, 2:])

@@ -13,25 +13,13 @@ import pytest
 
 import cases
 import oracle_py as O
+from chan_driver import OUT_RATE, chain, channelize, cplx, error_ratio, reference_channel, rotate
 from t41_sdr_b200 import rx, synth
-from test_channelizer import reference_channel
 
 CHANNELS = (64, 512)
 MIRRORED = (rx.DEMOD_USB, rx.DEMOD_LSB, rx.DEMOD_AM, rx.DEMOD_SAM)
 PLAIN = (rx.DEMOD_NFM, rx.DEMOD_PSK31)
 BLOCK = rx.BLOCK
-OUT_RATE = 192000
-
-
-def rotate(z, phase0, shift, m0=0):
-    """float64 z[m] exp(2 pi j phi / 192000), phi = (phase0 + shift (m0 + m)) mod 192000 in integers."""
-    m = np.arange(z.size, dtype=np.int64) + m0
-    phi = (phase0 + shift * m) % OUT_RATE
-    return z * np.exp(2j * np.pi * phi / OUT_RATE)
-
-
-def _cplx(capture):
-    return capture[:, 0].astype(np.float64) + 1j * capture[:, 1].astype(np.float64)
 
 
 def _iq(z, n_blocks):
@@ -84,7 +72,7 @@ def _oracle_audio(mode, nco, iq, skip=4, **kw):
 def _placed_feed(capture, M, mode, offset, n_blocks):
     """the float64 channel t41rx_chan_place picks for offset, rotated by its shift from m = 0; and its nco_freq"""
     ch, shift, nco = rx.chan_place(M, mode, offset)
-    z = reference_channel(_cplx(capture), rx.chan_taps(M), M, ch, n_blocks * BLOCK)
+    z = reference_channel(cplx(capture), rx.chan_taps(M), M, ch, n_blocks * BLOCK)
     return _iq(rotate(z, 0, shift), n_blocks), nco
 
 
@@ -115,7 +103,7 @@ def test_nfm_placement_sign_on_the_oracle():
     f = rx.chan_centre(M, 13) + 20000.0
     capture = synth.wideband(2, M, T, [("nfm", f, {"amp": 0.1})])
     ch, nco_direct = rx.chan_tune(M, rx.DEMOD_NFM, f)
-    z = reference_channel(_cplx(capture), rx.chan_taps(M), M, ch, T * BLOCK)
+    z = reference_channel(cplx(capture), rx.chan_taps(M), M, ch, T * BLOCK)
     direct = _oracle_audio(rx.DEMOD_NFM, nco_direct, _iq(z, T))
     _, shift, nco = rx.chan_place(M, rx.DEMOD_NFM, f)
     assert (shift, nco) == (20000 - 48000, 0)
@@ -153,44 +141,12 @@ def test_psk31_decodes_at_a_channel_centre_on_the_oracle():
 
 # ---------------------------------------------------------------- GPU tier
 
-def _channelize(M, n_recv, capture, calls, maps, shifts=None, fill=12345.0):
-    """One channelizer over `capture` in calls of calls[i] blocks; maps[i] and shifts[i] (each None or a list for
-    receivers 0 ...) are set before call i.  Returns host iq [n_recv, sum(calls), 2048, 2]."""
-    import torch
-    shifts = shifts or [None] * len(calls)
-    per_block = BLOCK * M // 2
-    d_cap = torch.from_numpy(np.ascontiguousarray(capture)).cuda()
-    outs = []
-    with rx.Channelizer(M, n_recv) as ch:
-        b0 = 0
-        for nb, chmap, sh in zip(calls, maps, shifts):
-            if chmap is not None:
-                ch.set_map(chmap)
-            if sh is not None:
-                ch.set_shift(sh)
-            d_iq = torch.full((n_recv, nb, BLOCK, 2), fill, dtype=torch.float32, device="cuda")
-            ch.process_device(d_cap[b0 * per_block:(b0 + nb) * per_block].data_ptr(), d_iq.data_ptr(), nb)
-            ch.synchronize()
-            outs.append(d_iq.cpu().numpy())
-            b0 += nb
-    return np.concatenate(outs, axis=1)
-
-
 def _test_capture(M, n_blocks, seed):
     r = np.random.default_rng(seed)
     fs = synth.wideband_rate(M)
     sig = [("tone", float(r.uniform(-fs / 2, fs / 2)), {"amp": float(r.uniform(0.05, 0.5))}) for _ in range(6)]
     sig.append(("tone", rx.chan_centre(M, 7) + 1234.5, {"amp": 0.3}))
     return synth.wideband(seed, M, n_blocks, sig, sigma=0.2)
-
-
-def _error_ratio(got, want_by_receiver, x):
-    err2, n_vals = 0.0, 0
-    for r, want in want_by_receiver.items():
-        g = got[r].reshape(-1, 2)
-        err2 += np.sum((g[:, 0] - want.real) ** 2 + (g[:, 1] - want.imag) ** 2)
-        n_vals += want.size
-    return np.sqrt(err2 / n_vals) / np.sqrt(np.mean(np.abs(x) ** 2))
 
 
 @pytest.mark.gpu
@@ -203,12 +159,12 @@ def test_formula_parity_with_shifts(M):
     capture = _test_capture(M, n_blocks, 200 + M)
     chmap = [7, 7, 1, M // 2, M - 1, 0, 3, -1, 7]
     shifts = [12345, -54321, 96000, -96000, 191999, -191999, 0, 5000, 48000]
-    got = _channelize(M, len(chmap), capture, [1, n_blocks - 1], [chmap, None], [shifts, None])
-    x, taps = _cplx(capture), rx.chan_taps(M)
+    got = channelize(M, len(chmap), capture, [1, n_blocks - 1], [chmap, None], [shifts, None])
+    x, taps = cplx(capture), rx.chan_taps(M)
     want = {r: rotate(reference_channel(x, taps, M, k, n_blocks * BLOCK), 0, s)
             for r, (k, s) in enumerate(zip(chmap, shifts)) if k >= 0}
     assert np.all(got[chmap.index(-1)] == 12345.0)
-    ratio = _error_ratio(got, want, x)
+    ratio = error_ratio(got, want, x)
     print("M=%d: error RMS / capture RMS = %.3g" % (M, ratio))
     assert ratio <= 1e-6
 
@@ -222,10 +178,10 @@ def test_unshifted_receivers_and_split_calls_are_bit_identical():
     capture = _test_capture(M, T, 5)
     chmap = [3, 40, 3, 63, 32, 40, -1]
     shifts = [48000, 0, 0, -20000, 0, 95999, 777]
-    plain = _channelize(M, 7, capture, [T], [chmap])
-    one = _channelize(M, 7, capture, [T], [chmap], [shifts])
-    split = _channelize(M, 7, capture, [1, 2, 5], [chmap, None, None], [shifts, None, None])
-    zeros = _channelize(M, 7, capture, [1, 2, 5], [chmap, None, None], [[0] * 7, None, [0] * 7])
+    plain = channelize(M, 7, capture, [T], [chmap])
+    one = channelize(M, 7, capture, [T], [chmap], [shifts])
+    split = channelize(M, 7, capture, [1, 2, 5], [chmap, None, None], [shifts, None, None])
+    zeros = channelize(M, 7, capture, [1, 2, 5], [chmap, None, None], [[0] * 7, None, [0] * 7])
     assert np.array_equal(one.view(np.uint32), split.view(np.uint32))
     assert np.array_equal(zeros.view(np.uint32), plain.view(np.uint32))
     for r, s in enumerate(shifts):
@@ -242,15 +198,15 @@ def test_shift_change_keeps_the_phase_continuous():
     chmap = [7, 7, 20, 50]
     s1 = [30000, -70000, 0, 12345]
     s2 = [-45000, 0, 60000, 12345]
-    got = _channelize(M, 4, capture, [T1, T - T1], [chmap, None], [s1, s2])
-    x, taps = _cplx(capture), rx.chan_taps(M)
+    got = channelize(M, 4, capture, [T1, T - T1], [chmap, None], [s1, s2])
+    x, taps = cplx(capture), rx.chan_taps(M)
     m1 = T1 * BLOCK
     want = {}
     for r, k in enumerate(chmap):
         z = reference_channel(x, taps, M, k, T * BLOCK)
         phase1 = (s1[r] * m1) % OUT_RATE                       # where the first shift has brought the phase at m1
         want[r] = np.concatenate([rotate(z[:m1], 0, s1[r]), rotate(z[m1:], phase1, s2[r])])
-    ratio = _error_ratio(got, want, x)
+    ratio = error_ratio(got, want, x)
     print("error RMS / capture RMS = %.3g" % ratio)
     assert ratio <= 1e-6
 
@@ -268,14 +224,6 @@ def test_set_shift_rejects_bad_input():
         ch.set_shift([191999, -191999, 0, 96000])
 
 
-def _chain(params, iq, want_psk=False):
-    with rx.Receiver(len(params)) as eng:
-        eng.set_params_each(params)
-        out = eng.process(iq, want_psk=want_psk, flags=0)
-        out["debug"] = [eng.debug(s) for s in range(len(params))]
-    return out
-
-
 @pytest.mark.gpu
 def test_sideband_at_a_channel_centre_end_to_end():
     """A tone 1 kHz above a USB dial at the centre of channel M - 13, placed by chan_place: 1 kHz audio in USB and
@@ -286,10 +234,10 @@ def test_sideband_at_a_channel_centre_end_to_end():
     assert placed == rx.chan_place(M, rx.DEMOD_LSB, dial) == (M - 13, 48000, 0)
     ch, shift, nco = placed
     capture = synth.wideband(1, M, T, [("tone", dial + 1000.0, {"amp": 0.1})])
-    iq = _channelize(M, 2, capture, [T], [[ch, ch]], [[shift, shift]])
+    iq = channelize(M, 2, capture, [T], [[ch, ch]], [[shift, shift]])
     ps = [rx.make_params(mode=rx.DEMOD_USB, nco_freq=nco, agc_mode=0),
           rx.make_params(mode=rx.DEMOD_LSB, nco_freq=nco, agc_mode=0)]
-    audio = _chain(ps, iq)["audio"][:, 4:].reshape(2, -1).astype(np.float64)
+    audio = chain(ps, iq)["audio"][:, 4:].reshape(2, -1).astype(np.float64)
     spec = np.abs(np.fft.rfft(audio[0] * np.hanning(audio.shape[1])))
     f_peak = np.argmax(spec) * float(OUT_RATE) / audio.shape[1]
     assert abs(f_peak - 1000.0) <= 2 * OUT_RATE / audio.shape[1], f_peak
@@ -308,10 +256,10 @@ def test_psk31_decodes_at_channel_centres_end_to_end():
     capture, T, step = _psk_capture(M, offsets)
     calls = [min(step, T - b0) for b0 in range(0, T, step)]
     rest = [None] * (len(calls) - 1)
-    iq = _channelize(M, 2, capture, calls, [[c for c, _, _ in placed]] + rest, [[s for _, s, _ in placed]] + rest)
+    iq = channelize(M, 2, capture, calls, [[c for c, _, _ in placed]] + rest, [[s for _, s, _ in placed]] + rest)
     ps = [rx.make_params(mode=rx.DEMOD_USB, f_lo_cut=-100, f_hi_cut=100, agc_mode=0, psk31_enable=1, nco_freq=nco)
           for _, _, nco in placed]
-    out = _chain(ps, iq, want_psk=True)
+    out = chain(ps, iq, want_psk=True)
     for s in range(2):
         chars = bytes(out["psk_chars"][s][out["psk_chars"][s] > 0])
         assert cases.PSK_TEXT.encode() in chars, (s, chars)
@@ -350,11 +298,11 @@ def test_bank_placed_by_chan_place_matches_rotated_reference_feed():
         else:
             params.append(rx.make_params(mode=mode, nco_freq=nco))
     capture = synth.wideband(9, M, T, signals, sigma=0.002)
-    got_iq = _channelize(M, n, capture, [T], [chmap], [shifts])
-    x, taps = _cplx(capture), rx.chan_taps(M)
+    got_iq = channelize(M, n, capture, [T], [chmap], [shifts])
+    x, taps = cplx(capture), rx.chan_taps(M)
     ref_iq = np.stack([_iq(rotate(reference_channel(x, taps, M, k, T * BLOCK), 0, s), T)
                        for k, s in zip(chmap, shifts)])
-    got, want = _chain(params, got_iq), _chain(params, ref_iq)
+    got, want = chain(params, got_iq), chain(params, ref_iq)
     worst = np.inf
     for s in range(n):
         snr = O.snr_db(want["audio"][s, 2:], got["audio"][s, 2:])

@@ -8,35 +8,16 @@ decoded through the wideband path.
 """
 import numpy as np
 import pytest
-from scipy.signal import fftconvolve
 
 import cases
 import oracle_py as O
+from chan_driver import chain, channelize, cplx, reference_channel, response_db
 from t41_sdr_b200 import rx, synth
 
 CHANNELS = (64, 512)
 MIRRORED = (rx.DEMOD_USB, rx.DEMOD_LSB, rx.DEMOD_AM, rx.DEMOD_SAM)
 PLAIN = (rx.DEMOD_NFM, rx.DEMOD_PSK31)
 BLOCK = rx.BLOCK
-
-
-def _response_db(taps, M, n_fft=1 << 20):
-    H = np.fft.fft(taps.astype(np.float64), n_fft)
-    f = np.fft.fftfreq(n_fft, 1.0 / synth.wideband_rate(M))
-    return f, 20.0 * np.log10(np.maximum(np.abs(H), 1e-300))
-
-
-def reference_channel(x, taps, M, k, n_out):
-    """float64 z_k[m] = conj(sum_i h[i] x[mD - i] exp(-2 pi j k (mD - i) / M)), m < n_out: direct mix, convolution,
-    decimation.  x: complex capture from n = 0 (x[n < 0] = 0)."""
-    D = M // 2
-    n = np.arange(x.size)
-    y = x * np.exp(-2j * np.pi * ((k * n) % M) / M)
-    return np.conj(fftconvolve(y, taps.astype(np.float64))[:x.size][0:n_out * D:D])
-
-
-def _cplx(capture):
-    return capture[:, 0].astype(np.float64) + 1j * capture[:, 1].astype(np.float64)
 
 
 # ---------------------------------------------------------------- CPU tier
@@ -47,7 +28,7 @@ def test_prototype_design(M):
     assert taps.dtype == np.float32 and taps.size == 10 * M
     assert np.array_equal(taps, taps[::-1])
     assert abs(float(np.sum(taps, dtype=np.float64)) - 1.0) <= 1e-6
-    f, db = _response_db(taps, M)
+    f, db = response_db(taps, M)
     passband = db[np.abs(f) <= 60e3]
     assert passband.min() >= -0.01 and passband.max() <= 0.01
     assert db[np.abs(f) >= 132e3].max() <= -90.0
@@ -98,26 +79,6 @@ def test_create_without_device_is_enodev():
 
 # ---------------------------------------------------------------- GPU tier
 
-def _channelize(M, n_recv, capture, calls, maps, fill=12345.0):
-    """Run one channelizer over `capture` in calls of calls[i] blocks; maps[i] (or None) is set before call i.
-    Returns host iq [n_recv, sum(calls), 2048, 2]; rows of unmapped receivers keep `fill`."""
-    import torch
-    per_block = BLOCK * M // 2
-    d_cap = torch.from_numpy(np.ascontiguousarray(capture)).cuda()
-    outs = []
-    with rx.Channelizer(M, n_recv) as ch:
-        b0 = 0
-        for nb, chmap in zip(calls, maps):
-            if chmap is not None:
-                ch.set_map(chmap)
-            d_iq = torch.full((n_recv, nb, BLOCK, 2), fill, dtype=torch.float32, device="cuda")
-            ch.process_device(d_cap[b0 * per_block:(b0 + nb) * per_block].data_ptr(), d_iq.data_ptr(), nb)
-            ch.synchronize()
-            outs.append(d_iq.cpu().numpy())
-            b0 += nb
-    return np.concatenate(outs, axis=1)
-
-
 def _test_capture(M, n_blocks, seed):
     r = np.random.default_rng(seed)
     fs = synth.wideband_rate(M)
@@ -134,9 +95,9 @@ def test_formula_parity(M):
     capture = _test_capture(M, n_blocks, 100 + M)
     check = sorted({0, 1, M // 2 - 1, M // 2, M - 1, 7, M // 2 + 5})
     chmap = check + [7, -1]
-    got = _channelize(M, len(chmap), capture, [1, n_blocks - 1], [chmap, None])
+    got = channelize(M, len(chmap), capture, [1, n_blocks - 1], [chmap, None])
     taps = rx.chan_taps(M)
-    x = _cplx(capture)
+    x = cplx(capture)
     n_out = n_blocks * BLOCK
     err2 = 0.0
     for r, k in enumerate(chmap):
@@ -158,12 +119,12 @@ def test_split_calls_and_map_changes_are_bit_identical():
     capture = _test_capture(M, T, 5)
     map1 = [3, 40, -1, 3, 63, 32]
     map2 = [40, 3, 63, -1, 32, 3]
-    one = _channelize(M, 6, capture, [T], [map1])
-    split = _channelize(M, 6, capture, [1, 2, 5], [map1, None, None])
+    one = channelize(M, 6, capture, [T], [map1])
+    split = channelize(M, 6, capture, [1, 2, 5], [map1, None, None])
     assert np.array_equal(one.view(np.uint32), split.view(np.uint32))
     assert np.all(one[2] == 12345.0)                                   # unmapped: sentinel kept
     assert np.array_equal(one[0].view(np.uint32), one[3].view(np.uint32))   # a shared channel: identical copies
-    changed = _channelize(M, 6, capture, [1, 2, 5], [map1, None, map2])
+    changed = channelize(M, 6, capture, [1, 2, 5], [map1, None, map2])
     assert np.array_equal(changed[:, :3].view(np.uint32), one[:, :3].view(np.uint32))
     by_channel = {k: one[r] for r, k in enumerate(map1) if k >= 0}
     for r, k in enumerate(map2):
@@ -178,19 +139,11 @@ def test_split_calls_and_map_changes_are_bit_identical():
 def test_stopband_through_the_kernel(k):
     M, T, amp = 64, 3, 0.5
     capture = synth.wideband(0, M, T, [("tone", rx.chan_centre(M, k), {"amp": amp})])
-    got = _channelize(M, M, capture, [T], [list(range(M))])[:, 1:]     # after the first block (the filter's start-up)
+    got = channelize(M, M, capture, [T], [list(range(M))])[:, 1:]     # after the first block (the filter's start-up)
     level = 20.0 * np.log10(np.sqrt(np.mean(got.astype(np.float64) ** 2 * 2, axis=(1, 2, 3))) / amp)
     assert abs(level[k]) <= 0.01, level[k]
     far = [j for j in range(M) if min((j - k) % M, (k - j) % M) >= 2]
     assert level[far].max() <= -90.0, level[far].max()
-
-
-def _chain(params, iq, want_psk=False):
-    with rx.Receiver(len(params)) as eng:
-        eng.set_params_each(params)
-        out = eng.process(iq, want_psk=want_psk, flags=0)
-        out["debug"] = [eng.debug(s) for s in range(len(params))]
-    return out
 
 
 @pytest.mark.gpu
@@ -204,10 +157,10 @@ def test_sideband_convention_end_to_end():
     ch_l, nco_l = rx.chan_tune(M, rx.DEMOD_LSB, dial)
     assert (ch_u, nco_u) == (ch_l, nco_l) == (M - 13, 4433)
     capture = synth.wideband(1, M, T, [("tone", dial + 1000.0, {"amp": 0.1})])
-    iq = _channelize(M, 2, capture, [T], [[ch_u, ch_l]])
+    iq = channelize(M, 2, capture, [T], [[ch_u, ch_l]])
     ps = [rx.make_params(mode=rx.DEMOD_USB, nco_freq=nco_u, agc_mode=0),
           rx.make_params(mode=rx.DEMOD_LSB, nco_freq=nco_l, agc_mode=0)]
-    audio = _chain(ps, iq)["audio"][:, 4:].reshape(2, -1).astype(np.float64)
+    audio = chain(ps, iq)["audio"][:, 4:].reshape(2, -1).astype(np.float64)
     spec = np.abs(np.fft.rfft(audio[0] * np.hanning(audio.shape[1])))
     f_peak = np.argmax(spec) * 192000.0 / audio.shape[1]
     assert abs(f_peak - 1000.0) <= 2 * 192000.0 / audio.shape[1], f_peak
@@ -247,14 +200,14 @@ def test_bank_fed_by_channelizer_matches_reference_feed():
         else:
             params.append(rx.make_params(mode=mode, nco_freq=nco))
     capture = synth.wideband(9, M, T, signals, sigma=0.002)
-    got_iq = _channelize(M, n, capture, [T], [chmap])
-    x, taps = _cplx(capture), rx.chan_taps(M)
+    got_iq = channelize(M, n, capture, [T], [chmap])
+    x, taps = cplx(capture), rx.chan_taps(M)
     ref_iq = np.empty_like(got_iq)
     for s, k in enumerate(chmap):
         z = reference_channel(x, taps, M, k, T * BLOCK)
         ref_iq[s, ..., 0] = z.real.reshape(T, BLOCK)
         ref_iq[s, ..., 1] = z.imag.reshape(T, BLOCK)
-    got, want = _chain(params, got_iq), _chain(params, ref_iq)
+    got, want = chain(params, got_iq), chain(params, ref_iq)
     worst = np.inf
     for s in range(n):
         snr = O.snr_db(want["audio"][s, 2:], got["audio"][s, 2:])
@@ -282,10 +235,10 @@ def test_psk31_decodes_through_the_wideband_path():
         pieces.append(synth.wideband(31, M, nb, signals, sigma=0.01, start_block=b0))
     capture = np.concatenate(pieces)
     calls = [min(step, T - b0) for b0 in range(0, T, step)]
-    iq = _channelize(M, 2, capture, calls, [[c for c, _ in chs]] + [None] * (len(calls) - 1))
+    iq = channelize(M, 2, capture, calls, [[c for c, _ in chs]] + [None] * (len(calls) - 1))
     ps = [rx.make_params(mode=rx.DEMOD_USB, f_lo_cut=-100, f_hi_cut=100, agc_mode=0, psk31_enable=1, nco_freq=nco)
           for _, nco in chs]
-    out = _chain(ps, iq, want_psk=True)
+    out = chain(ps, iq, want_psk=True)
     for s in range(2):
         chars = bytes(out["psk_chars"][s][out["psk_chars"][s] > 0])
         assert cases.PSK_TEXT.encode() in chars, (s, chars)
