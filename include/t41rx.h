@@ -249,8 +249,9 @@ int t41rx_multi_gather_rows(t41rx_multi *m, const void *const *rows, size_t byte
 const char *t41rx_multi_last_error(void);
 
 /* ---- polyphase channelizer: one wideband capture -> the receivers' iq blocks (DESIGN §3.7) ----
- * The capture x[n] is interleaved complex float at Fs_in = M x 96 kS/s, M = n_channels in {64, 512} (6.144 or
- * 49.152 MS/s); n counts samples since t41rx_chan_create, x[n < 0] = 0.  Prototype h[0..N), N = 10 M: Kaiser-windowed
+ * The capture x[n] is interleaved complex float at Fs_in = M x 96 kS/s, M = n_channels in {64, 320, 512, 640} (6.144,
+ * 30.72, 49.152 or 61.44 MS/s; 30.72 and 61.44 are the LTE-family rates of AD936x / USRP N3xx digitizers, DESIGN
+ * §3.10); n counts samples since t41rx_chan_create, x[n < 0] = 0.  Prototype h[0..N), N = 10 M: Kaiser-windowed
  * sinc (beta 8.96), cutoff 96 kHz, designed in FP64, symmetric, unit DC gain, rounded to float: flat to +-60 kHz,
  * <= -90 dB from 132 kHz.  Decimation D = M / 2: every channel comes out at 192 kS/s, channel k centred at
  * (k < M/2 ? k : k - M) x 96 kHz, so any frequency of the capture lies within 48 kHz of some centre.  Sample m of
@@ -272,7 +273,7 @@ const char *t41rx_multi_last_error(void);
  * operating point, t41rx_chan_tune (no shift) on NCOFreq 48000 +- f_rel. */
 typedef struct t41rx_chan t41rx_chan;
 /* n_receivers = the n_streams of the context the iq output feeds; every receiver starts unmapped (-1).  ENODEV without
- * a CUDA device, EINVAL for n_channels other than 64 / 512. */
+ * a CUDA device, EINVAL for n_channels other than 64 / 320 / 512 / 640. */
 int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device);
 void t41rx_chan_destroy(t41rx_chan *c);
 /* receivers [first, first + count) take channel[i] in [0, n_channels), or -1 = not written (their iq rows keep whatever
@@ -289,11 +290,12 @@ int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shi
  * not ordered against each other by the library (the capture tail lives in the channelizer). */
 int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream);
 int t41rx_chan_synchronize(t41rx_chan *c);
-/* Host only, no GPU needed: the prototype (10 * n_channels floats, h[0] first; n_channels 64, 128, 512 or 1024), and where to put a receiver whose
- * carrier or dial point sits offset_hz from the capture's centre: the nearest channel centre (|f_rel| <= 48 kHz) and
+/* Host only, no GPU needed: the prototype (10 * n_channels floats, h[0] first; n_channels 64, 128, 320, 512, 640, 800,
+ * 1024 or 1280), and where to put a receiver whose carrier or dial point sits offset_hz from the capture's centre: the nearest channel centre (|f_rel| <= 48 kHz) and
  * nco_freq = 48000 + f_rel for USB / LSB / AM / SAM, 48000 - f_rel for NFM / PSK31 (rounded to integer Hz).  EINVAL
  * outside [-Fs_in / 2, Fs_in / 2) or for a mode t41rx_set_params rejects.  Offsets within 48 kHz below +Fs_in / 2 go
- * to channel M / 2, whose centre -Fs_in / 2 is the same frequency. */
+ * to channel M / 2, whose centre -Fs_in / 2 is the same frequency.  t41rx_chan_tune / t41rx_chan_place take the
+ * complex channel counts 64, 320, 512 and 640. */
 int t41rx_chan_taps(int n_channels, float *taps);
 int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *nco_freq);
 /* Host only, the placement to use with fine tuning: the channel t41rx_chan_tune picks, the shift that brings the
@@ -303,7 +305,9 @@ int t41rx_chan_tune(int n_channels, int32_t mode, double offset_hz, int32_t *cha
 int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *channel, int32_t *shift_hz,
                      int32_t *nco_freq);
 /* Real captures (DESIGN §3.8), as a direct-sampling ADC delivers them: s[n] int16 at Fs_in = M x 96 kS/s, M =
- * n_channels in {128, 1024} (12.288 MS/s: 0 - 6.144 MHz; 98.304 MS/s: 0 - 49.152 MHz, all of HF).  x[n] = s[n] / 32768
+ * n_channels in {128, 800, 1024, 1280} (12.288 MS/s: 0 - 6.144 MHz; 76.8 MS/s: 0 - 38.4 MHz, Hermes-Lite 2's ADC
+ * clock; 98.304 MS/s: 0 - 49.152 MHz, all of HF; 122.88 MS/s: 0 - 61.44 MHz, the HPSDR family's ADC clock, DESIGN
+ * §3.10).  x[n] = s[n] / 32768
  * (as arm_q15_to_float), then the formula above unchanged (prototype N = 10 M, D = M / 2, the conjugate).  Only
  * channels k = 0 ... M / 2 are distinct, channel k centred at +k x 96 kHz; a real tone A cos(2 pi f t) appears in its
  * channel with amplitude A / 2.  Mirror caveat: channel 0 holds its band together with its mirror image about 0 Hz,
@@ -311,12 +315,12 @@ int t41rx_chan_place(int n_channels, int32_t mode, double offset_hz, int32_t *ch
  * M / 2) hears the band and its mirror image at once.
  * t41rx_chan_set_map takes channels in [0, M / 2] on a real channelizer; set_map, set_shift, synchronize, destroy, the
  * iq layout, the phase rule and the ordering contract are those of the complex channelizer.
- * t41rx_chan_create_real: ENODEV without a CUDA device, EINVAL for n_channels other than 128 / 1024.
+ * t41rx_chan_create_real: ENODEV without a CUDA device, EINVAL for n_channels other than 128 / 800 / 1024 / 1280.
  * t41rx_chan_process_device_real: capture int16 [n_blocks * 2048 * n_channels / 2], a DEVICE pointer, 16-byte aligned;
  * iq and cuda_stream as t41rx_chan_process_device.  Each kind of channelizer rejects the other kinds' process calls
  * (EINVAL).
  * t41rx_chan_tune_real / t41rx_chan_place_real: host only, freq_hz the absolute frequency in [0, Fs_in / 2] (EINVAL
- * outside it, for NaN, for a mode t41rx_set_params rejects, for n_channels other than 128 / 1024): channel =
+ * outside it, for NaN, for a mode t41rx_set_params rejects, for n_channels other than 128 / 800 / 1024 / 1280): channel =
  * round(freq_hz / 96000), f_rel = freq_hz - channel x 96000, nco_freq and shift_hz by the rules of t41rx_chan_tune /
  * t41rx_chan_place. */
 int t41rx_chan_create_real(t41rx_chan **out, int n_channels, int n_receivers, int device);
@@ -325,12 +329,12 @@ int t41rx_chan_tune_real(int n_channels, int32_t mode, double freq_hz, int32_t *
 int t41rx_chan_place_real(int n_channels, int32_t mode, double freq_hz, int32_t *channel, int32_t *shift_hz,
                           int32_t *nco_freq);
 /* Complex int16 captures (DESIGN §3.9), as wideband I/Q digitizers stream them (sc16: USRP-class, AD936x / LMS7002,
- * SDRplay): interleaved (I, Q) int16 pairs at Fs_in = M x 96 kS/s, M = n_channels in {64, 512}.  x[n] = (I[n] + j Q[n])
+ * SDRplay): interleaved (I, Q) int16 pairs at Fs_in = M x 96 kS/s, M = n_channels in {64, 320, 512, 640}.  x[n] = (I[n] + j Q[n])
  * / 32768 (as arm_q15_to_float), then the complex channelizer unchanged: channels, fine tuning, t41rx_chan_tune /
  * t41rx_chan_place, set_map (channels [0, M)), set_shift, synchronize, destroy, the iq layout, the n_blocks limit and
  * the ordering contract.  The output is bit for bit that of t41rx_chan_create's channelizer fed with s / 32768 as
  * float (exact), while the capture takes half the bytes and needs no conversion pass.
- * t41rx_chan_create_q15: ENODEV without a CUDA device, EINVAL for n_channels other than 64 / 512.
+ * t41rx_chan_create_q15: ENODEV without a CUDA device, EINVAL for n_channels other than 64 / 320 / 512 / 640.
  * t41rx_chan_process_device_q15: capture int16 [n_blocks * 2048 * n_channels / 2][2], a DEVICE pointer, 16-byte
  * aligned; iq and cuda_stream as t41rx_chan_process_device. */
 int t41rx_chan_create_q15(t41rx_chan **out, int n_channels, int n_receivers, int device);

@@ -1,6 +1,6 @@
 /*
  * rx_chan.cu — polyphase channelizer (t41rx_chan_*, include/t41rx.h): one wideband complex capture at M x 96 kS/s
- * (M = 64 or 512 channels) cut into M channels of 192 kS/s, delivered in t41rx_process_device's iq layout.
+ * (M = 64, 320, 512 or 640 channels) cut into M channels of 192 kS/s, delivered in t41rx_process_device's iq layout.
  *
  * Transform (DESIGN §3.7): prototype h[0..N), N = K M, K = 10; decimation D = M / 2; channel k centred at
  * (k < M/2 ? k : k - M) x 96 kHz;
@@ -26,17 +26,22 @@
  * channelizer ((x, y) (1, 0) would turn -0 into +0); a call in which no receiver is rotated runs the kernel instance
  * without fine tuning.
  *
- * Real captures (t41rx_chan_create_real, DESIGN §3.8): int16 s[n] at M x 96 kS/s, M = 128 or 1024, x = s / 32768, the
+ * Real captures (t41rx_chan_create_real, DESIGN §3.8): int16 s[n] at M x 96 kS/s, M = 128, 800, 1024 or 1280, x = s / 32768, the
  * same formula; channels k = 0 .. M/2 are distinct, channel k centred at +k x 96 kHz.  u_p[m] is real, so the M-point DFT
  * of a row is one M/2-point complex FFT of y[n] = u[2n] + j u[2n + 1] and a split,
  *     X[k] = (Y[k] + conj Y[-k]) / 2 - j e^(-j 2 pi k / M) (Y[k] - conj Y[-k]) / 2,   k = 0 .. M/2, indices mod M/2;
  * the odd-m shift of u by M/2 is a shift of y by M/4.  t41rx_chan_real_kernel is the complex kernel at M/2: thread n owns
  * branches 2n and 2n + 1 (20 taps), the span is staged as int16, the split runs in the store loop.
  *
- * Complex int16 captures (t41rx_chan_create_q15, DESIGN §3.9): (I, Q) int16 pairs, x = (I + jQ) / 32768, M = 64 or 512.
+ * Complex int16 captures (t41rx_chan_create_q15, DESIGN §3.9): (I, Q) int16 pairs, x = (I + jQ) / 32768, M as for float.
  * t41rx_chan_kernel<M, kRotate, short> converts the span once as it stages it; the rest of the kernel is the float
  * instance's, with the 1 / 32768 in the taps: the same FMAs on the same values, so the same bits as the float
  * channelizer on s / 32768.
+ *
+ * Digitizers' clocks (DESIGN §3.10): M = 320, 640 (complex) and 800, 1280 (real) give FFT lengths 320, 640 and 400, which
+ * are 2^a 5^b.  Their rows are in natural order and run the mixed-radix DIF passes of ChanPlan (radix 5 beside 8, a
+ * radix-2 pass where the factorisation needs it); X[k] ends at the mixed-radix digit reversal of k.  The power-of-two
+ * instances never reach that code (if constexpr on kChanPow2), so their SASS is the same as before it was added.
  */
 #include <cuda_runtime.h>
 
@@ -64,11 +69,17 @@ constexpr int kChanOutRate = 192000;      /* the phase of a fine-tuning rotation
 constexpr int kRotCoarse = 480, kRotFine = 400;   /* kChanOutRate = kRotCoarse x kRotFine */
 static_assert(kRotCoarse * kRotFine == kChanOutRate && kChanOutRate % 512 == 0, "rotation table shape");
 
+/* FFT lengths that are not a power of two (320, 400, 640 = 2^a 5^b) run the mixed-radix passes of ChanPlan */
+template <int L> constexpr bool kChanPow2 = (L & (L - 1)) == 0;
+
 template <int M>
 struct ChanShape {
   static constexpr int D = M / 2;
   static constexpr int N = kChanTaps * M;
   static constexpr int kThreads = M >= 256 ? M : 256;
+  /* CTAs per SM (__launch_bounds__): shared memory allows 4 at M = 64, 3 at 320 (72 KiB each), 2 at 512, 1 at 640
+     (137 KiB) */
+  static constexpr int kMinBlocks = M == 512 ? 2 : M == 320 ? 3 : M == 640 ? 1 : 4;
   static constexpr int kGroups = kThreads / M;                  /* threads per branch */
   static constexpr int kTimes = kChanTile / kGroups;            /* output times per thread */
   static constexpr int kSpan = kChanTile * D + N;               /* capture samples a tile stages (one spare at the end) */
@@ -87,8 +98,37 @@ struct ChanShape {
 
 /* FFT row layout: element i (natural index) of a row lives at Phys(i); the DIF passes leave X[k] at OutPos(k) */
 template <int M> __device__ __forceinline__ int ChanPhys(int i) { return M == 512 ? FftPhys(i) : i; }
+
+/* mixed-radix DIF plans (DESIGN §3.10): the radices in pass order.  Rows of these lengths are in natural order */
+template <int L> struct ChanPlan;
+template <> struct ChanPlan<320> { static constexpr int kPasses = 3, kRadix[3] = {5, 8, 8}; };
+template <> struct ChanPlan<400> { static constexpr int kPasses = 4, kRadix[4] = {5, 5, 8, 2}; };
+template <> struct ChanPlan<640> { static constexpr int kPasses = 4, kRadix[4] = {5, 8, 8, 2}; };
+
+/* where the DIF passes of ChanPlan<L> leave X[k]: the mixed-radix digit reversal.  The digits of k, least significant
+   first, are in the radices r_0, r_1, ... of the passes, and digit s weighs L / (r_0 ... r_s) in the position */
+template <int L, int kPass = 0, int Ls = L>
+__device__ __forceinline__ int ChanMixedOutPos(int k) {
+  constexpr int R = ChanPlan<L>::kRadix[kPass];
+  if constexpr (kPass + 1 < ChanPlan<L>::kPasses) return (k % R) * (Ls / R) + ChanMixedOutPos<L, kPass + 1, Ls / R>(k / R);
+  else return k * (Ls / R);
+}
+
 template <int M> __device__ __forceinline__ int ChanOutPos(int k) {
-  return M == 512 ? FftPhys((int)OctRev3((unsigned)k)) : (((k & 7) << 3) | (k >> 3));
+  if constexpr (!kChanPow2<M>) return ChanMixedOutPos<M>(k);
+  else return M == 512 ? FftPhys((int)OctRev3((unsigned)k)) : (((k & 7) << 3) | (k >> 3));
+}
+
+/* (p + L/2) mod L for p in [0, L): the odd-m circular shift of a row's input */
+template <int L> __device__ __forceinline__ int ChanHalfTurn(int p) {
+  if constexpr (kChanPow2<L>) return p ^ (L / 2);
+  else return p < L / 2 ? p + L / 2 : p - L / 2;
+}
+
+/* k mod L for k in [0, L] */
+template <int L> __device__ __forceinline__ int ChanWrap(int k) {
+  if constexpr (kChanPow2<L>) return k & (L - 1);
+  else return k == L ? 0 : k;
 }
 
 /* one radix-8 DIF butterfly of the 64-point transform (two passes), twiddles from the 512-entry table */
@@ -139,18 +179,85 @@ __device__ __forceinline__ float2 ChanRotor(const float2 *tab, int2 sp, unsigned
   return float2{ca.x * cb.x - ca.y * cb.y, ca.x * cb.y + ca.y * cb.x};
 }
 
-/* the in-place FFTs of the kChanTile rows of a tile (M-point; S::RowBase places the rows) */
+constexpr float kC51 = 0.309016994374947f, kC52 = -0.809016994374947f;   /* cos(2 pi / 5), cos(4 pi / 5) */
+constexpr float kS51 = 0.951056516295154f, kS52 = 0.587785252292473f;    /* sin(2 pi / 5), sin(4 pi / 5) */
+
+/* R-point DFTs (R = 2, 5, 8: the radices of ChanPlan), forward, natural-order output; r[], i[] are overwritten */
+template <int R> __device__ __forceinline__ void ChanDft(float *r, float *i);
+template <> __device__ __forceinline__ void ChanDft<8>(float *r, float *i) { Dft8(r, i); }
+template <> __device__ __forceinline__ void ChanDft<5>(float *r, float *i) {
+  const float t1r = r[1] + r[4], t1i = i[1] + i[4], t3r = r[1] - r[4], t3i = i[1] - i[4];
+  const float t2r = r[2] + r[3], t2i = i[2] + i[3], t4r = r[2] - r[3], t4i = i[2] - i[3];
+  const float a1r = r[0] + kC51 * t1r + kC52 * t2r, a1i = i[0] + kC51 * t1i + kC52 * t2i;
+  const float a2r = r[0] + kC52 * t1r + kC51 * t2r, a2i = i[0] + kC52 * t1i + kC51 * t2i;
+  const float b1r = kS51 * t3r + kS52 * t4r, b1i = kS51 * t3i + kS52 * t4i;   /* X1, X4 = a1 -/+ j b1 */
+  const float b2r = kS52 * t3r - kS51 * t4r, b2i = kS52 * t3i - kS51 * t4i;   /* X2, X3 = a2 -/+ j b2 */
+  r[0] = r[0] + t1r + t2r; i[0] = i[0] + t1i + t2i;
+  r[1] = a1r + b1i; i[1] = a1i - b1r;
+  r[4] = a1r - b1i; i[4] = a1i + b1r;
+  r[2] = a2r + b2i; i[2] = a2i - b2r;
+  r[3] = a2r - b2i; i[3] = a2i + b2r;
+}
+template <> __device__ __forceinline__ void ChanDft<2>(float *r, float *i) {
+  const float sr = r[0] + r[1], si = i[0] + i[1];
+  r[1] = r[0] - r[1]; i[1] = i[0] - i[1];
+  r[0] = sr; i[0] = si;
+}
+
+/* butterfly b of a radix-R DIF pass that splits sub-transforms of length Ls of an L-point row (natural order):
+   inputs i0 + m Ls / R, outputs k times exp(-j 2 pi j k / Ls) from tw, the L (cos, sin) of 2 pi t / L */
+template <int L, int Ls, int R>
+__device__ __forceinline__ void ChanMixedButterfly(float2 *row, const float2 *tw, int b) {
+  constexpr int n2 = Ls / R;
+  const int j = b % n2, i0 = (b / n2) * Ls + j;
+  float r[R], im[R];
+#pragma unroll
+  for (int m = 0; m < R; ++m) {
+    const float2 x = row[i0 + m * n2];
+    r[m] = x.x;
+    im[m] = x.y;
+  }
+  ChanDft<R>(r, im);
+  row[i0] = float2{r[0], im[0]};
+#pragma unroll
+  for (int k = 1; k < R; ++k) {
+    float re = r[k], ie = im[k];
+    if (n2 > 1 && j != 0) {
+      const float2 w = tw[j * k * (L / Ls)];
+      re = r[k] * w.x + im[k] * w.y;
+      ie = im[k] * w.x - r[k] * w.y;
+    }
+    row[i0 + k * n2] = float2{re, ie};
+  }
+}
+
+/* pass kPass and the ones after it of the kChanTile rows' L-point FFTs; Ls: the sub-transform length it splits */
+template <int L, typename S, int kPass, int Ls>
+__device__ __forceinline__ void ChanMixedPasses(float2 *smem, const float2 *tw, int tid) {
+  constexpr int R = ChanPlan<L>::kRadix[kPass], kBflyPerRow = L / R, kBfly = kChanTile * kBflyPerRow;
+  for (int b = tid; b < kBfly; b += S::kThreads)
+    ChanMixedButterfly<L, Ls, R>(smem + S::RowBase(b / kBflyPerRow), tw, b % kBflyPerRow);
+  __syncthreads();
+  if constexpr (kPass + 1 < ChanPlan<L>::kPasses) ChanMixedPasses<L, S, kPass + 1, Ls / R>(smem, tw, tid);
+}
+
+/* the in-place FFTs of the kChanTile rows of a tile (M-point; S::RowBase places the rows).  tw512: the 512 (cos, sin)
+   of 2 pi k / 512, or for a mixed-radix M the M of 2 pi k / M */
 template <int M, typename S>
 __device__ __forceinline__ void ChanRowsFft(float2 *smem, const float2 *tw512, int tid) {
-  constexpr int kBflyPerRow = M / 8, kBfly = kChanTile * kBflyPerRow;
+  if constexpr (!kChanPow2<M>) {
+    ChanMixedPasses<M, S, 0, M>(smem, tw512, tid);
+  } else {
+    constexpr int kBflyPerRow = M / 8, kBfly = kChanTile * kBflyPerRow;
 #pragma unroll
-  for (int pass = 0; pass < (M == 512 ? 3 : 2); ++pass) {
-    for (int b = tid; b < kBfly; b += S::kThreads) {
-      float2 *row = smem + S::RowBase(b / kBflyPerRow);
-      if (M == 512) Radix8Butterfly<true>(row, tw512, pass, b % kBflyPerRow);
-      else Radix8Butterfly64(row, tw512, pass, b % kBflyPerRow);
+    for (int pass = 0; pass < (M == 512 ? 3 : 2); ++pass) {
+      for (int b = tid; b < kBfly; b += S::kThreads) {
+        float2 *row = smem + S::RowBase(b / kBflyPerRow);
+        if (M == 512) Radix8Butterfly<true>(row, tw512, pass, b % kBflyPerRow);
+        else Radix8Butterfly64(row, tw512, pass, b % kBflyPerRow);
+      }
+      __syncthreads();
     }
-    __syncthreads();
   }
 }
 
@@ -181,7 +288,7 @@ template <> __device__ __forceinline__ float2 *ChanSmem<short>() {
    it, and the rest of the kernel is the same for both.  h / 32768 times I is h times I / 32768 exactly, so every FMA,
    and every output bit, is that of the float instance on x = s / 32768. */
 template <int M, bool kRotate, typename T>
-__global__ void __launch_bounds__(ChanShape<M>::kThreads, M == 512 ? 2 : 4)
+__global__ void __launch_bounds__(ChanShape<M>::kThreads, ChanShape<M>::kMinBlocks)
 t41rx_chan_kernel(const T *__restrict__ capture, const T *__restrict__ tail, const float *__restrict__ taps,
                   const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
                   const int2 *__restrict__ phase, const float2 *__restrict__ rot, int m_base, int n_entries,
@@ -250,7 +357,7 @@ t41rx_chan_kernel(const T *__restrict__ capture, const T *__restrict__ tail, con
   };
   auto slot = [&](int t) {
     const int mm = g + S::kGroups * t;
-    return S::RowBase(mm) + ChanPhys<M>((mm & 1) ? (p ^ (M / 2)) : p);
+    return S::RowBase(mm) + ChanPhys<M>((mm & 1) ? ChanHalfTurn<M>(p) : p);
   };
   constexpr int kLate = S::kTimes / 2;
 #pragma unroll
@@ -301,6 +408,8 @@ struct ChanRealShape {
   static constexpr int D = M / 2;
   static constexpr int N = kChanTaps * M;
   static constexpr int kThreads = Mc >= 256 ? Mc : 256;
+  /* CTAs per SM (__launch_bounds__): 4 at M = 128, 2 at 800 (76 KiB each) and 1024, 1 at 1280 (117 KiB) */
+  static constexpr int kMinBlocks = M == 1024 || M == 800 ? 2 : M == 1280 ? 1 : 4;
   static constexpr int kGroups = kThreads / Mc;                 /* threads per branch pair */
   static constexpr int kTimes = kChanTile / kGroups;
   static constexpr int kSpan = kChanTile * D + N;               /* int16 capture samples a tile stages */
@@ -324,7 +433,7 @@ struct ChanRealShape {
 /* capture / tail: int16, 16-byte aligned; taps: h / 65536 (the 1 / 32768 of the input scale and the split's 1 / 2,
    both exact); split: (cos, sin) of 2 pi k / M, k <= M / 2; the rest as t41rx_chan_kernel.  Channel k in [0, M/2]. */
 template <int M, bool kRotate>
-__global__ void __launch_bounds__(ChanRealShape<M>::kThreads, M == 1024 ? 2 : 4)
+__global__ void __launch_bounds__(ChanRealShape<M>::kThreads, ChanRealShape<M>::kMinBlocks)
 t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restrict__ tail, const float *__restrict__ taps,
                        const float2 *__restrict__ tw512, const float2 *__restrict__ split, const int32_t *__restrict__ recv,
                        const int32_t *__restrict__ chan, const int2 *__restrict__ phase, const float2 *__restrict__ rot,
@@ -369,7 +478,7 @@ t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restric
   };
   auto slot = [&](int t) {
     const int mm = g + S::kGroups * t;
-    return S::RowBase(mm) + ChanPhys<Mc>((mm & 1) ? (p ^ (Mc / 2)) : p);
+    return S::RowBase(mm) + ChanPhys<Mc>((mm & 1) ? ChanHalfTurn<Mc>(p) : p);
   };
   constexpr int kEarlyTimes = S::kTimes - S::kLateTimes;
   /* not unrolled: interleaving the output times' loads pushes two taps out of the 64 registers at M = 1024 */
@@ -388,8 +497,8 @@ t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restric
   /* X[k] of row mm from Y[k] and Y[Mc - k] (the 1 / 2 is in the taps) */
   const float2 *w_tab = smem + S::kSplitBase;
   auto sample = [&](int mm, int k) {
-    const float2 a = smem[S::RowBase(mm) + ChanOutPos<Mc>(k & (Mc - 1))];
-    const float2 b = smem[S::RowBase(mm) + ChanOutPos<Mc>((Mc - k) & (Mc - 1))];
+    const float2 a = smem[S::RowBase(mm) + ChanOutPos<Mc>(ChanWrap<Mc>(k))];
+    const float2 b = smem[S::RowBase(mm) + ChanOutPos<Mc>(ChanWrap<Mc>(Mc - k))];
     const float2 w = w_tab[k];
     const float sr = a.x + b.x, si = a.y - b.y, dr = a.x - b.x, di = a.y + b.y;
     return float2{sr + w.x * di - w.y * dr, si - w.y * di - w.x * dr};
@@ -449,8 +558,13 @@ static void DesignChanTaps(int M, float *out) {
   for (int n = 0; n < N; ++n) out[n] = (float)(h[n] / sum);
 }
 
-static bool ChanCountOk(int n_channels) { return n_channels == 64 || n_channels == 512; }
-static bool ChanRealCountOk(int n_channels) { return n_channels == 128 || n_channels == 1024; }
+/* complex: 6.144, 30.72, 49.152, 61.44 MS/s; real: 12.288, 76.8, 98.304, 122.88 MS/s */
+static bool ChanCountOk(int n_channels) {
+  return n_channels == 64 || n_channels == 320 || n_channels == 512 || n_channels == 640;
+}
+static bool ChanRealCountOk(int n_channels) {
+  return n_channels == 128 || n_channels == 800 || n_channels == 1024 || n_channels == 1280;
+}
 
 template <typename K>
 static cudaError_t ChanSmemAttr(K plain, int plain_bytes, K rotating, int rotating_bytes) {
@@ -547,7 +661,7 @@ struct t41rx_chan {
   cudaEvent_t ev_ext = nullptr;
   bool ext_pending = false;
   float *d_taps = nullptr;       /* N (real: h / 65536, q15: h / 32768) */
-  float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512 */
+  float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512, or L of 2 pi k / L (mixed-radix FFT length L) */
   float2 *d_split = nullptr;     /* real: n_channels / 2 + 1 (cos, sin) of 2 pi k / n_channels */
   void *d_tail = nullptr;        /* the last N capture samples of the previous calls (zeros at creation) */
   int32_t *d_recv = nullptr, *d_chan = nullptr;   /* mapped receivers grouped by channel, and their channel */
@@ -605,6 +719,27 @@ struct ChanReal {
 template <typename K>
 constexpr ChanKernels kChanKernels{K::Prepare, K::Launch};
 
+/* the kernel pair of a kind at a channel count its Chan*CountOk accepts */
+template <int M>
+static ChanKernels ChanComplexKernels(ChanKind kind) {
+  return kind == ChanKind::kQ15 ? kChanKernels<ChanComplex<M, short>> : kChanKernels<ChanComplex<M, float2>>;
+}
+static ChanKernels ChanKernelsFor(ChanKind kind, int n_channels) {
+  if (kind == ChanKind::kReal)
+    switch (n_channels) {
+      case 128: return kChanKernels<ChanReal<128>>;
+      case 800: return kChanKernels<ChanReal<800>>;
+      case 1024: return kChanKernels<ChanReal<1024>>;
+      default: return kChanKernels<ChanReal<1280>>;
+    }
+  switch (n_channels) {
+    case 64: return ChanComplexKernels<64>(kind);
+    case 320: return ChanComplexKernels<320>(kind);
+    case 512: return ChanComplexKernels<512>(kind);
+    default: return ChanComplexKernels<640>(kind);
+  }
+}
+
 static int ChanQuiesce(t41rx_chan *c) {
   if (c->ext_pending) {
     if (cudaEventSynchronize(c->ev_ext) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan: synchronisation failed");
@@ -636,8 +771,8 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   const std::string f(fn);
   const bool real = kind == ChanKind::kReal;
   if (!out || !(real ? ChanRealCountOk(n_channels) : ChanCountOk(n_channels)) || n_receivers <= 0)
-    return SetApiError(T41RX_EINVAL, (f + (real ? ": bad arguments (n_channels must be 128 or 1024)"
-                                               : ": bad arguments (n_channels must be 64 or 512)")).c_str());
+    return SetApiError(T41RX_EINVAL, (f + (real ? ": bad arguments (n_channels must be 128, 800, 1024 or 1280)"
+                                               : ": bad arguments (n_channels must be 64, 320, 512 or 640)")).c_str());
   *out = nullptr;
   int n_dev = 0;
   if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev <= 0)
@@ -660,10 +795,7 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": stream/event creation failed").c_str()));
-  const bool large = n_channels == 512 || n_channels == 1024;
-  c->kernels = real ? (large ? kChanKernels<ChanReal<1024>> : kChanKernels<ChanReal<128>>)
-               : kind == ChanKind::kQ15 ? (large ? kChanKernels<ChanComplex<512, short>> : kChanKernels<ChanComplex<64, short>>)
-               : large ? kChanKernels<ChanComplex<512, float2>> : kChanKernels<ChanComplex<64, float2>>;
+  c->kernels = ChanKernelsFor(kind, n_channels);
   if (c->kernels.prepare() != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": kernel image for this GPU missing (built for sm_100a)").c_str()));
   const int N = kChanTaps * n_channels;
@@ -673,8 +805,12 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
     for (float &h : taps) h = ldexpf(h, -16);   /* x = s / 32768 and the split's 1 / 2, exact */
   if (kind == ChanKind::kQ15)
     for (float &h : taps) h = ldexpf(h, -15);   /* x = s / 32768, exact */
-  std::vector<float2> tw(512);
-  for (int k = 0; k < 512; ++k) tw[k] = float2{(float)cos(2.0 * M_PI * k / 512.0), (float)sin(2.0 * M_PI * k / 512.0)};
+  /* the row FFTs' twiddles: 2 pi k / 512 for the radix-8 lengths 64 and 512, 2 pi k / L for a mixed-radix length L */
+  const int fft_len = real ? n_channels / 2 : n_channels;
+  const int tw_len = (fft_len & (fft_len - 1)) == 0 ? 512 : fft_len;
+  std::vector<float2> tw(tw_len);
+  for (int k = 0; k < tw_len; ++k)
+    tw[k] = float2{(float)cos(2.0 * M_PI * k / tw_len), (float)sin(2.0 * M_PI * k / tw_len)};
   std::vector<float2> split(real ? n_channels / 2 + 1 : 0);
   for (size_t k = 0; k < split.size(); ++k)
     split[k] = float2{(float)cos(2.0 * M_PI * k / n_channels), (float)sin(2.0 * M_PI * k / n_channels)};
@@ -683,7 +819,7 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   for (int b = 0; b < kRotFine; ++b)
     rot[kRotCoarse + b] = float2{(float)cos(2.0 * M_PI * b / kChanOutRate), (float)sin(2.0 * M_PI * b / kChanOutRate)};
   const size_t tail_bytes = ChanSampleBytes(kind) * N;
-  if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * 512) != cudaSuccess ||
+  if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * tw_len) != cudaSuccess ||
       (real && cudaMalloc(&c->d_split, sizeof(float2) * split.size()) != cudaSuccess) ||
       cudaMalloc(&c->d_tail, tail_bytes) != cudaSuccess ||
       cudaMalloc(&c->d_recv, sizeof(int32_t) * n_receivers) != cudaSuccess ||
@@ -692,7 +828,7 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
       cudaMalloc(&c->d_rot, sizeof(float2) * rot.size()) != cudaSuccess)
     return bail(SetApiError(T41RX_ENOMEM, (f + ": device allocation failed").c_str()));
   if (cudaMemcpy(c->d_taps, taps.data(), sizeof(float) * N, cudaMemcpyHostToDevice) != cudaSuccess ||
-      cudaMemcpy(c->d_tw, tw.data(), sizeof(float2) * 512, cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy(c->d_tw, tw.data(), sizeof(float2) * tw_len, cudaMemcpyHostToDevice) != cudaSuccess ||
       (real && cudaMemcpy(c->d_split, split.data(), sizeof(float2) * split.size(), cudaMemcpyHostToDevice) != cudaSuccess) ||
       cudaMemcpy(c->d_rot, rot.data(), sizeof(float2) * rot.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
       cudaMemset(c->d_tail, 0, tail_bytes) != cudaSuccess)
@@ -844,7 +980,7 @@ int t41rx_chan_synchronize(t41rx_chan *c) {
 
 int t41rx_chan_taps(int n_channels, float *taps) {
   if (!taps || !(ChanCountOk(n_channels) || ChanRealCountOk(n_channels)))
-    return SetApiError(T41RX_EINVAL, "t41rx_chan_taps: bad arguments (n_channels must be 64, 128, 512 or 1024)");
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_taps: bad arguments (n_channels must be 64, 128, 320, 512, 640, 800, 1024 or 1280)");
   DesignChanTaps(n_channels, taps);
   return T41RX_OK;
 }

@@ -560,7 +560,7 @@ def chan_centre_real(channel):
 
 
 def chan_tune_real(n_channels, mode, freq_hz):
-    """chan_tune for a real capture (n_channels 128 or 1024): freq_hz absolute, in [0, Fs/2]; host only."""
+    """chan_tune for a real capture (n_channels 128, 800, 1024 or 1280): freq_hz absolute, in [0, Fs/2]; host only."""
     ch, nco = C.c_int32(), C.c_int32()
     _check(lib().t41rx_chan_tune_real(int(n_channels), int(mode), float(freq_hz), C.byref(ch), C.byref(nco)),
            "t41rx_chan_tune_real")
@@ -568,7 +568,7 @@ def chan_tune_real(n_channels, mode, freq_hz):
 
 
 def chan_place_real(n_channels, mode, freq_hz):
-    """chan_place for a real capture (n_channels 128 or 1024): freq_hz absolute, in [0, Fs/2]; host only."""
+    """chan_place for a real capture (n_channels 128, 800, 1024 or 1280): freq_hz absolute, in [0, Fs/2]; host only."""
     ch, shift, nco = C.c_int32(), C.c_int32(), C.c_int32()
     _check(lib().t41rx_chan_place_real(int(n_channels), int(mode), float(freq_hz), C.byref(ch), C.byref(shift),
                                        C.byref(nco)), "t41rx_chan_place_real")
@@ -578,9 +578,9 @@ def chan_place_real(n_channels, mode, freq_hz):
 class Channelizer:
     """Polyphase channelizer on one CUDA device: a wideband capture at n_channels x 96 kS/s in, the iq blocks of
     n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr().
-    real=True: an int16 real capture (n_channels 128 or 1024, channels 0 ... n_channels / 2); q15=True: a complex
-    capture of interleaved int16 (I, Q) pairs, x = (I + jQ) / 32768 (n_channels 64 or 512); else complex float
-    (n_channels 64 or 512)."""
+    real=True: an int16 real capture (n_channels 128, 800, 1024 or 1280: 12.288, 76.8, 98.304 or 122.88 MS/s; channels
+    0 ... n_channels / 2); q15=True: a complex capture of interleaved int16 (I, Q) pairs, x = (I + jQ) / 32768
+    (n_channels 64, 320, 512 or 640: 6.144, 30.72, 49.152 or 61.44 MS/s); else complex float (the same n_channels)."""
 
     def __init__(self, n_channels, n_receivers, device=0, real=False, q15=False):
         if real and q15:

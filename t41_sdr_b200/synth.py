@@ -219,17 +219,17 @@ def wideband(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
 
 
 def wideband_real(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
-    """A real capture at n_channels x 96 kS/s (n_channels 128 or 1024) as a direct-sampling ADC delivers it: int16
-    round(32768 Re z), saturated, n_blocks * 2048 * n_channels / 2 samples.  z is the sum wideband() forms with the
-    same arguments, f measured from 0 Hz, so a ("tone", f, {amp}) is amp cos(2 pi f t)."""
+    """A real capture at n_channels x 96 kS/s (n_channels 128, 800, 1024 or 1280) as a direct-sampling ADC delivers
+    it: int16 round(32768 Re z), saturated, n_blocks * 2048 * n_channels / 2 samples.  z is the sum wideband() forms
+    with the same arguments, f measured from 0 Hz, so a ("tone", f, {amp}) is amp cos(2 pi f t)."""
     z = _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block)
     return np.clip(np.round(32768.0 * z.real), -32768, 32767).astype(np.int16)
 
 
 def wideband_q15(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
-    """A complex capture at n_channels x 96 kS/s (n_channels 64 or 512) as a wideband I/Q digitizer streams it (sc16):
-    int16 [n, 2] interleaved (I, Q), round(32768 z) saturated to [-32768, 32767] per component.  z is the sum
-    wideband() forms with the same arguments, so wideband_q15 / 32768 is wideband() quantised."""
+    """A complex capture at n_channels x 96 kS/s (n_channels 64, 320, 512 or 640) as a wideband I/Q digitizer streams
+    it (sc16): int16 [n, 2] interleaved (I, Q), round(32768 z) saturated to [-32768, 32767] per component.  z is the
+    sum wideband() forms with the same arguments, so wideband_q15 / 32768 is wideband() quantised."""
     z = _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block)
     out = np.empty((z.size, 2), np.int16)
     out[:, 0] = np.clip(np.round(32768.0 * z.real), -32768, 32767)

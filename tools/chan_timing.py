@@ -1,6 +1,6 @@
 """Channelizer timing on one GPU (DESIGN §3.7 - 3.9): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
 
-    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--json OUT]
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--rates] [--json OUT]
 
 Prints the card's name and power limit (a query), then CUDA-event times of
   - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
@@ -14,6 +14,11 @@ Prints the card's name and power limit (a query), then CUDA-event times of
   - with --q15, at the same M and 1024 receivers: t41rx_chan_process_device_q15 on an interleaved int16 capture (134 MB
     at M = 512), and what a user of the float call does with such a capture: int16 -> float32 / 32768 with torch into
     a float capture, then t41rx_chan_process_device (with --shift also the q15 call with every receiver shifted),
+  - with --rates (DESIGN §3.10), every channel count beside its power-of-two neighbour: the complex float call at
+    M = 320, 512 and 640 and the real call at M = 800, 1024 and 1280, each without and with every receiver shifted.
+    The same 1024 receivers, 2 per channel on channels 0 ... 511 (at M = 320 and 800, which have fewer channels, on
+    channel (r / 2) mod 320 and mod 401), 64 blocks per call; the calls alternate between two captures, so that the
+    captures a size reads (2 x 105 MB at real M = 800, more elsewhere) do not fit the L2,
 each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
 receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
 """
@@ -51,6 +56,54 @@ def c2_params(n):
     return out
 
 
+def rate_table(g, dev, iq, sp, timed, shifts, S, T):
+    """the --rates measurements: per (kind, M) the call's time without and with every receiver shifted, and each
+    mixed-radix size against its power-of-two neighbour, per call and per capture sample"""
+    import torch
+    out = {}
+    for kind, M in (("complex", 320), ("complex", 512), ("complex", 640), ("real", 800), ("real", 1024), ("real", 1280)):
+        real = kind == "real"
+        n_cap = T * rx.BLOCK * M // 2
+        if real:
+            caps = [torch.randint(-3277, 3278, (n_cap,), generator=g, device=dev, dtype=torch.int16) for _ in range(2)]
+        else:
+            caps = [(0.1 * torch.randn((n_cap, 2), generator=g, device=dev)).contiguous() for _ in range(2)]
+        n_chan = M // 2 + 1 if real else M
+        chan = rx.Channelizer(M, S, real=real)
+        chan.set_map([(r // 2) % min(512, n_chan) for r in range(S)])
+        calls = [0]
+
+        def do():
+            chan.process_device(caps[calls[0] % 2].data_ptr(), iq.data_ptr(), T, stream=sp)
+            calls[0] += 1
+
+        t = timed(do)
+        chan.set_shift(shifts)
+        t_shift = timed(do)
+        chan.synchronize()
+        chan.close()
+        cap_bytes = n_cap * (2 if real else 8)
+        moved = cap_bytes + S * T * rx.BLOCK * 8
+        out["%s_%d" % (kind, M)] = {
+            "capture_msps": M * 96e3 / 1e6, "capture_bytes": cap_bytes, "bytes_moved": moved,
+            "chan_ms": {"median": t[0], "min": t[1], "max": t[2]},
+            "all_shifted_ms": {"median": t_shift[0], "min": t_shift[1], "max": t_shift[2]},
+            "ns_per_capture_sample": t[0] * 1e6 / n_cap,
+            "all_shifted_ns_per_capture_sample": t_shift[0] * 1e6 / n_cap,
+            "hbm_share_of_7p7_tbs": moved / (t[0] * 1e-3) / HBM_BYTES_PER_S}
+        del caps
+    for new, old in (("complex_320", "complex_512"), ("complex_640", "complex_512"), ("real_800", "real_1024"),
+                     ("real_1280", "real_1024")):
+        n, o = out[new], out[old]
+        for key, ms in (("", "chan_ms"), ("all_shifted_", "all_shifted_ms")):
+            n[key + "per_sample_over_" + old] = n[key + "ns_per_capture_sample"] / o[key + "ns_per_capture_sample"]
+            n[key + "goal_per_sample_le_" + old] = n[key + "ns_per_capture_sample"] <= o[key + "ns_per_capture_sample"]
+            if new in ("complex_640", "real_1280"):
+                n[key + "call_over_" + old] = n[ms]["median"] / o[ms]["median"]
+                n[key + "goal_call_le_1p25_of_" + old] = n[ms]["median"] <= 1.25 * o[ms]["median"]
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--channels", type=int, default=512)
@@ -61,6 +114,7 @@ def main():
     ap.add_argument("--shift", action="store_true", help="also time the channelizer with every receiver shifted")
     ap.add_argument("--real", action="store_true", help="also time the real M = 1024 channelizer")
     ap.add_argument("--q15", action="store_true", help="also time the q15 channelizer and torch conversion + float")
+    ap.add_argument("--rates", action="store_true", help="also time every channel count beside its power-of-two neighbour")
     ap.add_argument("--json", default=None, help="also write the result here")
     a = ap.parse_args()
     import torch
@@ -158,6 +212,7 @@ def main():
         for c in (chan_q15, chan_conv):
             c.synchronize()
             c.close()
+    rates = rate_table(g, dev, iq, sp, timed, shifts, S, T) if a.rates else None
     eng.synchronize()
     bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
     res = {
@@ -206,6 +261,8 @@ def main():
         if t_q15_shift:
             res["q15"]["all_shifted_ms"] = {"median": t_q15_shift[0], "min": t_q15_shift[1], "max": t_q15_shift[2]}
             res["q15"]["shift_overhead"] = t_q15_shift[0] / t_q15[0] - 1.0
+    if rates:
+        res["rates"] = rates
     print(json.dumps(res, indent=1))
     if a.json:
         with open(a.json, "w") as f:
