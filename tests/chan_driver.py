@@ -42,6 +42,24 @@ def reference_channel(x, taps, M, k, n_out):
     return np.conj(fftconvolve(y, taps.astype(np.float64))[:x.size][0:n_out * D:D])
 
 
+def reference_all_channels(x, taps, M, n_out):
+    """float64 z_k[m] of every channel k < M at once, m < n_out (complex128 [M, n_out]; a real capture's channels are
+    rows 0 .. M/2): the defining formula factored as u_p[m] = sum_q h[p + qM] x[mD - p - qM] (x[n < 0] = 0), one
+    M-point DFT of conj(u[m]) per output time, and the sign (-1)^(k m)."""
+    D, K = M // 2, taps.size // M
+    h = taps.astype(np.float64).reshape(K, M)
+    xp = np.concatenate([np.zeros(K * M, np.complex128), np.asarray(x, np.complex128)])
+    win = np.lib.stride_tricks.sliding_window_view(xp, M)      # win[j, t] = xp[j + t]
+    m = np.arange(n_out)
+    u = np.zeros((n_out, M), np.complex128)
+    for q in range(K):
+        # x[mD - p - qM] for p = 0 .. M-1 is win[mD + (K - 1 - q) M + 1] read backwards
+        u += h[q] * win[m * D + (K - 1 - q) * M + 1][:, ::-1]
+    z = np.fft.fft(np.conj(u), axis=1)
+    z[1::2, 1::2] *= -1.0
+    return z.T
+
+
 def rotate(z, phase0, shift, m0=0):
     """float64 z[m] exp(2 pi j phi / 192000), phi = (phase0 + shift (m0 + m)) mod 192000 in integers."""
     m = np.arange(z.size, dtype=np.int64) + m0
