@@ -339,6 +339,34 @@ int t41rx_chan_place_real(int n_channels, int32_t mode, double freq_hz, int32_t 
  * aligned; iq and cuda_stream as t41rx_chan_process_device. */
 int t41rx_chan_create_q15(t41rx_chan **out, int n_channels, int n_receivers, int device);
 int t41rx_chan_process_device_q15(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream);
+/* Diversity (DESIGN §3.11): n_inputs in {2, 3, 4} coherent captures of one kind, sampled on one clock (sample n of every
+ * input is the same instant: two to four ADCs of one digitizer), and one complex weight per (receiver, input).
+ * Receiver r mapped to channel k gets
+ *     iq_r[m] = rot_r(m) sum_a w[r][a] z^(a)_k[m]
+ * where z^(a)_k is exactly what the single-input channelizer of that kind delivers for input a (same prototype, D,
+ * conjugate; each input keeps its own tail) and rot_r is the fine-tuning rotation with its phase rule.  The weights
+ * multiply the channel as delivered, after the conjugate: an input-1 copy c x of a complex interferer x on input 0
+ * appears in channel k as conj(c) times input 0's, so it is nulled by w[r][1] = -w[r][0] / conj(c).  Each receiver has
+ * its own weights, so each can null a different source or none.
+ * kind: T41RX_CHAN_FLOAT, _Q15 or _REAL, with the n_channels that kind's create call takes.  Every receiver starts
+ * unmapped, unshifted and with the default weights w[r][0] = 1, w[r][a > 0] = 0, with which it gets the single-input
+ * channelizer's output for input 0 bit for bit.  EINVAL for an unknown kind, an n_channels the kind does not take or
+ * n_inputs outside 2 ... 4; ENODEV without a CUDA device.
+ * t41rx_chan_set_weights: receivers [first, first + count) take w[i][a] = (w[2 (i n_inputs + a)], w[2 (i n_inputs + a)
+ * + 1]) (re, im), finite (EINVAL otherwise, and on a single-input channelizer).  Effective from the next call; it waits
+ * for the channelizer's calls like set_map.  Weights change in a step at the call boundary: there is no ramp.
+ * t41rx_chan_process_device_diversity: captures[a], a < n_inputs, DEVICE pointers with the layout and alignment of the
+ * kind's process call (float: 8-byte, int16: 16-byte aligned); iq, the n_blocks limit, cuda_stream and the ordering
+ * contract as t41rx_chan_process_device.  set_map, set_shift, synchronize, destroy and tune / place are the kind's.  A
+ * diversity channelizer rejects the three single-input process calls, and a single-input one the diversity call
+ * (EINVAL, naming the entry point it takes). */
+#define T41RX_CHAN_FLOAT 0   /* kinds of t41rx_chan_create, _q15, _real */
+#define T41RX_CHAN_Q15   1
+#define T41RX_CHAN_REAL  2
+int t41rx_chan_create_diversity(t41rx_chan **out, int kind, int n_channels, int n_inputs, int n_receivers, int device);
+int t41rx_chan_set_weights(t41rx_chan *c, int first, int count, const float *w);
+int t41rx_chan_process_device_diversity(t41rx_chan *c, const void *const *captures, float *iq, int n_blocks,
+                                        void *cuda_stream);
 
 /* Audio-spectrum + S-meter by-product of the row-producing blocks (Process.cpp:550-570; NFM: 791-805):
  *   audio_ypixel      int32 [n_streams][n_rows][270]  audioYPixel[k], k < AUDIO_SPEC_BOX_W - 2 (Process.cpp:34,555)

@@ -42,6 +42,11 @@
  * are 2^a 5^b.  Their rows are in natural order and run the mixed-radix DIF passes of ChanPlan (radix 5 beside 8, a
  * radix-2 pass where the factorisation needs it); X[k] ends at the mixed-radix digit reversal of k.  The power-of-two
  * instances never reach that code (if constexpr on kChanPow2), so their SASS is the same as before it was added.
+ *
+ * Diversity (t41rx_chan_create_diversity, DESIGN §3.11): 2 - 4 coherent captures of one kind, receiver r getting
+ * rot_r(m) sum_a w[r][a] z^(a)_k[m].  A call runs the kind's kernel once per input on one stream, input 0's pass
+ * storing v w f and the others adding it to iq (the kStore template parameter, behind if constexpr); each input keeps
+ * its own tail.
  */
 #include <cuda_runtime.h>
 
@@ -179,6 +184,71 @@ __device__ __forceinline__ float2 ChanRotor(const float2 *tab, int2 sp, unsigned
   return float2{ca.x * cb.x - ca.y * cb.y, ca.x * cb.y + ca.y * cb.x};
 }
 
+/* the store stage of a kernel instance (DESIGN §3.11): kChanPlain writes the (rotated) sample, as a single-input
+   channelizer does; a diversity call runs the kernel once per input, kChanWeighted for input 0 (writes v w f) and
+   kChanAccumulate for the others (adds v w f to iq) */
+constexpr int kChanPlain = 0, kChanWeighted = 1, kChanAccumulate = 2;
+
+/* complex products with every rounding spelled out (__fmul_rn / __fmaf_rn are never contracted), so that the weighted
+   instances round as the plain ones' SASS does whatever the compiler makes of their context:
+   ChanMulRn(v, f) = (fma(v.x, f.x, -(v.y f.y)), fma(v.x, f.y, v.y f.x)), the plain store loop's v f;
+   ChanRotorRn is ChanRotor's ca cb = (fma(ca.x, cb.x, -(ca.y cb.y)), fma(ca.y, cb.x, ca.x cb.y)) */
+__device__ __forceinline__ float2 ChanMulRn(float2 v, float2 f) {
+  return float2{__fmaf_rn(v.x, f.x, -__fmul_rn(v.y, f.y)), __fmaf_rn(v.x, f.y, __fmul_rn(v.y, f.x))};
+}
+__device__ __forceinline__ float2 ChanRotorRn(const float2 *tab, int2 sp, unsigned m_abs) {
+  const unsigned phi = ChanPhase((unsigned)sp.x, m_abs, (unsigned)sp.y), a = phi / kRotFine;
+  const float2 ca = tab[a], cb = tab[kRotCoarse + (phi - a * kRotFine)];
+  return float2{__fmaf_rn(ca.x, cb.x, -__fmul_rn(ca.y, cb.y)), __fmaf_rn(ca.y, cb.x, __fmul_rn(ca.x, cb.y))};
+}
+
+/* a weighted instance's sample of one entry: v, its rotation factor f (from ChanRotorRn) and whether the entry is
+   rotated (its phase is not identically 0) */
+struct ChanSample {
+  float2 v, f;
+  bool rotated;
+};
+
+/* the store loop of the weighted instances: entry e = w / kChanTile, w = tid, tid + kThreads, ... < n_entries x
+   kChanTile, four at a time; sample(e) is its ChanSample, iq the thread's sample of receiver 0's run (the thread
+   always stores the same sample of the tile).  g = w f is formed once per sample; selects keep the default weights
+   bit-exact: w = (1, 0) takes g = f, so v g is the plain instance's v f bit for bit, an entry with w = (1, 0) and no
+   rotation stores v itself, and a zero weight leaves the accumulating pass's sample untouched rather than adding +0
+   (-0 + 0 is +0).  The accumulating pass loads the four old samples before it stores any: with a store ahead of each
+   next load (the compiler cannot tell the entries' addresses apart) every entry would wait for its own load */
+template <int kStore, int kThreads, typename Sample>
+__device__ __forceinline__ void ChanWeightedLoop(float2 *__restrict__ iq, const int32_t *__restrict__ recv,
+                                                 const float2 *__restrict__ weight, int n_entries, int n_blocks, int tid,
+                                                 Sample sample) {
+  constexpr int kBatch = 4;
+  const int n = n_entries * kChanTile;
+  for (int w0 = tid; w0 < n; w0 += kBatch * kThreads) {
+    float2 *dst[kBatch];
+    float2 wt[kBatch], old[kBatch];
+#pragma unroll
+    for (int u = 0; u < kBatch; ++u) {
+      const int e = min(w0 + u * kThreads, n - 1) / kChanTile;
+      dst[u] = iq + (long long)__ldg(recv + e) * n_blocks * T41RX_BLOCK_SAMPLES;
+      wt[u] = __ldg(weight + e);
+      if (kStore == kChanAccumulate && w0 + u * kThreads < n && (wt[u].x != 0.f || wt[u].y != 0.f)) old[u] = *dst[u];
+    }
+#pragma unroll
+    for (int u = 0; u < kBatch; ++u) {
+      if (w0 + u * kThreads >= n) break;
+      const float2 w = wt[u];
+      const bool unit = w.x == 1.f && w.y == 0.f;
+      if (kStore == kChanAccumulate && w.x == 0.f && w.y == 0.f) continue;
+      const ChanSample s = sample((w0 + u * kThreads) / kChanTile);
+      const float2 g = !s.rotated ? w : unit ? s.f : ChanMulRn(w, s.f);
+      const float2 p = ChanMulRn(s.v, g);
+      if constexpr (kStore == kChanWeighted)
+        *dst[u] = !s.rotated && unit ? s.v : p;
+      else
+        *dst[u] = float2{__fadd_rn(old[u].x, p.x), __fadd_rn(old[u].y, p.y)};
+    }
+  }
+}
+
 constexpr float kC51 = 0.309016994374947f, kC52 = -0.809016994374947f;   /* cos(2 pi / 5), cos(4 pi / 5) */
 constexpr float kS51 = 0.951056516295154f, kS52 = 0.587785252292473f;    /* sin(2 pi / 5), sin(4 pi / 5) */
 
@@ -283,16 +353,18 @@ template <> __device__ __forceinline__ float2 *ChanSmem<short>() {
    channel (CSR order) and the channel of each; phase: each entry's (shift, P) in [0, 192000), or null when no entry is
    rotated; rot: the 480 + 400 factors of the rotation table; m_base: outputs before this call, mod 192000;
    iq: [n_receivers][n_blocks][2048].  kRotate = false (no entry rotated) is the kernel without fine tuning.
+   kStore: the store stage (ChanWeightedLoop); weight: each entry's weight for this pass's input, in the order of
+   recv (read by the weighted instances only).
    The int16 span goes through registers (16-byte loads of four pairs) and lands converted, (I, Q) as integer-valued
    floats, where the float span is staged: each sample is converted once, not at each of the ~9 branch loads that read
    it, and the rest of the kernel is the same for both.  h / 32768 times I is h times I / 32768 exactly, so every FMA,
    and every output bit, is that of the float instance on x = s / 32768. */
-template <int M, bool kRotate, typename T>
+template <int M, bool kRotate, typename T, int kStore>
 __global__ void __launch_bounds__(ChanShape<M>::kThreads, ChanShape<M>::kMinBlocks)
 t41rx_chan_kernel(const T *__restrict__ capture, const T *__restrict__ tail, const float *__restrict__ taps,
                   const float2 *__restrict__ tw512, const int32_t *__restrict__ recv, const int32_t *__restrict__ chan,
                   const int2 *__restrict__ phase, const float2 *__restrict__ rot, int m_base, int n_entries,
-                  float2 *__restrict__ iq, int n_blocks) {
+                  float2 *__restrict__ iq, int n_blocks, const float2 *__restrict__ weight) {
   using S = ChanShape<M>;
   float2 *smem = ChanSmem<T>();
   const int tid = threadIdx.x;
@@ -377,6 +449,21 @@ t41rx_chan_kernel(const T *__restrict__ capture, const T *__restrict__ tail, con
      they compile to different (longer) code in every instance of this kernel. */
   const long long blk = m0 / T41RX_BLOCK_SAMPLES;
   const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
+  if constexpr (kStore != kChanPlain) {
+    const int mm = tid % kChanTile;
+    const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
+    ChanWeightedLoop<kStore, S::kThreads>(iq + (blk * T41RX_BLOCK_SAMPLES + s0 + mm), recv, weight, n_entries, n_blocks,
+                                          tid, [&](int e) {
+      const float2 v = smem[S::RowBase(mm) + ChanOutPos<M>(__ldg(chan + e))];
+      if constexpr (!kRotate) {
+        return ChanSample{v, float2{1.f, 0.f}, false};
+      } else {
+        const int2 sp = __ldg(phase + e);
+        return ChanSample{v, ChanRotorRn(smem + S::kRotBase, sp, m_abs), (sp.x | sp.y) != 0};
+      }
+    });
+    return;
+  }
   if (!kRotate) {
     for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
       const int e = w / kChanTile, mm = w % kChanTile;
@@ -432,12 +519,12 @@ struct ChanRealShape {
 
 /* capture / tail: int16, 16-byte aligned; taps: h / 65536 (the 1 / 32768 of the input scale and the split's 1 / 2,
    both exact); split: (cos, sin) of 2 pi k / M, k <= M / 2; the rest as t41rx_chan_kernel.  Channel k in [0, M/2]. */
-template <int M, bool kRotate>
+template <int M, bool kRotate, int kStore>
 __global__ void __launch_bounds__(ChanRealShape<M>::kThreads, ChanRealShape<M>::kMinBlocks)
 t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restrict__ tail, const float *__restrict__ taps,
                        const float2 *__restrict__ tw512, const float2 *__restrict__ split, const int32_t *__restrict__ recv,
                        const int32_t *__restrict__ chan, const int2 *__restrict__ phase, const float2 *__restrict__ rot,
-                       int m_base, int n_entries, float2 *__restrict__ iq, int n_blocks) {
+                       int m_base, int n_entries, float2 *__restrict__ iq, int n_blocks, const float2 *__restrict__ weight) {
   using S = ChanRealShape<M>;
   constexpr int Mc = S::Mc;
   extern __shared__ float2 smem[];
@@ -506,6 +593,20 @@ t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restric
   const long long blk = m0 / T41RX_BLOCK_SAMPLES;
   const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
   const int mm = tid % kChanTile;    /* w % kChanTile below: kThreads is a multiple of kChanTile */
+  if constexpr (kStore != kChanPlain) {
+    const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
+    ChanWeightedLoop<kStore, S::kThreads>(iq + (blk * T41RX_BLOCK_SAMPLES + s0 + mm), recv, weight, n_entries, n_blocks,
+                                          tid, [&](int e) {
+      const float2 v = sample(mm, __ldg(chan + e));
+      if constexpr (!kRotate) {
+        return ChanSample{v, float2{1.f, 0.f}, false};
+      } else {
+        const int2 sp = __ldg(phase + e);
+        return ChanSample{v, ChanRotorRn(smem + S::kRotBase, sp, m_abs), (sp.x | sp.y) != 0};
+      }
+    });
+    return;
+  }
   if (!kRotate) {
     for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
       const int e = w / kChanTile;
@@ -631,19 +732,13 @@ static size_t ChanSampleBytes(ChanKind kind) {
   return kind == ChanKind::kFloat ? sizeof(float2) : kind == ChanKind::kReal ? sizeof(int16_t) : 2 * sizeof(int16_t);
 }
 
-/* fn was called on a channelizer of another kind: EINVAL, naming the entry point this one takes */
-static int ChanWrongKind(const char *fn, ChanKind kind) {
-  const char *takes = kind == ChanKind::kFloat ? ": a complex float channelizer takes t41rx_chan_process_device"
-                      : kind == ChanKind::kReal ? ": a real channelizer takes t41rx_chan_process_device_real"
-                                                : ": a q15 channelizer takes t41rx_chan_process_device_q15";
-  return SetApiError(T41RX_EINVAL, (std::string(fn) + takes).c_str());
-}
-
-/* a channelizer's kernel pair (without and with fine tuning), chosen by kind and M at creation: prepare raises the
-   pair's dynamic shared memory limits, launch enqueues one call */
+/* a channelizer's kernels (without and with fine tuning, in each store mode), chosen by kind and M at creation: prepare
+   raises their dynamic shared memory limits, launch enqueues one pass over one input: capture and tail are that
+   input's, store its kChanPlain / kChanWeighted / kChanAccumulate, weight its entries' weights */
 struct ChanKernels {
   cudaError_t (*prepare)();
-  cudaError_t (*launch)(const t41rx_chan *c, const void *capture, float2 *iq, int n_blocks, cudaStream_t st);
+  cudaError_t (*launch)(const t41rx_chan *c, const void *capture, const void *tail, int store, const float2 *weight,
+                        float2 *iq, int n_blocks, cudaStream_t st);
 };
 
 }  // namespace t41rx
@@ -655,6 +750,7 @@ struct t41rx_chan {
   int n_channels = 0;
   int n_receivers = 0;
   ChanKind kind = ChanKind::kFloat;
+  int n_inputs = 1;              /* 2 .. 4: a diversity channelizer (t41rx_chan_create_diversity) */
   cudaStream_t stream = nullptr;
   /* t41rx_chan_process_device may enqueue on a caller-supplied stream: its end is recorded here, and set_map /
      synchronize / destroy wait for it (the ordering contract of t41rx_process_device) */
@@ -663,81 +759,129 @@ struct t41rx_chan {
   float *d_taps = nullptr;       /* N (real: h / 65536, q15: h / 32768) */
   float2 *d_tw = nullptr;        /* 512 (cos, sin) of 2 pi k / 512, or L of 2 pi k / L (mixed-radix FFT length L) */
   float2 *d_split = nullptr;     /* real: n_channels / 2 + 1 (cos, sin) of 2 pi k / n_channels */
-  void *d_tail = nullptr;        /* the last N capture samples of the previous calls (zeros at creation) */
+  void *d_tail = nullptr;        /* per input, the last N capture samples of the previous calls (zeros at creation) */
   int32_t *d_recv = nullptr, *d_chan = nullptr;   /* mapped receivers grouped by channel, and their channel */
   int2 *d_phase = nullptr;       /* each entry's (shift, P), in the order of d_recv */
+  float2 *d_weight = nullptr;    /* diversity: [n_inputs][n_receivers], input a's weight of each entry, in the order of d_recv */
   float2 *d_rot = nullptr;       /* 480 + 400: exp(j 2 pi a / 480), exp(j 2 pi b / 192000) */
   int n_entries = 0;
   bool any_rotated = false;      /* some entry's phase is not identically 0 */
   std::vector<int32_t> map;      /* receiver -> channel or -1 */
   std::vector<int32_t> shift, p0;   /* receiver -> shift and phase offset P, both in [0, 192000) */
+  std::vector<float2> weight;    /* diversity: [n_receivers][n_inputs], (1, 0) for input 0 and 0 for the others at creation */
   int m_done = 0;                /* outputs produced since creation, mod 192000 */
   ChanKernels kernels{};
 };
+
+/* fn was called on a channelizer of another kind, or with a diversity channelizer's call on a single-input one or the
+   other way round: EINVAL, naming the entry point this one takes */
+static int ChanWrongKind(const char *fn, const t41rx_chan *c) {
+  const char *takes = c->n_inputs > 1 ? ": a diversity channelizer takes t41rx_chan_process_device_diversity"
+                      : c->kind == ChanKind::kFloat ? ": a complex float channelizer takes t41rx_chan_process_device"
+                      : c->kind == ChanKind::kReal  ? ": a real channelizer takes t41rx_chan_process_device_real"
+                                                    : ": a q15 channelizer takes t41rx_chan_process_device_q15";
+  return SetApiError(T41RX_EINVAL, (std::string(fn) + takes).c_str());
+}
+
+/* K::Pass<kStore> launches the kernel of one store mode, the one without or with fine tuning by c->any_rotated.  A
+   single-input channelizer's kernels are the plain ones, a diversity channelizer's the two weighted modes.  They are
+   kept apart (kDiversity) so that the plain instances are instantiated first and in the order they always were: the
+   compiler's code for the M = 320 and 512 instances depends on where the other instances fall in the module */
+template <typename K, bool kDiversity>
+static cudaError_t ChanPrepare() {
+  if constexpr (!kDiversity) {
+    return K::template PrepareStore<kChanPlain>();
+  } else {
+    const cudaError_t e = K::template PrepareStore<kChanWeighted>();
+    return e == cudaSuccess ? K::template PrepareStore<kChanAccumulate>() : e;
+  }
+}
+template <typename K, bool kDiversity>
+static cudaError_t ChanLaunch(const t41rx_chan *c, const void *capture, const void *tail, int store,
+                              const float2 *weight, float2 *iq, int n_blocks, cudaStream_t st) {
+  if constexpr (!kDiversity) K::template Pass<kChanPlain>(c, capture, tail, weight, iq, n_blocks, st);
+  else if (store == kChanWeighted) K::template Pass<kChanWeighted>(c, capture, tail, weight, iq, n_blocks, st);
+  else K::template Pass<kChanAccumulate>(c, capture, tail, weight, iq, n_blocks, st);
+  return cudaGetLastError();
+}
 
 /* T = float2 (t41rx_chan_create) or short (t41rx_chan_create_q15) */
 template <int M, typename T>
 struct ChanComplex {
   using S = ChanShape<M>;
-  static cudaError_t Prepare() {
-    return ChanSmemAttr(t41rx_chan_kernel<M, false, T>, S::kSmemBytes, t41rx_chan_kernel<M, true, T>, S::kSmemRotBytes);
+  template <int kStore>
+  static cudaError_t PrepareStore() {
+    return ChanSmemAttr(t41rx_chan_kernel<M, false, T, kStore>, S::kSmemBytes, t41rx_chan_kernel<M, true, T, kStore>,
+                        S::kSmemRotBytes);
   }
-  static cudaError_t Launch(const t41rx_chan *c, const void *capture, float2 *iq, int n_blocks, cudaStream_t st) {
+  template <int kStore>
+  static void Pass(const t41rx_chan *c, const void *capture, const void *tail, const float2 *weight, float2 *iq,
+                   int n_blocks, cudaStream_t st) {
     const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
-    const T *cap = (const T *)capture, *tail = (const T *)c->d_tail;
+    const T *cap = (const T *)capture, *tl = (const T *)tail;
     if (c->any_rotated)
-      t41rx_chan_kernel<M, true, T><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
-          cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->d_phase, c->d_rot, c->m_done, c->n_entries, iq, n_blocks);
+      t41rx_chan_kernel<M, true, T, kStore><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
+          cap, tl, c->d_taps, c->d_tw, c->d_recv, c->d_chan, c->d_phase, c->d_rot, c->m_done, c->n_entries, iq, n_blocks,
+          weight);
     else
-      t41rx_chan_kernel<M, false, T><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
-          cap, tail, c->d_taps, c->d_tw, c->d_recv, c->d_chan, nullptr, c->d_rot, c->m_done, c->n_entries, iq, n_blocks);
-    return cudaGetLastError();
+      t41rx_chan_kernel<M, false, T, kStore><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
+          cap, tl, c->d_taps, c->d_tw, c->d_recv, c->d_chan, nullptr, c->d_rot, c->m_done, c->n_entries, iq, n_blocks,
+          weight);
   }
 };
 
 template <int M>
 struct ChanReal {
   using S = ChanRealShape<M>;
-  static cudaError_t Prepare() {
-    return ChanSmemAttr(t41rx_chan_real_kernel<M, false>, S::kSmemBytes, t41rx_chan_real_kernel<M, true>, S::kSmemRotBytes);
+  template <int kStore>
+  static cudaError_t PrepareStore() {
+    return ChanSmemAttr(t41rx_chan_real_kernel<M, false, kStore>, S::kSmemBytes, t41rx_chan_real_kernel<M, true, kStore>,
+                        S::kSmemRotBytes);
   }
-  static cudaError_t Launch(const t41rx_chan *c, const void *capture, float2 *iq, int n_blocks, cudaStream_t st) {
+  template <int kStore>
+  static void Pass(const t41rx_chan *c, const void *capture, const void *tail, const float2 *weight, float2 *iq,
+                   int n_blocks, cudaStream_t st) {
     const int tiles = n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
-    const short *cap = (const short *)capture, *tail = (const short *)c->d_tail;
+    const short *cap = (const short *)capture, *tl = (const short *)tail;
     if (c->any_rotated)
-      t41rx_chan_real_kernel<M, true><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
-          cap, tail, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, c->d_phase, c->d_rot, c->m_done, c->n_entries,
-          iq, n_blocks);
+      t41rx_chan_real_kernel<M, true, kStore><<<tiles, S::kThreads, S::kSmemRotBytes, st>>>(
+          cap, tl, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, c->d_phase, c->d_rot, c->m_done, c->n_entries,
+          iq, n_blocks, weight);
     else
-      t41rx_chan_real_kernel<M, false><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
-          cap, tail, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, nullptr, c->d_rot, c->m_done, c->n_entries, iq,
-          n_blocks);
-    return cudaGetLastError();
+      t41rx_chan_real_kernel<M, false, kStore><<<tiles, S::kThreads, S::kSmemBytes, st>>>(
+          cap, tl, c->d_taps, c->d_tw, c->d_split, c->d_recv, c->d_chan, nullptr, c->d_rot, c->m_done, c->n_entries, iq,
+          n_blocks, weight);
   }
 };
 
-template <typename K>
-constexpr ChanKernels kChanKernels{K::Prepare, K::Launch};
+template <typename K, bool kDiversity>
+constexpr ChanKernels kChanKernels{ChanPrepare<K, kDiversity>, ChanLaunch<K, kDiversity>};
 
-/* the kernel pair of a kind at a channel count its Chan*CountOk accepts */
-template <int M>
+/* the kernels of a kind at a channel count its Chan*CountOk accepts */
+template <int M, bool kDiversity>
 static ChanKernels ChanComplexKernels(ChanKind kind) {
-  return kind == ChanKind::kQ15 ? kChanKernels<ChanComplex<M, short>> : kChanKernels<ChanComplex<M, float2>>;
+  return kind == ChanKind::kQ15 ? kChanKernels<ChanComplex<M, short>, kDiversity>
+                                : kChanKernels<ChanComplex<M, float2>, kDiversity>;
 }
-static ChanKernels ChanKernelsFor(ChanKind kind, int n_channels) {
+template <bool kDiversity>
+static ChanKernels ChanKernelsOf(ChanKind kind, int n_channels) {
   if (kind == ChanKind::kReal)
     switch (n_channels) {
-      case 128: return kChanKernels<ChanReal<128>>;
-      case 800: return kChanKernels<ChanReal<800>>;
-      case 1024: return kChanKernels<ChanReal<1024>>;
-      default: return kChanKernels<ChanReal<1280>>;
+      case 128: return kChanKernels<ChanReal<128>, kDiversity>;
+      case 800: return kChanKernels<ChanReal<800>, kDiversity>;
+      case 1024: return kChanKernels<ChanReal<1024>, kDiversity>;
+      default: return kChanKernels<ChanReal<1280>, kDiversity>;
     }
   switch (n_channels) {
-    case 64: return ChanComplexKernels<64>(kind);
-    case 320: return ChanComplexKernels<320>(kind);
-    case 512: return ChanComplexKernels<512>(kind);
-    default: return ChanComplexKernels<640>(kind);
+    case 64: return ChanComplexKernels<64, kDiversity>(kind);
+    case 320: return ChanComplexKernels<320, kDiversity>(kind);
+    case 512: return ChanComplexKernels<512, kDiversity>(kind);
+    default: return ChanComplexKernels<640, kDiversity>(kind);
   }
+}
+static ChanKernels ChanKernelsFor(ChanKind kind, int n_channels, int n_inputs) {
+  if (n_inputs == 1) return ChanKernelsOf<false>(kind, n_channels);
+  return ChanKernelsOf<true>(kind, n_channels);
 }
 
 static int ChanQuiesce(t41rx_chan *c) {
@@ -756,7 +900,7 @@ void t41rx_chan_destroy(t41rx_chan *c) {
   cudaSetDevice(c->device);
   if (c->ext_pending && c->ev_ext) cudaEventSynchronize(c->ev_ext);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  void *bufs[] = {c->d_taps, c->d_tw, c->d_split, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_rot};
+  void *bufs[] = {c->d_taps, c->d_tw, c->d_split, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_weight, c->d_rot};
   for (void *b : bufs)
     if (b) cudaFree(b);
   if (c->ev_ext) cudaEventDestroy(c->ev_ext);
@@ -766,8 +910,10 @@ void t41rx_chan_destroy(t41rx_chan *c) {
 
 }  // extern "C"
 
-/* t41rx_chan_create / _create_real / _create_q15; fn names the entry point in error messages */
-static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_channels, int n_receivers, int device) {
+/* t41rx_chan_create / _create_real / _create_q15 (n_inputs 1) and _create_diversity; fn names the entry point in
+   error messages */
+static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_channels, int n_inputs, int n_receivers,
+                      int device) {
   const std::string f(fn);
   const bool real = kind == ChanKind::kReal;
   if (!out || !(real ? ChanRealCountOk(n_channels) : ChanCountOk(n_channels)) || n_receivers <= 0)
@@ -785,9 +931,14 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   c->n_channels = n_channels;
   c->n_receivers = n_receivers;
   c->kind = kind;
+  c->n_inputs = n_inputs;
   c->map.assign(n_receivers, -1);
   c->shift.assign(n_receivers, 0);
   c->p0.assign(n_receivers, 0);
+  if (n_inputs > 1) {
+    c->weight.assign((size_t)n_receivers * n_inputs, float2{0.f, 0.f});
+    for (int r = 0; r < n_receivers; ++r) c->weight[(size_t)r * n_inputs] = float2{1.f, 0.f};
+  }
   auto bail = [&](int code) {
     t41rx_chan_destroy(c);
     return code;
@@ -795,7 +946,7 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": stream/event creation failed").c_str()));
-  c->kernels = ChanKernelsFor(kind, n_channels);
+  c->kernels = ChanKernelsFor(kind, n_channels, n_inputs);
   if (c->kernels.prepare() != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": kernel image for this GPU missing (built for sm_100a)").c_str()));
   const int N = kChanTaps * n_channels;
@@ -818,13 +969,14 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   for (int a = 0; a < kRotCoarse; ++a) rot[a] = float2{(float)cos(2.0 * M_PI * a / kRotCoarse), (float)sin(2.0 * M_PI * a / kRotCoarse)};
   for (int b = 0; b < kRotFine; ++b)
     rot[kRotCoarse + b] = float2{(float)cos(2.0 * M_PI * b / kChanOutRate), (float)sin(2.0 * M_PI * b / kChanOutRate)};
-  const size_t tail_bytes = ChanSampleBytes(kind) * N;
+  const size_t tail_bytes = ChanSampleBytes(kind) * N * n_inputs;
   if (cudaMalloc(&c->d_taps, sizeof(float) * N) != cudaSuccess || cudaMalloc(&c->d_tw, sizeof(float2) * tw_len) != cudaSuccess ||
       (real && cudaMalloc(&c->d_split, sizeof(float2) * split.size()) != cudaSuccess) ||
       cudaMalloc(&c->d_tail, tail_bytes) != cudaSuccess ||
       cudaMalloc(&c->d_recv, sizeof(int32_t) * n_receivers) != cudaSuccess ||
       cudaMalloc(&c->d_chan, sizeof(int32_t) * n_receivers) != cudaSuccess ||
       cudaMalloc(&c->d_phase, sizeof(int2) * n_receivers) != cudaSuccess ||
+      (n_inputs > 1 && cudaMalloc(&c->d_weight, sizeof(float2) * n_receivers * n_inputs) != cudaSuccess) ||
       cudaMalloc(&c->d_rot, sizeof(float2) * rot.size()) != cudaSuccess)
     return bail(SetApiError(T41RX_ENOMEM, (f + ": device allocation failed").c_str()));
   if (cudaMemcpy(c->d_taps, taps.data(), sizeof(float) * N, cudaMemcpyHostToDevice) != cudaSuccess ||
@@ -840,21 +992,33 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
 extern "C" {
 
 int t41rx_chan_create(t41rx_chan **out, int n_channels, int n_receivers, int device) {
-  return ChanCreate("t41rx_chan_create", ChanKind::kFloat, out, n_channels, n_receivers, device);
+  return ChanCreate("t41rx_chan_create", ChanKind::kFloat, out, n_channels, 1, n_receivers, device);
 }
 
 int t41rx_chan_create_real(t41rx_chan **out, int n_channels, int n_receivers, int device) {
-  return ChanCreate("t41rx_chan_create_real", ChanKind::kReal, out, n_channels, n_receivers, device);
+  return ChanCreate("t41rx_chan_create_real", ChanKind::kReal, out, n_channels, 1, n_receivers, device);
 }
 
 int t41rx_chan_create_q15(t41rx_chan **out, int n_channels, int n_receivers, int device) {
-  return ChanCreate("t41rx_chan_create_q15", ChanKind::kQ15, out, n_channels, n_receivers, device);
+  return ChanCreate("t41rx_chan_create_q15", ChanKind::kQ15, out, n_channels, 1, n_receivers, device);
+}
+
+int t41rx_chan_create_diversity(t41rx_chan **out, int kind, int n_channels, int n_inputs, int n_receivers, int device) {
+  const char *fn = "t41rx_chan_create_diversity";
+  if (kind != T41RX_CHAN_FLOAT && kind != T41RX_CHAN_Q15 && kind != T41RX_CHAN_REAL)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_create_diversity: bad arguments (kind must be T41RX_CHAN_FLOAT, "
+                                     "T41RX_CHAN_Q15 or T41RX_CHAN_REAL)");
+  if (n_inputs < 2 || n_inputs > 4)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_create_diversity: bad arguments (n_inputs must be 2, 3 or 4)");
+  const ChanKind k = kind == T41RX_CHAN_FLOAT ? ChanKind::kFloat : kind == T41RX_CHAN_Q15 ? ChanKind::kQ15 : ChanKind::kReal;
+  return ChanCreate(fn, k, out, n_channels, n_inputs, n_receivers, device);
 }
 
 }  // extern "C"
 
-/* the map, shifts and phase offsets as the kernel reads them (after ChanQuiesce): CSR order, receivers grouped by
-   channel, ascending within a channel, each entry with its channel and (shift, P) */
+/* the map, shifts, phase offsets and weights as the kernel reads them (after ChanQuiesce): CSR order, receivers grouped
+   by channel, ascending within a channel, each entry with its channel and (shift, P); a diversity channelizer's
+   weights input by input, input a's n_entries from d_weight + a * n_entries */
 static int ChanUpload(t41rx_chan *c, const char *what) {
   std::vector<int32_t> start(c->n_channels + 1, 0);
   for (int32_t k : c->map)
@@ -863,6 +1027,7 @@ static int ChanUpload(t41rx_chan *c, const char *what) {
   const int n = start[c->n_channels];
   std::vector<int32_t> recv(std::max(n, 1)), chan(std::max(n, 1)), fill(start.begin(), start.end() - 1);
   std::vector<int2> phase(std::max(n, 1));
+  std::vector<float2> weight((size_t)std::max(n, 1) * (c->n_inputs > 1 ? c->n_inputs : 0));
   bool any = false;
   for (int r = 0; r < c->n_receivers; ++r)
     if (c->map[r] >= 0) {
@@ -870,11 +1035,15 @@ static int ChanUpload(t41rx_chan *c, const char *what) {
       recv[e] = r;
       chan[e] = c->map[r];
       phase[e] = int2{c->shift[r], c->p0[r]};
+      if (c->n_inputs > 1)
+        for (int a = 0; a < c->n_inputs; ++a) weight[(size_t)a * n + e] = c->weight[(size_t)r * c->n_inputs + a];
       any = any || c->shift[r] != 0 || c->p0[r] != 0;
     }
   if (n > 0 && (cudaMemcpy(c->d_recv, recv.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
                 cudaMemcpy(c->d_chan, chan.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
-                cudaMemcpy(c->d_phase, phase.data(), sizeof(int2) * n, cudaMemcpyHostToDevice) != cudaSuccess)) {
+                cudaMemcpy(c->d_phase, phase.data(), sizeof(int2) * n, cudaMemcpyHostToDevice) != cudaSuccess ||
+                (c->n_inputs > 1 && cudaMemcpy(c->d_weight, weight.data(), sizeof(float2) * n * c->n_inputs,
+                                               cudaMemcpyHostToDevice) != cudaSuccess))) {
     c->n_entries = 0;    /* a partial upload must not be used */
     return SetApiError(T41RX_ECUDA, what);
   }
@@ -919,24 +1088,50 @@ int t41rx_chan_set_shift(t41rx_chan *c, int first, int count, const int32_t *shi
   return ChanUpload(c, "t41rx_chan_set_shift: upload failed");
 }
 
+int t41rx_chan_set_weights(t41rx_chan *c, int first, int count, const float *w) {
+  if (!c || !w || first < 0 || count <= 0 || first + count > c->n_receivers)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_set_weights: bad range");
+  if (c->n_inputs < 2)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_set_weights: a single-input channelizer has no weights (create it with "
+                                     "t41rx_chan_create_diversity)");
+  const size_t n = (size_t)count * c->n_inputs;
+  for (size_t i = 0; i < 2 * n; ++i)
+    if (!std::isfinite(w[i])) return SetApiError(T41RX_EINVAL, "t41rx_chan_set_weights: weights must be finite");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_set_weights: cudaSetDevice failed");
+  int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  for (size_t i = 0; i < n; ++i) c->weight[(size_t)first * c->n_inputs + i] = float2{w[2 * i], w[2 * i + 1]};
+  return ChanUpload(c, "t41rx_chan_set_weights: upload failed");
+}
+
 }  // extern "C"
 
-/* one call of any kind (the caller has checked the pointers and the kind): capture holds n_blocks x 2048 x D samples
-   of ChanSampleBytes(c->kind) each */
-static int ChanProcess(const char *fn, t41rx_chan *c, const void *capture, float *iq, int n_blocks, void *cuda_stream) {
+/* one call of any kind (the caller has checked the pointers and the kind): captures[a], a < n_inputs, holds
+   n_blocks x 2048 x D samples of ChanSampleBytes(c->kind) each.  A diversity call runs one pass per input on the same
+   stream, input 0 storing and the others accumulating, always in this order, so cutting a run into calls gives the
+   same bits */
+static int ChanProcess(const char *fn, t41rx_chan *c, const void *const *captures, float *iq, int n_blocks,
+                       void *cuda_stream) {
   const std::string f(fn);
   if (n_blocks > INT_MAX / (T41RX_BLOCK_SAMPLES / kChanTile))
     return SetApiError(T41RX_EINVAL, (f + ": n_blocks too large for one call").c_str());
   if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, (f + ": cudaSetDevice failed").c_str());
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
-  cudaError_t e = c->n_entries > 0 ? c->kernels.launch(c, capture, (float2 *)iq, n_blocks, st) : cudaSuccess;
-  /* the new tail: the call's last N samples, copied after the kernel on the same stream so no tile reads it early */
   const size_t N = (size_t)kChanTaps * c->n_channels;
   const size_t total = (size_t)n_blocks * T41RX_BLOCK_SAMPLES * (c->n_channels / 2);
   const size_t sample_bytes = ChanSampleBytes(c->kind);
-  if (e == cudaSuccess)
-    e = cudaMemcpyAsync(c->d_tail, (const char *)capture + (total - N) * sample_bytes, sample_bytes * N,
-                        cudaMemcpyDeviceToDevice, st);
+  char *tails = (char *)c->d_tail;
+  cudaError_t e = cudaSuccess;
+  for (int a = 0; a < c->n_inputs && c->n_entries > 0 && e == cudaSuccess; ++a) {
+    const int store = c->n_inputs == 1 ? kChanPlain : a == 0 ? kChanWeighted : kChanAccumulate;
+    e = c->kernels.launch(c, captures[a], tails + a * N * sample_bytes, store,
+                          c->d_weight ? c->d_weight + (size_t)a * c->n_entries : nullptr, (float2 *)iq, n_blocks, st);
+  }
+  /* the new tails: each input's last N samples, copied after the last pass on the same stream so no tile reads them
+     early */
+  for (int a = 0; a < c->n_inputs && e == cudaSuccess; ++a)
+    e = cudaMemcpyAsync(tails + a * N * sample_bytes, (const char *)captures[a] + (total - N) * sample_bytes,
+                        sample_bytes * N, cudaMemcpyDeviceToDevice, st);
   if (e == cudaSuccess)
     c->m_done = (int)((c->m_done + (long long)n_blocks * T41RX_BLOCK_SAMPLES) % kChanOutRate);
   if (st != c->stream) {
@@ -952,24 +1147,41 @@ extern "C" {
 int t41rx_chan_process_device(t41rx_chan *c, const float *capture, float *iq, int n_blocks, void *cuda_stream) {
   if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 7) || ((uintptr_t)iq & 7))
     return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device: bad arguments (null or not 8-byte aligned pointer, n_blocks <= 0)");
-  if (c->kind != ChanKind::kFloat) return ChanWrongKind("t41rx_chan_process_device", c->kind);
-  return ChanProcess("t41rx_chan_process_device", c, capture, iq, n_blocks, cuda_stream);
+  if (c->kind != ChanKind::kFloat || c->n_inputs > 1) return ChanWrongKind("t41rx_chan_process_device", c);
+  const void *captures[] = {capture};
+  return ChanProcess("t41rx_chan_process_device", c, captures, iq, n_blocks, cuda_stream);
 }
 
 int t41rx_chan_process_device_real(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream) {
   if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 15) || ((uintptr_t)iq & 7))
     return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_real: bad arguments (null pointer, capture not 16-byte or "
                                      "iq not 8-byte aligned, n_blocks <= 0)");
-  if (c->kind != ChanKind::kReal) return ChanWrongKind("t41rx_chan_process_device_real", c->kind);
-  return ChanProcess("t41rx_chan_process_device_real", c, capture, iq, n_blocks, cuda_stream);
+  if (c->kind != ChanKind::kReal || c->n_inputs > 1) return ChanWrongKind("t41rx_chan_process_device_real", c);
+  const void *captures[] = {capture};
+  return ChanProcess("t41rx_chan_process_device_real", c, captures, iq, n_blocks, cuda_stream);
 }
 
 int t41rx_chan_process_device_q15(t41rx_chan *c, const int16_t *capture, float *iq, int n_blocks, void *cuda_stream) {
   if (!c || !capture || !iq || n_blocks <= 0 || ((uintptr_t)capture & 15) || ((uintptr_t)iq & 7))
     return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_q15: bad arguments (null pointer, capture not 16-byte or "
                                      "iq not 8-byte aligned, n_blocks <= 0)");
-  if (c->kind != ChanKind::kQ15) return ChanWrongKind("t41rx_chan_process_device_q15", c->kind);
-  return ChanProcess("t41rx_chan_process_device_q15", c, capture, iq, n_blocks, cuda_stream);
+  if (c->kind != ChanKind::kQ15 || c->n_inputs > 1) return ChanWrongKind("t41rx_chan_process_device_q15", c);
+  const void *captures[] = {capture};
+  return ChanProcess("t41rx_chan_process_device_q15", c, captures, iq, n_blocks, cuda_stream);
+}
+
+int t41rx_chan_process_device_diversity(t41rx_chan *c, const void *const *captures, float *iq, int n_blocks,
+                                        void *cuda_stream) {
+  if (!c || !captures || !iq || n_blocks <= 0 || ((uintptr_t)iq & 7))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_process_device_diversity: bad arguments (null pointer, iq not 8-byte "
+                                     "aligned, n_blocks <= 0)");
+  if (c->n_inputs < 2) return ChanWrongKind("t41rx_chan_process_device_diversity", c);
+  const uintptr_t align = c->kind == ChanKind::kFloat ? 7 : 15;
+  for (int a = 0; a < c->n_inputs; ++a)
+    if (!captures[a] || ((uintptr_t)captures[a] & align))
+      return SetApiError(T41RX_EINVAL, (std::string("t41rx_chan_process_device_diversity: capture ") + std::to_string(a) +
+                                        (align == 7 ? " null or not 8-byte aligned" : " null or not 16-byte aligned")).c_str());
+  return ChanProcess("t41rx_chan_process_device_diversity", c, captures, iq, n_blocks, cuda_stream);
 }
 
 int t41rx_chan_synchronize(t41rx_chan *c) {

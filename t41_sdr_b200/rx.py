@@ -92,10 +92,13 @@ EXPORTS = (
     "t41rx_chan_create", "t41rx_chan_destroy", "t41rx_chan_set_map", "t41rx_chan_process_device", "t41rx_chan_synchronize",
     "t41rx_chan_taps", "t41rx_chan_tune", "t41rx_chan_set_shift", "t41rx_chan_place",
     "t41rx_chan_create_real", "t41rx_chan_process_device_real", "t41rx_chan_tune_real", "t41rx_chan_place_real",
-    "t41rx_chan_create_q15", "t41rx_chan_process_device_q15")
+    "t41rx_chan_create_q15", "t41rx_chan_process_device_q15",
+    "t41rx_chan_create_diversity", "t41rx_chan_set_weights", "t41rx_chan_process_device_diversity")
 
 CHAN_TAPS_PER_BRANCH = 10     # prototype length = 10 * n_channels
 CHAN_SPACING = 96000.0        # channel spacing (Hz); every channel comes out at 192 kS/s
+CHAN_FLOAT, CHAN_Q15, CHAN_REAL = 0, 1, 2   # capture kinds of t41rx_chan_create_diversity
+CHAN_MAX_INPUTS = 4           # a diversity channelizer takes 2 ... 4 coherent captures
 
 
 def build_library():
@@ -176,6 +179,9 @@ def lib():
         L.t41rx_chan_process_device_real.argtypes = [vp, vp, vp, ip, vp]
         L.t41rx_chan_create_q15.argtypes = [C.POINTER(vp), ip, ip, ip]
         L.t41rx_chan_process_device_q15.argtypes = [vp, vp, vp, ip, vp]
+        L.t41rx_chan_create_diversity.argtypes = [C.POINTER(vp), ip, ip, ip, ip, ip]
+        L.t41rx_chan_set_weights.argtypes = [vp, ip, ip, C.POINTER(C.c_float)]
+        L.t41rx_chan_process_device_diversity.argtypes = [vp, C.POINTER(vp), vp, ip, vp]
         L.t41rx_chan_tune_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.t41rx_chan_place_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                             C.POINTER(C.c_int32)]
@@ -580,17 +586,29 @@ class Channelizer:
     n_receivers receivers out (t41rx_process_device's layout).  Device pointers, e.g. torch.Tensor.data_ptr().
     real=True: an int16 real capture (n_channels 128, 800, 1024 or 1280: 12.288, 76.8, 98.304 or 122.88 MS/s; channels
     0 ... n_channels / 2); q15=True: a complex capture of interleaved int16 (I, Q) pairs, x = (I + jQ) / 32768
-    (n_channels 64, 320, 512 or 640: 6.144, 30.72, 49.152 or 61.44 MS/s); else complex float (the same n_channels)."""
+    (n_channels 64, 320, 512 or 640: 6.144, 30.72, 49.152 or 61.44 MS/s); else complex float (the same n_channels).
+    n_inputs = 2 ... 4: a diversity channelizer (DESIGN §3.11) on that many coherent captures of the kind, receiver r
+    getting rot_r(m) sum_a w[r][a] z^(a)_k[m] with its own weights (set_weights; default: input 0 alone)."""
 
-    def __init__(self, n_channels, n_receivers, device=0, real=False, q15=False):
+    def __init__(self, n_channels, n_receivers, device=0, real=False, q15=False, n_inputs=1):
         if real and q15:
             raise ValueError("Channelizer: real and q15 are different capture kinds; pass at most one")
+        if not isinstance(n_inputs, (int, np.integer)) or not 1 <= n_inputs <= CHAN_MAX_INPUTS:
+            raise ValueError("Channelizer: n_inputs must be 1 (one capture) or 2 ... %d (diversity), not %r" % (
+                CHAN_MAX_INPUTS, n_inputs))
         self._h = C.c_void_p()
         self.n_channels = int(n_channels)
         self.n_receivers = int(n_receivers)
         self.device = int(device)
         self.real = bool(real)
         self.q15 = bool(q15)
+        self.n_inputs = int(n_inputs)
+        if self.n_inputs > 1:
+            self._create, self._process = "t41rx_chan_create_diversity", "t41rx_chan_process_device_diversity"
+            kind = CHAN_REAL if self.real else CHAN_Q15 if self.q15 else CHAN_FLOAT
+            _check(lib().t41rx_chan_create_diversity(C.byref(self._h), kind, self.n_channels, self.n_inputs,
+                                                     self.n_receivers, self.device), self._create)
+            return
         self._create, self._process = (("t41rx_chan_create_real", "t41rx_chan_process_device_real") if self.real else
                                        ("t41rx_chan_create_q15", "t41rx_chan_process_device_q15") if self.q15 else
                                        ("t41rx_chan_create", "t41rx_chan_process_device"))
@@ -627,10 +645,29 @@ class Channelizer:
         _check(lib().t41rx_chan_set_shift(self._h, int(first), int(arr.size), arr.ctypes.data_as(C.POINTER(C.c_int32))),
                "t41rx_chan_set_shift")
 
+    def set_weights(self, w, first=0):
+        """diversity: receivers first, first + 1, ... take the complex weights w[i] (array [count, n_inputs]), applied to
+        each input's channel as delivered (after the channelizer's conjugate): an input-1 copy c x of an interferer x on
+        input 0 is nulled by w[i][1] = -w[i][0] / conj(c).  Effective from the next call, in a step (no ramp)"""
+        w = np.asarray(w, dtype=np.complex128)
+        if w.ndim != 2 or w.shape[1] != self.n_inputs:
+            raise ValueError("Channelizer.set_weights: w must be [count, %d], not %s" % (self.n_inputs, w.shape))
+        arr = np.ascontiguousarray(np.stack([w.real, w.imag], axis=-1), dtype=np.float32)
+        _check(lib().t41rx_chan_set_weights(self._h, int(first), int(w.shape[0]), arr.ctypes.data_as(C.POINTER(C.c_float))),
+               "t41rx_chan_set_weights")
+
     def process_device(self, capture_ptr, iq_ptr, n_blocks, stream=None):
         """capture float32 [n_blocks * 2048 * n_channels / 2, 2] (real: int16 [n_blocks * 2048 * n_channels / 2];
         q15: int16 [n_blocks * 2048 * n_channels / 2, 2]; both 16-byte aligned) -> iq float32 [n_receivers, n_blocks,
-        2048, 2]"""
+        2048, 2].  Diversity: capture_ptr is a list of n_inputs such pointers, input 0 first"""
+        if self.n_inputs > 1:
+            ptrs = list(capture_ptr) if isinstance(capture_ptr, (list, tuple)) else None
+            if ptrs is None or len(ptrs) != self.n_inputs:
+                raise ValueError("Channelizer.process_device: a diversity channelizer takes a list of %d capture "
+                                 "pointers" % self.n_inputs)
+            _check(lib().t41rx_chan_process_device_diversity(self._h, (C.c_void_p * self.n_inputs)(*ptrs), iq_ptr,
+                                                             int(n_blocks), stream), self._process)
+            return
         _check(getattr(lib(), self._process)(self._h, capture_ptr, iq_ptr, int(n_blocks), stream), self._process)
 
     def synchronize(self):

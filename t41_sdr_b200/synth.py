@@ -237,12 +237,13 @@ def wideband_q15(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
     return out
 
 
-def _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block):
-    """complex128 signal sum and noise of wideband() / wideband_real() / wideband_q15()"""
+def _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block, delay=0):
+    """complex128 signal sum and noise of wideband() / wideband_real() / wideband_q15(); delay: the signals (not the
+    noise) delayed by that many capture samples"""
     fs = wideband_rate(n_channels)
     per_block = BLOCK * n_channels // 2
     n = n_blocks * per_block
-    n0 = start_block * per_block
+    n0 = start_block * per_block - int(delay)
     t = (n0 + np.arange(n)) / fs
     z = np.zeros(n, np.complex128)
     for kind, f, kw in signals:
@@ -264,3 +265,55 @@ def _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block):
     if sigma > 0.0:
         z += _noise(np.random.Generator(np.random.PCG64([SEED_BASE + int(seed), int(start_block)])), n, sigma)
     return z
+
+
+# ---- coherent captures for the diversity channelizer (t41rx_chan_create_diversity) ----
+
+def diversity_sums(seed, n_channels, n_blocks, wanted, interferers, gains, delays=None, sigma=0.0, start_block=0):
+    """complex128 [n] per input of n_inputs = len(gains) coherent captures, sampled on one clock, as two to four ADCs
+    of one digitizer deliver them: input a holds gains[a] times the `interferers` (a signal list as wideband() takes)
+    delayed by delays[a] capture samples (default 0), input 0 also the `wanted` signals, and every input its own
+    independent noise (sigma per component, seeded by seed, start_block and a).  With sigma = 0 and no wanted
+    signal, input a is exactly gains[a] / gains[0] times input 0 when the delays are equal."""
+    per_block = BLOCK * n_channels // 2
+    n = n_blocks * per_block
+    out = []
+    for a, g in enumerate(gains):
+        d = 0 if delays is None else int(delays[a])
+        z = g * _wideband_sum(seed, n_channels, n_blocks, interferers, 0.0, start_block, delay=d)
+        if a == 0 and wanted:
+            z = z + _wideband_sum(seed, n_channels, n_blocks, wanted, 0.0, start_block)
+        if sigma > 0.0:
+            z = z + _noise(np.random.Generator(np.random.PCG64([SEED_BASE + int(seed), int(start_block), 1 + a])), n, sigma)
+        out.append(z)
+    return out
+
+
+def wideband_diversity(seed, n_channels, n_blocks, wanted, interferers, gains, sigma=0.0, start_block=0):
+    """diversity_sums() as complex float captures (float32 [n, 2] each, not quantised, as wideband()); gains complex"""
+    out = []
+    for z in diversity_sums(seed, n_channels, n_blocks, wanted, interferers, gains, None, sigma, start_block):
+        c = np.empty((z.size, 2), np.float32)
+        c[:, 0] = z.real
+        c[:, 1] = z.imag
+        out.append(c)
+    return out
+
+
+def wideband_diversity_q15(seed, n_channels, n_blocks, wanted, interferers, gains, sigma=0.0, start_block=0):
+    """diversity_sums() as interleaved int16 (I, Q) captures, quantised as wideband_q15(); gains complex"""
+    out = []
+    for z in diversity_sums(seed, n_channels, n_blocks, wanted, interferers, gains, None, sigma, start_block):
+        c = np.empty((z.size, 2), np.int16)
+        c[:, 0] = np.clip(np.round(32768.0 * z.real), -32768, 32767)
+        c[:, 1] = np.clip(np.round(32768.0 * z.imag), -32768, 32767)
+        out.append(c)
+    return out
+
+
+def wideband_diversity_real(seed, n_channels, n_blocks, wanted, interferers, gains, delays, sigma=0.0, start_block=0):
+    """diversity_sums() as real int16 captures of direct-sampling ADCs, quantised as wideband_real(): input a holds
+    the interferers times the real gains[a], delayed by the integer delays[a] capture samples (a second antenna's
+    cable and distance)"""
+    return [np.clip(np.round(32768.0 * z.real), -32768, 32767).astype(np.int16)
+            for z in diversity_sums(seed, n_channels, n_blocks, wanted, interferers, gains, delays, sigma, start_block)]

@@ -1,6 +1,6 @@
 """Channelizer timing on one GPU (DESIGN §3.7 - 3.9): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
 
-    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--rates] [--json OUT]
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--rates] [--diversity N] [--json OUT]
 
 Prints the card's name and power limit (a query), then CUDA-event times of
   - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
@@ -19,6 +19,10 @@ Prints the card's name and power limit (a query), then CUDA-event times of
     The same 1024 receivers, 2 per channel on channels 0 ... 511 (at M = 320 and 800, which have fewer channels, on
     channel (r / 2) mod 320 and mod 401), 64 blocks per call; the calls alternate between two captures, so that the
     captures a size reads (2 x 105 MB at real M = 800, more elsewhere) do not fit the L2,
+  - with --diversity N (DESIGN §3.11), an N-input diversity call against the single-input call of the same kind and
+    shape: complex float and int16 pairs at M = 512, real at M = 1024 and 1280; the same 1024 receivers, 2 per channel,
+    64 blocks per call, every receiver shifted and given seeded weights on every input (none of them the default).  The
+    single-input call alternates between two of the N captures; the N-input call reads all N (each at least 134 MB),
 each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
 receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
 """
@@ -104,6 +108,65 @@ def rate_table(g, dev, iq, sp, timed, shifts, S, T):
     return out
 
 
+def diversity_table(g, dev, iq, sp, timed, shifts, S, T, n_inputs):
+    """the --diversity measurements: per (kind, M) the single-input call (before and after) and the n_inputs diversity
+    call, in the same run, and their ratio against the goal (at most 2.5 x)"""
+    import torch
+    r = np.random.Generator(np.random.PCG64(2026))
+    w = (0.2 + r.uniform(0, 1, (S, n_inputs))) * np.exp(2j * np.pi * r.uniform(0, 1, (S, n_inputs)))
+    chmap = [(i // 2) % 512 for i in range(S)]
+    out = {}
+    for kind, M in (("complex", 512), ("q15", 512), ("real", 1024), ("real", 1280)):
+        real, q15 = kind == "real", kind == "q15"
+        n_cap = T * rx.BLOCK * M // 2
+        if real:
+            caps = [torch.randint(-3277, 3278, (n_cap,), generator=g, device=dev, dtype=torch.int16) for _ in range(n_inputs)]
+        elif q15:
+            caps = [torch.randint(-3277, 3278, (n_cap, 2), generator=g, device=dev, dtype=torch.int16) for _ in range(n_inputs)]
+        else:
+            caps = [(0.1 * torch.randn((n_cap, 2), generator=g, device=dev)).contiguous() for _ in range(n_inputs)]
+        single = rx.Channelizer(M, S, real=real, q15=q15)
+        div = rx.Channelizer(M, S, real=real, q15=q15, n_inputs=n_inputs)
+        for c in (single, div):
+            c.set_map(chmap)
+            c.set_shift(shifts)
+        div.set_weights(w)
+        ptrs = [c.data_ptr() for c in caps]
+        calls = [0]
+
+        def do_single():
+            single.process_device(ptrs[calls[0] % 2], iq.data_ptr(), T, stream=sp)
+            calls[0] += 1
+
+        def do_div():
+            div.process_device(ptrs, iq.data_ptr(), T, stream=sp)
+
+        t_single = timed(do_single)
+        t_div = timed(do_div)
+        t_single2 = timed(do_single)
+        for c in (single, div):
+            c.synchronize()
+            c.close()
+        cap_bytes = caps[0].numel() * caps[0].element_size()
+        iq_bytes = S * T * rx.BLOCK * 8
+        moved_single = cap_bytes + iq_bytes
+        # every pass reads its capture; pass 0 writes iq, each later pass reads and writes it
+        moved_div = n_inputs * cap_bytes + iq_bytes + (n_inputs - 1) * 2 * iq_bytes
+        ratio = t_div[0] / min(t_single[0], t_single2[0])
+        out["%s_%d" % (kind, M)] = {
+            "capture_bytes_per_input": cap_bytes,
+            "single_ms": {"median": t_single[0], "min": t_single[1], "max": t_single[2]},
+            "single_again_ms": {"median": t_single2[0], "min": t_single2[1], "max": t_single2[2]},
+            "diversity_ms": {"median": t_div[0], "min": t_div[1], "max": t_div[2]},
+            "diversity_over_single": ratio,
+            "goal_le_2p5_x_single": ratio <= 2.5,
+            "single_bytes_moved": moved_single, "diversity_bytes_moved": moved_div,
+            "single_hbm_share_of_7p7_tbs": moved_single / (t_single[0] * 1e-3) / HBM_BYTES_PER_S,
+            "diversity_hbm_share_of_7p7_tbs": moved_div / (t_div[0] * 1e-3) / HBM_BYTES_PER_S}
+        del caps
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--channels", type=int, default=512)
@@ -115,6 +178,8 @@ def main():
     ap.add_argument("--real", action="store_true", help="also time the real M = 1024 channelizer")
     ap.add_argument("--q15", action="store_true", help="also time the q15 channelizer and torch conversion + float")
     ap.add_argument("--rates", action="store_true", help="also time every channel count beside its power-of-two neighbour")
+    ap.add_argument("--diversity", type=int, default=0, metavar="N",
+                    help="also time an N-input diversity call against the single-input call (N = 2 ... 4)")
     ap.add_argument("--json", default=None, help="also write the result here")
     a = ap.parse_args()
     import torch
@@ -213,6 +278,7 @@ def main():
             c.synchronize()
             c.close()
     rates = rate_table(g, dev, iq, sp, timed, shifts, S, T) if a.rates else None
+    diversity = diversity_table(g, dev, iq, sp, timed, shifts, S, T, a.diversity) if a.diversity else None
     eng.synchronize()
     bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
     res = {
@@ -263,6 +329,8 @@ def main():
             res["q15"]["shift_overhead"] = t_q15_shift[0] / t_q15[0] - 1.0
     if rates:
         res["rates"] = rates
+    if diversity:
+        res["diversity"] = {"n_inputs": a.diversity, "every_receiver_shifted_and_weighted": True, **diversity}
     print(json.dumps(res, indent=1))
     if a.json:
         with open(a.json, "w") as f:
