@@ -367,6 +367,46 @@ int t41rx_chan_create_diversity(t41rx_chan **out, int kind, int n_channels, int 
 int t41rx_chan_set_weights(t41rx_chan *c, int first, int count, const float *w);
 int t41rx_chan_process_device_diversity(t41rx_chan *c, const void *const *captures, float *iq, int n_blocks,
                                         void *cuda_stream);
+/* Image correction (DESIGN §3.12): complex single-input channelizers (t41rx_chan_create, t41rx_chan_create_q15).  An
+ * I/Q digitizer's gain, phase and delay mismatch between its I and Q branches puts an image of a signal at +f at -f,
+ * so a carrier on channel k leaks into channel kbar = (M - k) mod M.  Each channel has a complex coefficient c_k (0 at
+ * creation), and receiver r mapped to channel k gets
+ *     y_k[m]  = z_k[m] + c_k conj(z_kbar[m])
+ *     iq_r[m] = rot_r(m) y_k[m]
+ * z_k being the channel as delivered without correction (after the conjugate); the fine-tuning rotation and its phase
+ * rule are applied to y.  Channels 0 and M / 2 are their own mirrors.
+ * Model: a frequency-independent imbalance x = mu s + nu conj(s) is removed on every channel by c_k = -conj(nu) / mu.
+ * With gain g and phase phi on Q (Q' = g (Q cos phi + I sin phi)): mu = (1 + g e^(j phi)) / 2, nu = (1 - g e^(-j phi))
+ * / 2.  An imbalance that varies with frequency (I/Q delay skew) needs a different c_k per channel, and different values
+ * on k and kbar.
+ * Bits: with every c_k exactly 0 and tracking off a call runs the uncorrected channelizer and gives its bits; a channel
+ * whose c_k is 0 gets z_k unmodified (with its rotation rounded as without correction); with fixed coefficients,
+ * cutting a run into calls gives the same bits; the q15 channelizer gives the float one's bits on s / 32768.
+ * Tracking (opt-in, t41rx_chan_track_image): each call measures every mirror pair k = 0 ... M / 2 on its delivered y,
+ * A = sum_m y_k y_kbar (no conjugate), P_k = sum |y_k|^2, P_kbar = sum |y_kbar|^2 over the call's outputs (whether or
+ * not a receiver is mapped there), and for k = 1 ... M / 2 - 1 updates the coefficients the next call uses, on the
+ * device, without a host synchronisation: if P_k >= T P_kbar, c_kbar -= A / P_k; else if P_kbar >= T P_k, c_k -= A /
+ * P_kbar; else the pair is left alone (only the weak side of a pair where the other dominates is corrected).  Channels
+ * 0 and M / 2 are never updated.  With tracking, the coefficients, and so the bits, depend on where the call
+ * boundaries fall; calls cut the same way give identical bits.  The first tracking call, and any with more blocks
+ * than every earlier one, waits for the channelizer's earlier calls while it makes room for its per-tile sums.
+ * Every image entry point returns EINVAL on a real or a diversity channelizer (the message says why), and on a null c.
+ * t41rx_chan_set_image: channels [first, first + count) take c_k = (coef[2 i], coef[2 i + 1]), finite (EINVAL
+ * otherwise, and for a range outside [0, n_channels)).  Effective from the next call; waits for the channelizer's calls
+ * like t41rx_chan_set_shift.  Channels outside the range keep their coefficients, including ones tracking has moved.
+ * t41rx_chan_get_image: all n_channels coefficients as (re, im) pairs into coef[2 n_channels], including what tracking
+ * has made of them (save and restore a calibration per band with it); waits for the channelizer's calls.
+ * t41rx_chan_track_image: on != 0 turns tracking on with T = dominance_db (in [T41RX_CHAN_DOMINANCE_MIN_DB,
+ * T41RX_CHAN_DOMINANCE_MAX_DB], EINVAL outside it; 20 is a good default), from the next call; on = 0 turns it off
+ * (dominance_db is then not read), the coefficients staying where tracking left them.
+ * t41rx_chan_image_stats: stats[(M / 2 + 1) x 4], (Re A, Im A, P_k, P_kbar) of pair k = 0 ... M / 2 from the last
+ * call that ran with tracking on (EINVAL if none has); waits for the channelizer's calls. */
+#define T41RX_CHAN_DOMINANCE_MIN_DB 3.0f
+#define T41RX_CHAN_DOMINANCE_MAX_DB 60.0f
+int t41rx_chan_set_image(t41rx_chan *c, int first, int count, const float *coef);
+int t41rx_chan_get_image(t41rx_chan *c, float *coef);
+int t41rx_chan_track_image(t41rx_chan *c, int on, float dominance_db);
+int t41rx_chan_image_stats(t41rx_chan *c, double *stats);
 
 /* Audio-spectrum + S-meter by-product of the row-producing blocks (Process.cpp:550-570; NFM: 791-805):
  *   audio_ypixel      int32 [n_streams][n_rows][270]  audioYPixel[k], k < AUDIO_SPEC_BOX_W - 2 (Process.cpp:34,555)

@@ -47,6 +47,12 @@
  * rot_r(m) sum_a w[r][a] z^(a)_k[m].  A call runs the kind's kernel once per input on one stream, input 0's pass
  * storing v w f and the others adding it to iq (the kStore template parameter, behind if constexpr); each input keeps
  * its own tail.
+ *
+ * Image correction (t41rx_chan_set_image / _track_image, DESIGN §3.12), complex single-input channelizers: receiver r
+ * on channel k gets rot_r(m) (z_k[m] + c_k conj(z_kbar[m])), kbar = (M - k) mod M.  The kChanImage / kChanImageTrack
+ * instances correct the FFT rows in place, a mirror pair at a time, before the plain store loop; tracking also sums
+ * each pair's products per tile, and t41rx_chan_image_update reduces them in a fixed order and moves the coefficients
+ * the next call uses.  With every c_k 0 and tracking off a call runs the plain instances.
  */
 #include <cuda_runtime.h>
 
@@ -186,8 +192,9 @@ __device__ __forceinline__ float2 ChanRotor(const float2 *tab, int2 sp, unsigned
 
 /* the store stage of a kernel instance (DESIGN §3.11): kChanPlain writes the (rotated) sample, as a single-input
    channelizer does; a diversity call runs the kernel once per input, kChanWeighted for input 0 (writes v w f) and
-   kChanAccumulate for the others (adds v w f to iq) */
-constexpr int kChanPlain = 0, kChanWeighted = 1, kChanAccumulate = 2;
+   kChanAccumulate for the others (adds v w f to iq).  Image correction (DESIGN §3.12, complex kinds only): kChanImage
+   writes the (rotated) y_k = z_k + c_k conj(z_kbar), kChanImageTrack also writes each mirror pair's tile partials */
+constexpr int kChanPlain = 0, kChanWeighted = 1, kChanAccumulate = 2, kChanImage = 3, kChanImageTrack = 4;
 
 /* complex products with every rounding spelled out (__fmul_rn / __fmaf_rn are never contracted), so that the weighted
    instances round as the plain ones' SASS does whatever the compiler makes of their context:
@@ -246,6 +253,75 @@ __device__ __forceinline__ void ChanWeightedLoop(float2 *__restrict__ iq, const 
       else
         *dst[u] = float2{__fadd_rn(old[u].x, p.x), __fadd_rn(old[u].y, p.y)};
     }
+  }
+}
+
+/* z + c conj(zm), every rounding spelled out */
+__device__ __forceinline__ float2 ChanImageRn(float2 z, float2 zm, float2 c) {
+  return float2{__fmaf_rn(c.x, zm.x, __fmaf_rn(c.y, zm.y, z.x)), __fmaf_rn(c.y, zm.x, __fmaf_rn(-c.x, zm.y, z.y))};
+}
+
+/* the store stage of the kChanImage / kChanImageTrack instances.  image: the channelizer's image table, the M
+   coefficients c_k and after them the tracking partials, float4 (Re A, Im A, P_k, P_kbar) [M/2 + 1][gridDim.x] (pair
+   k, tile).
+   First the FFT rows are corrected in place, a mirror pair (k, kbar = (M - k) mod M) at a time: y_k = z_k + c_k
+   conj(z_kbar) and y_kbar = z_kbar + c_kbar conj(z_k) from the same z, each, when its c is 0, the z itself, selected.
+   The rows hold every z_k with its (-1)^(k m) applied, and (-1)^((M - k) m) = (-1)^(k m) as M is even, so the mirror
+   sample is used as it stands.  Half-warp h takes pairs h, h + kThreads / 16, ..., lane mm row mm (conflict-free: row
+   r starts in bank column r); the tracking instance also sums the pair's three products over the 16 rows by a fixed
+   shuffle tree.  Then the store loop is the plain one on the corrected rows, the rotation rounded as the plain
+   instance's SASS rounds it (the Rn forms), so a channel whose c_k is 0 gets the plain instance's bits. */
+template <int M, bool kRotate, bool kTrack, typename S>
+__device__ __forceinline__ void ChanImageStore(float2 *smem, const int32_t *__restrict__ recv,
+                                               const int32_t *__restrict__ chan, const int2 *__restrict__ phase,
+                                               int m_base, long long m0, int n_entries, float2 *__restrict__ iq,
+                                               int n_blocks, const float2 *__restrict__ image) {
+  /* tid read again here: kept live from the span stage it spills a register in the q15 M = 512 tracking instance */
+  int tid;
+  asm volatile("mov.u32 %0, %%tid.x;" : "=r"(tid));
+  constexpr int kPairs = M / 2 + 1, kHalfWarps = S::kThreads / kChanTile;
+  const int mm = tid % kChanTile;
+  float2 *row = smem + S::RowBase(mm);
+  float4 *part = reinterpret_cast<float4 *>(const_cast<float2 *>(image + M)) + blockIdx.x;
+  /* unrolled 3 times without tracking, not with it (measured: about 0.5 % faster without, 1 - 2 % slower with) */
+#pragma unroll (kTrack ? 1 : 3)
+  for (int k0 = 0; k0 < kPairs; k0 += kHalfWarps) {    /* uniform over the warp: the shuffles need all 32 lanes */
+    const int k = k0 + tid / kChanTile;
+    if (!kTrack && k >= kPairs) break;
+    const int kk = k < kPairs ? k : 0, kb = ChanWrap<M>(M - kk);
+    const int pk = ChanOutPos<M>(kk), pb = ChanOutPos<M>(kb);
+    const float2 zk = row[pk], zb = row[pb], ck = __ldg(image + kk), cb = __ldg(image + kb);
+    const float2 yk = ck.x == 0.f && ck.y == 0.f ? zk : ChanImageRn(zk, zb, ck);
+    const float2 yb = cb.x == 0.f && cb.y == 0.f ? zb : ChanImageRn(zb, zk, cb);
+    if (k < kPairs) {
+      row[pk] = yk;
+      row[pb] = yb;    /* the same value as yk for the pairs 0 and M/2, their own mirrors */
+    }
+    if constexpr (kTrack) {
+      float s[4] = {yk.x * yb.x - yk.y * yb.y, yk.x * yb.y + yk.y * yb.x, yk.x * yk.x + yk.y * yk.y,
+                    yb.x * yb.x + yb.y * yb.y};
+#pragma unroll
+      for (int d = kChanTile / 2; d > 0; d >>= 1)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) s[i] += __shfl_xor_sync(0xffffffffu, s[i], d);
+      if (mm == 0 && k < kPairs) part[(long long)k * gridDim.x] = float4{s[0], s[1], s[2], s[3]};
+    }
+  }
+  __syncthreads();
+  const long long blk = m0 / T41RX_BLOCK_SAMPLES;
+  const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
+  const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
+#pragma unroll 4
+  for (int w = tid; w < n_entries * kChanTile; w += S::kThreads) {
+    const int e = w / kChanTile;
+    const int k = __ldg(chan + e), r = __ldg(recv + e);
+    const float2 y = row[ChanOutPos<M>(k)];
+    float2 out = y;
+    if constexpr (kRotate) {
+      const int2 sp = __ldg(phase + e);
+      out = (sp.x | sp.y) ? ChanMulRn(y, ChanRotorRn(smem + S::kRotBase, sp, m_abs)) : y;
+    }
+    iq[((long long)r * n_blocks + blk) * T41RX_BLOCK_SAMPLES + s0 + mm] = out;
   }
 }
 
@@ -353,8 +429,9 @@ template <> __device__ __forceinline__ float2 *ChanSmem<short>() {
    channel (CSR order) and the channel of each; phase: each entry's (shift, P) in [0, 192000), or null when no entry is
    rotated; rot: the 480 + 400 factors of the rotation table; m_base: outputs before this call, mod 192000;
    iq: [n_receivers][n_blocks][2048].  kRotate = false (no entry rotated) is the kernel without fine tuning.
-   kStore: the store stage (ChanWeightedLoop); weight: each entry's weight for this pass's input, in the order of
-   recv (read by the weighted instances only).
+   kStore: the store stage (ChanWeightedLoop, ChanImageStore); weight: each entry's weight for this pass's input, in
+   the order of recv (read by the weighted instances only), or for the image instances the channelizer's image table
+   (ChanImageStore).
    The int16 span goes through registers (16-byte loads of four pairs) and lands converted, (I, Q) as integer-valued
    floats, where the float span is staged: each sample is converted once, not at each of the ~9 branch loads that read
    it, and the rest of the kernel is the same for both.  h / 32768 times I is h times I / 32768 exactly, so every FMA,
@@ -447,9 +524,14 @@ t41rx_chan_kernel(const T *__restrict__ capture, const T *__restrict__ tail, con
   /* each receiver's run: kChanTile consecutive samples inside one block (the tile size divides 2048).  The store loops
      are written out here and again in t41rx_chan_real_kernel: as one __device__ function taking the sample as a lambda
      they compile to different (longer) code in every instance of this kernel. */
+  if constexpr (kStore == kChanImage || kStore == kChanImageTrack) {
+    ChanImageStore<M, kRotate, kStore == kChanImageTrack, S>(smem, recv, chan, phase, m_base, m0, n_entries, iq, n_blocks,
+                                                             weight);
+    return;
+  }
   const long long blk = m0 / T41RX_BLOCK_SAMPLES;
   const int s0 = (int)(m0 % T41RX_BLOCK_SAMPLES);
-  if constexpr (kStore != kChanPlain) {
+  if constexpr (kStore == kChanWeighted || kStore == kChanAccumulate) {
     const int mm = tid % kChanTile;
     const unsigned m_abs = (unsigned)((m_base + m0) % kChanOutRate) + mm;
     ChanWeightedLoop<kStore, S::kThreads>(iq + (blk * T41RX_BLOCK_SAMPLES + s0 + mm), recv, weight, n_entries, n_blocks,
@@ -629,6 +711,47 @@ t41rx_chan_real_kernel(const short *__restrict__ capture, const short *__restric
   }
 }
 
+/* image tracking, after a kChanImageTrack pass on the same stream: CTA k sums pair k's `tiles` partials in double, in
+   a fixed order (thread t takes tiles t, t + 256, ..., then a shared-memory tree), so the sums do not depend on how
+   the tiles were scheduled.  It writes stats[k] = (Re A, Im A, P_k, P_kbar) and, for k = 1 .. M/2 - 1, applies the
+   dominant-side rule: c_kbar -= A / P_k if P_k >= T P_kbar, else c_k -= A / P_kbar if P_kbar >= T P_k (T = dominance
+   >= 1, both P > 0), in double, rounded to float.  Channels 0 and M/2 are never updated. */
+constexpr int kChanImageThreads = 256;
+__global__ void __launch_bounds__(kChanImageThreads)
+t41rx_chan_image_update(float2 *__restrict__ image, int M, int tiles, double dominance, double *__restrict__ stats) {
+  __shared__ double red[4][kChanImageThreads];
+  const int k = blockIdx.x, tid = threadIdx.x;
+  const float4 *part = reinterpret_cast<const float4 *>(image + M) + (long long)k * tiles;
+  double s[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int t = tid; t < tiles; t += kChanImageThreads) {
+    const float4 v = part[t];
+    s[0] = __dadd_rn(s[0], (double)v.x);
+    s[1] = __dadd_rn(s[1], (double)v.y);
+    s[2] = __dadd_rn(s[2], (double)v.z);
+    s[3] = __dadd_rn(s[3], (double)v.w);
+  }
+  for (int i = 0; i < 4; ++i) red[i][tid] = s[i];
+  for (int h = kChanImageThreads / 2; h > 0; h >>= 1) {
+    __syncthreads();
+    if (tid < h)
+      for (int i = 0; i < 4; ++i) red[i][tid] = __dadd_rn(red[i][tid], red[i][tid + h]);
+  }
+  if (tid != 0) return;
+  const double ar = red[0][0], ai = red[1][0], pk = red[2][0], pb = red[3][0];
+  stats[4 * k] = ar;
+  stats[4 * k + 1] = ai;
+  stats[4 * k + 2] = pk;
+  stats[4 * k + 3] = pb;
+  if (k < 1 || k >= M / 2) return;
+  int j = -1;
+  double p = 0.0;
+  if (pk > 0.0 && pk >= __dmul_rn(dominance, pb)) j = M - k, p = pk;
+  else if (pb > 0.0 && pb >= __dmul_rn(dominance, pk)) j = k, p = pb;
+  if (j < 0) return;
+  const float2 c = image[j];
+  image[j] = float2{(float)__dsub_rn((double)c.x, __ddiv_rn(ar, p)), (float)__dsub_rn((double)c.y, __ddiv_rn(ai, p))};
+}
+
 /* modified Bessel function I0 (power series; terms fall below 1e-17 of the sum well before k = 60 for beta <= 9) */
 static double BesselI0(double x) {
   double sum = 1.0, term = 1.0;
@@ -771,6 +894,14 @@ struct t41rx_chan {
   std::vector<float2> weight;    /* diversity: [n_receivers][n_inputs], (1, 0) for input 0 and 0 for the others at creation */
   int m_done = 0;                /* outputs produced since creation, mod 192000 */
   ChanKernels kernels{};
+  /* image correction (complex single-input channelizers, DESIGN §3.12) */
+  ChanKernels image_kernels{};
+  float2 *d_image = nullptr;     /* the image table: n_channels c_k, then the tracking partials of image_tiles tiles */
+  double *d_image_stats = nullptr;   /* [n_channels / 2 + 1][4] of the last call with tracking on */
+  long long image_tiles = 0;
+  bool any_image = false;        /* some c_k is not 0 (as of the last set_image or tracking switch-off) */
+  bool track = false, has_stats = false;
+  double dominance = 100.0;      /* tracking's T, linear (20 dB) */
 };
 
 /* fn was called on a channelizer of another kind, or with a diversity channelizer's call on a single-input one or the
@@ -784,24 +915,36 @@ static int ChanWrongKind(const char *fn, const t41rx_chan *c) {
 }
 
 /* K::Pass<kStore> launches the kernel of one store mode, the one without or with fine tuning by c->any_rotated.  A
-   single-input channelizer's kernels are the plain ones, a diversity channelizer's the two weighted modes.  They are
-   kept apart (kDiversity) so that the plain instances are instantiated first and in the order they always were: the
-   compiler's code for the M = 320 and 512 instances depends on where the other instances fall in the module */
-template <typename K, bool kDiversity>
+   channelizer's kernels come in sets: a single-input channelizer's are the plain ones (kChanSetPlain), a diversity
+   channelizer's the two weighted modes (kChanSetDiversity), and a complex single-input channelizer also has the two
+   image modes (kChanSetImage).  The sets are kept apart so that the plain instances are instantiated first and in the
+   order they always were, then the weighted ones, then the image ones: the compiler's code for the M = 320 and 512
+   instances depends on where the other instances fall in the module */
+constexpr int kChanSetPlain = 0, kChanSetDiversity = 1, kChanSetImage = 2;
+template <typename K, int kSet>
 static cudaError_t ChanPrepare() {
-  if constexpr (!kDiversity) {
+  if constexpr (kSet == kChanSetPlain) {
     return K::template PrepareStore<kChanPlain>();
-  } else {
+  } else if constexpr (kSet == kChanSetDiversity) {
     const cudaError_t e = K::template PrepareStore<kChanWeighted>();
     return e == cudaSuccess ? K::template PrepareStore<kChanAccumulate>() : e;
+  } else {
+    const cudaError_t e = K::template PrepareStore<kChanImage>();
+    return e == cudaSuccess ? K::template PrepareStore<kChanImageTrack>() : e;
   }
 }
-template <typename K, bool kDiversity>
+template <typename K, int kSet>
 static cudaError_t ChanLaunch(const t41rx_chan *c, const void *capture, const void *tail, int store,
                               const float2 *weight, float2 *iq, int n_blocks, cudaStream_t st) {
-  if constexpr (!kDiversity) K::template Pass<kChanPlain>(c, capture, tail, weight, iq, n_blocks, st);
-  else if (store == kChanWeighted) K::template Pass<kChanWeighted>(c, capture, tail, weight, iq, n_blocks, st);
-  else K::template Pass<kChanAccumulate>(c, capture, tail, weight, iq, n_blocks, st);
+  if constexpr (kSet == kChanSetPlain) {
+    K::template Pass<kChanPlain>(c, capture, tail, weight, iq, n_blocks, st);
+  } else if constexpr (kSet == kChanSetDiversity) {
+    if (store == kChanWeighted) K::template Pass<kChanWeighted>(c, capture, tail, weight, iq, n_blocks, st);
+    else K::template Pass<kChanAccumulate>(c, capture, tail, weight, iq, n_blocks, st);
+  } else {
+    if (store == kChanImage) K::template Pass<kChanImage>(c, capture, tail, weight, iq, n_blocks, st);
+    else K::template Pass<kChanImageTrack>(c, capture, tail, weight, iq, n_blocks, st);
+  }
   return cudaGetLastError();
 }
 
@@ -854,34 +997,42 @@ struct ChanReal {
   }
 };
 
-template <typename K, bool kDiversity>
-constexpr ChanKernels kChanKernels{ChanPrepare<K, kDiversity>, ChanLaunch<K, kDiversity>};
+template <typename K, int kSet>
+constexpr ChanKernels kChanKernels{ChanPrepare<K, kSet>, ChanLaunch<K, kSet>};
 
 /* the kernels of a kind at a channel count its Chan*CountOk accepts */
-template <int M, bool kDiversity>
+template <int M, int kSet>
 static ChanKernels ChanComplexKernels(ChanKind kind) {
-  return kind == ChanKind::kQ15 ? kChanKernels<ChanComplex<M, short>, kDiversity>
-                                : kChanKernels<ChanComplex<M, float2>, kDiversity>;
+  return kind == ChanKind::kQ15 ? kChanKernels<ChanComplex<M, short>, kSet> : kChanKernels<ChanComplex<M, float2>, kSet>;
 }
-template <bool kDiversity>
+template <int kSet>
 static ChanKernels ChanKernelsOf(ChanKind kind, int n_channels) {
   if (kind == ChanKind::kReal)
     switch (n_channels) {
-      case 128: return kChanKernels<ChanReal<128>, kDiversity>;
-      case 800: return kChanKernels<ChanReal<800>, kDiversity>;
-      case 1024: return kChanKernels<ChanReal<1024>, kDiversity>;
-      default: return kChanKernels<ChanReal<1280>, kDiversity>;
+      case 128: return kChanKernels<ChanReal<128>, kSet>;
+      case 800: return kChanKernels<ChanReal<800>, kSet>;
+      case 1024: return kChanKernels<ChanReal<1024>, kSet>;
+      default: return kChanKernels<ChanReal<1280>, kSet>;
     }
   switch (n_channels) {
-    case 64: return ChanComplexKernels<64, kDiversity>(kind);
-    case 320: return ChanComplexKernels<320, kDiversity>(kind);
-    case 512: return ChanComplexKernels<512, kDiversity>(kind);
-    default: return ChanComplexKernels<640, kDiversity>(kind);
+    case 64: return ChanComplexKernels<64, kSet>(kind);
+    case 320: return ChanComplexKernels<320, kSet>(kind);
+    case 512: return ChanComplexKernels<512, kSet>(kind);
+    default: return ChanComplexKernels<640, kSet>(kind);
   }
 }
 static ChanKernels ChanKernelsFor(ChanKind kind, int n_channels, int n_inputs) {
-  if (n_inputs == 1) return ChanKernelsOf<false>(kind, n_channels);
-  return ChanKernelsOf<true>(kind, n_channels);
+  if (n_inputs == 1) return ChanKernelsOf<kChanSetPlain>(kind, n_channels);
+  return ChanKernelsOf<kChanSetDiversity>(kind, n_channels);
+}
+/* a complex single-input channelizer's image-correcting kernels (DESIGN §3.12) */
+static ChanKernels ChanImageKernelsFor(ChanKind kind, int n_channels) {
+  switch (n_channels) {
+    case 64: return ChanComplexKernels<64, kChanSetImage>(kind);
+    case 320: return ChanComplexKernels<320, kChanSetImage>(kind);
+    case 512: return ChanComplexKernels<512, kChanSetImage>(kind);
+    default: return ChanComplexKernels<640, kChanSetImage>(kind);
+  }
 }
 
 static int ChanQuiesce(t41rx_chan *c) {
@@ -900,7 +1051,8 @@ void t41rx_chan_destroy(t41rx_chan *c) {
   cudaSetDevice(c->device);
   if (c->ext_pending && c->ev_ext) cudaEventSynchronize(c->ev_ext);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  void *bufs[] = {c->d_taps, c->d_tw, c->d_split, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_weight, c->d_rot};
+  void *bufs[] = {c->d_taps, c->d_tw, c->d_split, c->d_tail, c->d_recv, c->d_chan, c->d_phase, c->d_weight, c->d_rot,
+                  c->d_image, c->d_image_stats};
   for (void *b : bufs)
     if (b) cudaFree(b);
   if (c->ev_ext) cudaEventDestroy(c->ev_ext);
@@ -946,8 +1098,10 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_ext, cudaEventDisableTiming) != cudaSuccess)
     return bail(SetApiError(T41RX_ECUDA, (f + ": stream/event creation failed").c_str()));
+  const bool image = !real && n_inputs == 1;
   c->kernels = ChanKernelsFor(kind, n_channels, n_inputs);
-  if (c->kernels.prepare() != cudaSuccess)
+  if (image) c->image_kernels = ChanImageKernelsFor(kind, n_channels);
+  if (c->kernels.prepare() != cudaSuccess || (image && c->image_kernels.prepare() != cudaSuccess))
     return bail(SetApiError(T41RX_ECUDA, (f + ": kernel image for this GPU missing (built for sm_100a)").c_str()));
   const int N = kChanTaps * n_channels;
   std::vector<float> taps(N);
@@ -977,13 +1131,16 @@ static int ChanCreate(const char *fn, ChanKind kind, t41rx_chan **out, int n_cha
       cudaMalloc(&c->d_chan, sizeof(int32_t) * n_receivers) != cudaSuccess ||
       cudaMalloc(&c->d_phase, sizeof(int2) * n_receivers) != cudaSuccess ||
       (n_inputs > 1 && cudaMalloc(&c->d_weight, sizeof(float2) * n_receivers * n_inputs) != cudaSuccess) ||
-      cudaMalloc(&c->d_rot, sizeof(float2) * rot.size()) != cudaSuccess)
+      cudaMalloc(&c->d_rot, sizeof(float2) * rot.size()) != cudaSuccess ||
+      (image && (cudaMalloc(&c->d_image, sizeof(float2) * n_channels) != cudaSuccess ||
+                 cudaMalloc(&c->d_image_stats, sizeof(double) * 4 * (n_channels / 2 + 1)) != cudaSuccess)))
     return bail(SetApiError(T41RX_ENOMEM, (f + ": device allocation failed").c_str()));
   if (cudaMemcpy(c->d_taps, taps.data(), sizeof(float) * N, cudaMemcpyHostToDevice) != cudaSuccess ||
       cudaMemcpy(c->d_tw, tw.data(), sizeof(float2) * tw_len, cudaMemcpyHostToDevice) != cudaSuccess ||
       (real && cudaMemcpy(c->d_split, split.data(), sizeof(float2) * split.size(), cudaMemcpyHostToDevice) != cudaSuccess) ||
       cudaMemcpy(c->d_rot, rot.data(), sizeof(float2) * rot.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
-      cudaMemset(c->d_tail, 0, tail_bytes) != cudaSuccess)
+      cudaMemset(c->d_tail, 0, tail_bytes) != cudaSuccess ||
+      (image && cudaMemset(c->d_image, 0, sizeof(float2) * n_channels) != cudaSuccess))
     return bail(SetApiError(T41RX_ECUDA, (f + ": table upload failed").c_str()));
   *out = c;
   return T41RX_OK;
@@ -1106,6 +1263,114 @@ int t41rx_chan_set_weights(t41rx_chan *c, int first, int count, const float *w) 
 
 }  // extern "C"
 
+/* the image entry points (DESIGN §3.12) take a complex single-input channelizer; EINVAL on the others, saying why */
+static int ChanImageKind(const std::string &fn, const t41rx_chan *c) {
+  if (!c) return SetApiError(T41RX_EINVAL, (fn + ": null channelizer").c_str());
+  if (c->kind == ChanKind::kReal)
+    return SetApiError(T41RX_EINVAL, (fn + ": a real channelizer has no image correction (a real capture has no I/Q "
+                                           "imbalance, and channel M - k is not a channel it delivers)").c_str());
+  if (c->n_inputs > 1)
+    return SetApiError(T41RX_EINVAL, (fn + ": a diversity channelizer has no image correction (it acts on one "
+                                           "capture's mirror channels; use a single-input channelizer per capture)").c_str());
+  return T41RX_OK;
+}
+
+/* the image table's M coefficients as the next call will read them (after ChanQuiesce) */
+static int ChanImageDownload(t41rx_chan *c, float2 *coef, const std::string &fn) {
+  if (cudaMemcpy(coef, c->d_image, sizeof(float2) * c->n_channels, cudaMemcpyDeviceToHost) != cudaSuccess)
+    return SetApiError(T41RX_ECUDA, (fn + ": download failed").c_str());
+  return T41RX_OK;
+}
+
+static bool ChanImageAny(const std::vector<float2> &tab) {
+  return std::any_of(tab.begin(), tab.end(), [](float2 v) { return v.x != 0.f || v.y != 0.f; });
+}
+
+/* room for the tracking partials of `tiles` tiles: a larger image table, the coefficients copied over.  It waits for
+   the channelizer's calls (and the call's stream st) before it frees the old table */
+static int ChanImageReserve(t41rx_chan *c, long long tiles, cudaStream_t st, const std::string &fn) {
+  if (cudaStreamSynchronize(st) != cudaSuccess) return SetApiError(T41RX_ECUDA, (fn + ": synchronisation failed").c_str());
+  const int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  const size_t pairs = c->n_channels / 2 + 1;
+  float2 *buf = nullptr;
+  if (cudaMalloc(&buf, sizeof(float2) * c->n_channels + sizeof(float4) * pairs * tiles) != cudaSuccess)
+    return SetApiError(T41RX_ENOMEM, (fn + ": device allocation failed (image tracking partials)").c_str());
+  if (cudaMemcpy(buf, c->d_image, sizeof(float2) * c->n_channels, cudaMemcpyDeviceToDevice) != cudaSuccess) {
+    cudaFree(buf);
+    return SetApiError(T41RX_ECUDA, (fn + ": image table copy failed").c_str());
+  }
+  cudaFree(c->d_image);
+  c->d_image = buf;
+  c->image_tiles = tiles;
+  return T41RX_OK;
+}
+
+extern "C" {
+
+int t41rx_chan_set_image(t41rx_chan *c, int first, int count, const float *coef) {
+  const std::string fn = "t41rx_chan_set_image";
+  if (const int rc = ChanImageKind(fn, c)) return rc;
+  if (!coef || first < 0 || count <= 0 || count > c->n_channels - first)
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_set_image: bad range");
+  for (int i = 0; i < 2 * count; ++i)
+    if (!std::isfinite(coef[i])) return SetApiError(T41RX_EINVAL, "t41rx_chan_set_image: coefficients must be finite");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_set_image: cudaSetDevice failed");
+  int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  std::vector<float2> tab(c->n_channels);
+  if ((rc = ChanImageDownload(c, tab.data(), fn))) return rc;    /* tracking may have moved the others */
+  for (int i = 0; i < count; ++i) tab[first + i] = float2{coef[2 * i], coef[2 * i + 1]};
+  if (cudaMemcpy(c->d_image, tab.data(), sizeof(float2) * c->n_channels, cudaMemcpyHostToDevice) != cudaSuccess)
+    return SetApiError(T41RX_ECUDA, "t41rx_chan_set_image: upload failed");
+  c->any_image = ChanImageAny(tab);
+  return T41RX_OK;
+}
+
+int t41rx_chan_get_image(t41rx_chan *c, float *coef) {
+  const std::string fn = "t41rx_chan_get_image";
+  if (const int rc = ChanImageKind(fn, c)) return rc;
+  if (!coef) return SetApiError(T41RX_EINVAL, "t41rx_chan_get_image: null coef");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_get_image: cudaSetDevice failed");
+  const int rc = ChanQuiesce(c);
+  return rc ? rc : ChanImageDownload(c, reinterpret_cast<float2 *>(coef), fn);
+}
+
+int t41rx_chan_track_image(t41rx_chan *c, int on, float dominance_db) {
+  const std::string fn = "t41rx_chan_track_image";
+  if (const int rc = ChanImageKind(fn, c)) return rc;
+  if (on && !(dominance_db >= T41RX_CHAN_DOMINANCE_MIN_DB && dominance_db <= T41RX_CHAN_DOMINANCE_MAX_DB))
+    return SetApiError(T41RX_EINVAL, "t41rx_chan_track_image: dominance_db must be in [3, 60]");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_track_image: cudaSetDevice failed");
+  int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  if (on) {
+    c->track = true;
+    c->dominance = pow(10.0, (double)dominance_db / 10.0);
+    return T41RX_OK;
+  }
+  c->track = false;
+  std::vector<float2> tab(c->n_channels);
+  if ((rc = ChanImageDownload(c, tab.data(), fn))) return rc;
+  c->any_image = ChanImageAny(tab);
+  return T41RX_OK;
+}
+
+int t41rx_chan_image_stats(t41rx_chan *c, double *stats) {
+  const std::string fn = "t41rx_chan_image_stats";
+  if (const int rc = ChanImageKind(fn, c)) return rc;
+  if (!stats) return SetApiError(T41RX_EINVAL, "t41rx_chan_image_stats: null stats");
+  if (!c->has_stats) return SetApiError(T41RX_EINVAL, "t41rx_chan_image_stats: no call has run with tracking on");
+  if (cudaSetDevice(c->device) != cudaSuccess) return SetApiError(T41RX_ECUDA, "t41rx_chan_image_stats: cudaSetDevice failed");
+  const int rc = ChanQuiesce(c);
+  if (rc) return rc;
+  if (cudaMemcpy(stats, c->d_image_stats, sizeof(double) * 4 * (c->n_channels / 2 + 1), cudaMemcpyDeviceToHost) != cudaSuccess)
+    return SetApiError(T41RX_ECUDA, "t41rx_chan_image_stats: download failed");
+  return T41RX_OK;
+}
+
+}  // extern "C"
+
 /* one call of any kind (the caller has checked the pointers and the kind): captures[a], a < n_inputs, holds
    n_blocks x 2048 x D samples of ChanSampleBytes(c->kind) each.  A diversity call runs one pass per input on the same
    stream, input 0 storing and the others accumulating, always in this order, so cutting a run into calls gives the
@@ -1122,10 +1387,29 @@ static int ChanProcess(const char *fn, t41rx_chan *c, const void *const *capture
   const size_t sample_bytes = ChanSampleBytes(c->kind);
   char *tails = (char *)c->d_tail;
   cudaError_t e = cudaSuccess;
-  for (int a = 0; a < c->n_inputs && c->n_entries > 0 && e == cudaSuccess; ++a) {
-    const int store = c->n_inputs == 1 ? kChanPlain : a == 0 ? kChanWeighted : kChanAccumulate;
-    e = c->kernels.launch(c, captures[a], tails + a * N * sample_bytes, store,
-                          c->d_weight ? c->d_weight + (size_t)a * c->n_entries : nullptr, (float2 *)iq, n_blocks, st);
+  if (c->track || c->any_image) {
+    /* image correction (DESIGN §3.12): one pass of an image instance; with tracking, it runs whether or not a receiver
+       is mapped (every pair is measured), and the update follows it on the same stream */
+    const long long tiles = (long long)n_blocks * (T41RX_BLOCK_SAMPLES / kChanTile);
+    if (c->track && tiles > c->image_tiles) {
+      const int rc = ChanImageReserve(c, tiles, st, f);
+      if (rc) return rc;
+    }
+    if (c->n_entries > 0 || c->track)
+      e = c->image_kernels.launch(c, captures[0], tails, c->track ? kChanImageTrack : kChanImage, c->d_image,
+                                  (float2 *)iq, n_blocks, st);
+    if (c->track && e == cudaSuccess) {
+      t41rx_chan_image_update<<<c->n_channels / 2 + 1, kChanImageThreads, 0, st>>>(c->d_image, c->n_channels, (int)tiles,
+                                                                                     c->dominance, c->d_image_stats);
+      e = cudaGetLastError();
+      c->has_stats = c->has_stats || e == cudaSuccess;
+    }
+  } else {
+    for (int a = 0; a < c->n_inputs && c->n_entries > 0 && e == cudaSuccess; ++a) {
+      const int store = c->n_inputs == 1 ? kChanPlain : a == 0 ? kChanWeighted : kChanAccumulate;
+      e = c->kernels.launch(c, captures[a], tails + a * N * sample_bytes, store,
+                            c->d_weight ? c->d_weight + (size_t)a * c->n_entries : nullptr, (float2 *)iq, n_blocks, st);
+    }
   }
   /* the new tails: each input's last N samples, copied after the last pass on the same stream so no tile reads them
      early */

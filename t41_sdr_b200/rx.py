@@ -93,12 +93,14 @@ EXPORTS = (
     "t41rx_chan_taps", "t41rx_chan_tune", "t41rx_chan_set_shift", "t41rx_chan_place",
     "t41rx_chan_create_real", "t41rx_chan_process_device_real", "t41rx_chan_tune_real", "t41rx_chan_place_real",
     "t41rx_chan_create_q15", "t41rx_chan_process_device_q15",
-    "t41rx_chan_create_diversity", "t41rx_chan_set_weights", "t41rx_chan_process_device_diversity")
+    "t41rx_chan_create_diversity", "t41rx_chan_set_weights", "t41rx_chan_process_device_diversity",
+    "t41rx_chan_set_image", "t41rx_chan_get_image", "t41rx_chan_track_image", "t41rx_chan_image_stats")
 
 CHAN_TAPS_PER_BRANCH = 10     # prototype length = 10 * n_channels
 CHAN_SPACING = 96000.0        # channel spacing (Hz); every channel comes out at 192 kS/s
 CHAN_FLOAT, CHAN_Q15, CHAN_REAL = 0, 1, 2   # capture kinds of t41rx_chan_create_diversity
 CHAN_MAX_INPUTS = 4           # a diversity channelizer takes 2 ... 4 coherent captures
+CHAN_DOMINANCE_DB = (3.0, 60.0)   # image tracking's dominance threshold T (dB), T41RX_CHAN_DOMINANCE_MIN/MAX_DB
 
 
 def build_library():
@@ -182,6 +184,10 @@ def lib():
         L.t41rx_chan_create_diversity.argtypes = [C.POINTER(vp), ip, ip, ip, ip, ip]
         L.t41rx_chan_set_weights.argtypes = [vp, ip, ip, C.POINTER(C.c_float)]
         L.t41rx_chan_process_device_diversity.argtypes = [vp, C.POINTER(vp), vp, ip, vp]
+        L.t41rx_chan_set_image.argtypes = [vp, ip, ip, C.POINTER(C.c_float)]
+        L.t41rx_chan_get_image.argtypes = [vp, C.POINTER(C.c_float)]
+        L.t41rx_chan_track_image.argtypes = [vp, ip, C.c_float]
+        L.t41rx_chan_image_stats.argtypes = [vp, C.POINTER(C.c_double)]
         L.t41rx_chan_tune_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.t41rx_chan_place_real.argtypes = [ip, C.c_int32, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                             C.POINTER(C.c_int32)]
@@ -655,6 +661,33 @@ class Channelizer:
         arr = np.ascontiguousarray(np.stack([w.real, w.imag], axis=-1), dtype=np.float32)
         _check(lib().t41rx_chan_set_weights(self._h, int(first), int(w.shape[0]), arr.ctypes.data_as(C.POINTER(C.c_float))),
                "t41rx_chan_set_weights")
+
+    def set_image(self, coef, first=0):
+        """image correction (DESIGN §3.12, complex single-input channelizers): channels first, first + 1, ... take the
+        complex coefficients coef[i], receivers on channel k getting z_k + c_k conj(z_(M - k) mod M) (0 at creation: no
+        correction).  A frequency-independent imbalance x = mu s + nu conj(s) is removed by c_k = -conj(nu) / mu on every
+        channel.  Effective from the next call"""
+        c = np.atleast_1d(np.asarray(coef, dtype=np.complex128))
+        arr = np.ascontiguousarray(np.stack([c.real, c.imag], axis=-1), dtype=np.float32)
+        _check(lib().t41rx_chan_set_image(self._h, int(first), int(c.size), arr.ctypes.data_as(C.POINTER(C.c_float))),
+               "t41rx_chan_set_image")
+
+    def get_image(self):
+        """all n_channels image coefficients (complex64), including what tracking has made of them"""
+        arr = np.empty((self.n_channels, 2), np.float32)
+        _check(lib().t41rx_chan_get_image(self._h, arr.ctypes.data_as(C.POINTER(C.c_float))), "t41rx_chan_get_image")
+        return arr[:, 0] + 1j * arr[:, 1]
+
+    def track_image(self, on=True, dominance_db=20.0):
+        """image tracking on or off from the next call: each call measures every mirror pair and corrects the weak side
+        of a pair whose other side is dominance_db (3 ... 60) or more stronger, for the next call"""
+        _check(lib().t41rx_chan_track_image(self._h, int(bool(on)), float(dominance_db)), "t41rx_chan_track_image")
+
+    def image_stats(self):
+        """float64 [n_channels / 2 + 1, 4]: (Re A, Im A, P_k, P_kbar) of pair k from the last call with tracking on"""
+        out = np.empty((self.n_channels // 2 + 1, 4), np.float64)
+        _check(lib().t41rx_chan_image_stats(self._h, out.ctypes.data_as(C.POINTER(C.c_double))), "t41rx_chan_image_stats")
+        return out
 
     def process_device(self, capture_ptr, iq_ptr, n_blocks, stream=None):
         """capture float32 [n_blocks * 2048 * n_channels / 2, 2] (real: int16 [n_blocks * 2048 * n_channels / 2];

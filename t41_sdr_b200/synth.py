@@ -237,6 +237,35 @@ def wideband_q15(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
     return out
 
 
+def wideband_sum(seed, n_channels, n_blocks, signals, sigma=0.0, start_block=0):
+    """The complex128 sum wideband() rounds to float32, before any rounding or quantisation (e.g. for iq_imbalance)."""
+    return _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block)
+
+
+def iq_imbalance(z, gain, phase_deg, skew_samples=0.0):
+    """An I/Q digitizer's branch mismatch applied to a complex capture z (complex128), in float64: I' = Re z and
+        Q' = d(g (Q cos phi + I sin phi)),
+    g = gain, phi = phase_deg, d a delay of skew_samples (fractional) of the Q branch, band-limited and circular over z
+    (multiply the DFT of the branch by exp(-2 pi j f skew_samples), f in cycles per sample; the identity at 0).  With
+    skew 0 this is x = mu z + nu conj(z), mu = (1 + g e^(j phi)) / 2, nu = (1 - g e^(-j phi)) / 2."""
+    z = np.asarray(z, np.complex128)
+    phi = np.deg2rad(phase_deg)
+    q = gain * (z.imag * np.cos(phi) + z.real * np.sin(phi))
+    if skew_samples != 0.0:
+        f = np.fft.rfftfreq(z.size)
+        q = np.fft.irfft(np.fft.rfft(q) * np.exp(-2j * np.pi * f * skew_samples), z.size)
+    return z.real + 1j * q
+
+
+def iq_imbalance_q15(z, gain, phase_deg, skew_samples=0.0):
+    """iq_imbalance() as an sc16 capture: int16 [n, 2] (I, Q), quantised as wideband_q15()"""
+    x = iq_imbalance(z, gain, phase_deg, skew_samples)
+    out = np.empty((x.size, 2), np.int16)
+    out[:, 0] = np.clip(np.round(32768.0 * x.real), -32768, 32767)
+    out[:, 1] = np.clip(np.round(32768.0 * x.imag), -32768, 32767)
+    return out
+
+
 def _wideband_sum(seed, n_channels, n_blocks, signals, sigma, start_block, delay=0):
     """complex128 signal sum and noise of wideband() / wideband_real() / wideband_q15(); delay: the signals (not the
     noise) delayed by that many capture samples"""

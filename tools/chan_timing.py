@@ -1,6 +1,7 @@
 """Channelizer timing on one GPU (DESIGN §3.7 - 3.9): M = 512 channels, 1024 receivers (2 per channel), 64 blocks per call.
 
-    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--rates] [--diversity N] [--json OUT]
+    python tools/chan_timing.py [--calls 20] [--warmup 3] [--shift] [--real] [--q15] [--rates] [--diversity N] [--image]
+                                [--json OUT]
 
 Prints the card's name and power limit (a query), then CUDA-event times of
   - t41rx_chan_process_device alone (capture 268 MB, larger than the 126 MB L2; iq out 1 GiB),
@@ -23,6 +24,10 @@ Prints the card's name and power limit (a query), then CUDA-event times of
     shape: complex float and int16 pairs at M = 512, real at M = 1024 and 1280; the same 1024 receivers, 2 per channel,
     64 blocks per call, every receiver shifted and given seeded weights on every input (none of them the default).  The
     single-input call alternates between two of the N captures; the N-input call reads all N (each at least 134 MB),
+  - with --image (DESIGN §3.12), image correction against the plain call of the same channelizer: complex float at
+    M = 512 and int16 pairs at M = 640; the same 1024 receivers, 2 per channel, 64 blocks per call, every receiver
+    shifted; the plain call (every c_k 0), fixed seeded coefficients on every channel, tracking on (from those
+    coefficients), and the plain call again, in that order on one channelizer,
 each over --calls calls after --warmup calls.  Bytes moved are computed from shapes (capture read once, every mapped
 receiver's iq written once) and given as a share of the B200's 7.7 TB/s HBM3e.
 """
@@ -167,6 +172,50 @@ def diversity_table(g, dev, iq, sp, timed, shifts, S, T, n_inputs):
     return out
 
 
+def image_table(g, dev, iq, sp, timed, shifts, S, T):
+    """the --image measurements: per (kind, M) the plain call, fixed coefficients and tracking, and their ratios to
+    the plain call against the goals (at most 1.10 x fixed, 1.25 x tracking)"""
+    import torch
+    r = np.random.Generator(np.random.PCG64(2027))
+    chmap = [(i // 2) % 512 for i in range(S)]
+    out = {}
+    for kind, M in (("complex", 512), ("q15", 640)):
+        q15 = kind == "q15"
+        n_cap = T * rx.BLOCK * M // 2
+        if q15:
+            cap = torch.randint(-3277, 3278, (n_cap, 2), generator=g, device=dev, dtype=torch.int16)
+        else:
+            cap = (0.1 * torch.randn((n_cap, 2), generator=g, device=dev)).contiguous()
+        chan = rx.Channelizer(M, S, q15=q15)
+        chan.set_map(chmap)
+        chan.set_shift(shifts)
+
+        def do():
+            chan.process_device(cap.data_ptr(), iq.data_ptr(), T, stream=sp)
+
+        t_plain = timed(do)
+        chan.set_image(0.03 * r.uniform(0.1, 1, M) * np.exp(2j * np.pi * r.uniform(0, 1, M)))
+        t_fixed = timed(do)
+        chan.track_image(True, 20.0)
+        t_track = timed(do)
+        chan.track_image(False)
+        chan.set_image(np.zeros(M))
+        t_plain2 = timed(do)
+        chan.synchronize()
+        chan.close()
+        base = min(t_plain[0], t_plain2[0])
+        out["%s_%d" % (kind, M)] = {
+            "capture_bytes": cap.numel() * cap.element_size(),
+            "plain_ms": {"median": t_plain[0], "min": t_plain[1], "max": t_plain[2]},
+            "fixed_ms": {"median": t_fixed[0], "min": t_fixed[1], "max": t_fixed[2]},
+            "tracking_ms": {"median": t_track[0], "min": t_track[1], "max": t_track[2]},
+            "plain_again_ms": {"median": t_plain2[0], "min": t_plain2[1], "max": t_plain2[2]},
+            "fixed_over_plain": t_fixed[0] / base, "goal_fixed_le_1p10": t_fixed[0] <= 1.10 * base,
+            "tracking_over_plain": t_track[0] / base, "goal_tracking_le_1p25": t_track[0] <= 1.25 * base}
+        del cap
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--channels", type=int, default=512)
@@ -180,6 +229,7 @@ def main():
     ap.add_argument("--rates", action="store_true", help="also time every channel count beside its power-of-two neighbour")
     ap.add_argument("--diversity", type=int, default=0, metavar="N",
                     help="also time an N-input diversity call against the single-input call (N = 2 ... 4)")
+    ap.add_argument("--image", action="store_true", help="also time image correction, fixed and tracking")
     ap.add_argument("--json", default=None, help="also write the result here")
     a = ap.parse_args()
     import torch
@@ -279,6 +329,7 @@ def main():
             c.close()
     rates = rate_table(g, dev, iq, sp, timed, shifts, S, T) if a.rates else None
     diversity = diversity_table(g, dev, iq, sp, timed, shifts, S, T, a.diversity) if a.diversity else None
+    image = image_table(g, dev, iq, sp, timed, shifts, S, T) if a.image else None
     eng.synchronize()
     bytes_moved = n_cap * 8 + S * T * rx.BLOCK * 8
     res = {
@@ -331,6 +382,8 @@ def main():
         res["rates"] = rates
     if diversity:
         res["diversity"] = {"n_inputs": a.diversity, "every_receiver_shifted_and_weighted": True, **diversity}
+    if image:
+        res["image"] = {"every_receiver_shifted": True, **image}
     print(json.dumps(res, indent=1))
     if a.json:
         with open(a.json, "w") as f:
